@@ -3,6 +3,11 @@
 bench.py — CookTorrance forward+backward throughput (BASELINE.json metric), one JSON line on stdout.
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config c2|c1|c3|c4|c5|aux]
+                  [--dump-outputs DIR]
+
+Every GPU timing of our arm (the config's value, the configs block, the e2e legs, the c4 / aux kernel rows, the c1 CUDA
+graph replay) runs max(W, 3) warm-up steps and then exactly K timed steps.  The cpu_baseline and gpu_eager_baseline
+samples do not follow K: they are best-of-a-few samples bounded in time, so that the line stays affordable.
 
 Main line (default --config c2, N=1): BASELINE.json configs[1] — batch 64 materials 1024x1024, CookTorrance
 forward+backward, 1 point light, fp32, metallic workflow, sRGB albedo in / sRGB colour out.  A step = one forward pass
@@ -172,11 +177,14 @@ def lights_for(L):
 
 def config1_fixture():
     """BASELINE.json configs[0]: the reference's tests/data/tiles material at 256x256 with example_brdf.py's lighting
-    (tests/golden/config1_tiles_256.npz, written by tests/golden/make_golden.py from the reference's own loader)."""
+    (tests/golden/config1_tiles_256.npz and its normal map in config1_tiles_256.in_normal.npz, written by
+    tests/golden/make_golden.py from the reference's own loader)."""
     import numpy as np
 
-    z = np.load(os.path.join(ROOT, "tests", "golden", "config1_tiles_256.npz"))
-    maps = {k[3:]: torch.from_numpy(z[k]) for k in z.files if k.startswith("in_")}
+    golden = os.path.join(ROOT, "tests", "golden", "config1_tiles_256")
+    z = np.load(golden + ".npz")
+    normal = np.load(golden + ".in_normal.npz")["in_normal"]
+    maps = {k: torch.from_numpy(normal if k == "normal" else z["in_" + k]) for k in ("albedo", "normal", "roughness", "metallic")}
     return maps, torch.from_numpy(z["view"]), torch.from_numpy(z["lights"]), torch.from_numpy(z["intensity"])
 
 
@@ -478,9 +486,32 @@ def make_material(maps, dev, requires_grad):
     return mat, leaves
 
 
-def measure_shading(name, args, ctx, steps, warmup):
+DUMP_BYTES = 60_000_000   # --dump-outputs: what the sampled arrays may take, under a 64 MB cap for the whole directory
+
+
+def dump_outputs(out_dir, arrays, B, H, W):
+    """--dump-outputs: each (B, ..., H, W) array of `arrays` (or (C, H, W) with B = 1) as out_dir/<name>.npy in float32,
+    shaped (texels, channels) and taken at the same texel positions: all B*H*W in order when they fit DUMP_BYTES, else a
+    fixed sample (seed 0, sorted, no repeats).  Any other array is written whole, in float64."""
+    import numpy as np
+
+    os.makedirs(out_dir, exist_ok=True)
+    texels = B * H * W
+    planes = {k: v.detach().reshape(B, -1, H * W) for k, v in arrays.items() if v.dim() >= 3 and tuple(v.shape[-2:]) == (H, W)}
+    n = min(texels, DUMP_BYTES // (4 * sum(v.shape[1] for v in planes.values())))
+    idx = torch.randint(0, texels, (n,), generator=torch.Generator().manual_seed(0)).unique() if n < texels else torch.arange(texels)
+    idx = idx.to(next(iter(planes.values())).device)
+    b, p = idx // (H * W), idx % (H * W)
+    for k, v in arrays.items():
+        a = planes[k][b, :, p].float() if k in planes else v.detach().double()
+        np.save(os.path.join(out_dir, k + ".npy"), a.cpu().numpy())
+
+
+def measure_shading(name, args, ctx, steps, warmup, dump_dir=None):
     """One shading config (c2 / c3 / c5) on this rank's shard: W warm-up steps, then `steps` steps between two CUDA events,
-    bracketed by barrier + synchronize, max over ranks.  Returns the config's result object."""
+    bracketed by barrier + synchronize, max over ranks.  Returns the config's result object.
+    dump_dir: write what the last timed step returned to its caller there (dump_outputs; rank 0's shard): the forward output
+    and the map gradients, or for the fit (c5) the maps after the update and the step's loss buffer."""
     from pypbr_b200.fit import FusedAdam, allreduce_loss_and_shared, fit_step, fused_loss_step
     from pypbr_b200.models import CookTorranceBRDF
 
@@ -510,8 +541,9 @@ def measure_shading(name, args, ctx, steps, warmup):
     ev = lambda: torch.cuda.Event(enable_timing=True)
     fwd_ms, bwd_ms = [], []
     last = [None]
+    kept = {}   # what the last timed step returned, held only when it is to be dumped
 
-    def step(record=False):
+    def step(record=False, keep=False):
         if fused_fit:
             # one full step of the sharded fit: fused render + MSE + backward, ONE all-reduce, fused Adam + projection
             e0, e1, e2 = ev(), ev(), ev()
@@ -525,6 +557,8 @@ def measure_shading(name, args, ctx, steps, warmup):
                 e1.record()
                 if record:
                     bwd_ms.append((e0, e1))
+                if keep:
+                    kept["loss_buffer"] = last[0].buf if async_loss else last[0]
                 return
             # --shared-grads: the fit with unknown lighting - intensity, light position and view gradients ride along
             # (PbrCtGrads.d_intensity / d_lights / d_view; 1 + 6L + 3 floats to all-reduce instead of 1 + 3L)
@@ -538,16 +572,20 @@ def measure_shading(name, args, ctx, steps, warmup):
             if record:
                 bwd_ms.append((e0, e1))
                 adam_ms.append((e1, e2))
+            if keep:
+                kept["loss_buffer"] = buf
             return
         e0, e1, e2 = ev(), ev(), ev()
         e0.record()
         out = brdf(mat, view, lights, inten, 1.0)
         e1.record()
-        torch.autograd.grad(out, leaves, grad_out)
+        grads = torch.autograd.grad(out, leaves, grad_out)
         e2.record()
         if record:
             fwd_ms.append((e0, e1))
             bwd_ms.append((e1, e2))
+        if keep:
+            kept.update(out=out, **{"grad_" + k: t for k, t in zip(maps, grads)})
 
     for _ in range(warmup):
         step()
@@ -556,8 +594,8 @@ def measure_shading(name, args, ctx, steps, warmup):
     t_start, t_end = ev(), ev()
     with ClockSampler(ctx.local) as clk:
         t_start.record()
-        for _ in range(steps):
-            step(record=True)
+        for i in range(steps):
+            step(record=True, keep=dump_dir is not None and i == steps - 1)
         if async_loss and last[0] is not None:
             last[0].wait()   # the timed region ends when the last step's loss has been reduced as well
         t_end.record()
@@ -565,6 +603,11 @@ def measure_shading(name, args, ctx, steps, warmup):
     launches = ctx.cabi.launch_count() - launches0
     elapsed_ms = ctx.max_over_ranks(t_start.elapsed_time(t_end))
     ctx.barrier()
+    if dump_dir is not None and rank == 0:
+        if fused_fit:
+            kept.update((k, mat._maps[k]) for k in maps)   # the parameters as the last step's update left them
+        dump_outputs(dump_dir, kept, B, H, W)
+    kept.clear()
 
     texel_lights_per_step = B * H * W * L * world
     value = texel_lights_per_step * steps / (elapsed_ms * 1e-3) / 1e9
@@ -630,10 +673,11 @@ def measure_shading(name, args, ctx, steps, warmup):
     return res
 
 
-def measure_c1(args, ctx):
+def measure_c1(ctx, steps, warmup, dump_dir=None):
     """BASELINE.json configs[0]: one 256x256 material, one point light - a launch-latency-bound call.  Microseconds per
     `brdf()` call (forward) and per forward+backward through autograd, back to back, CUDA events around the loop (host
-    launch overhead included: that is what a caller sees)."""
+    launch overhead included: that is what a caller sees).  `warmup` + `steps` calls of each, and as many replays of the
+    CUDA graph.  dump_dir: write what the last timed forward+backward returned there (dump_outputs)."""
     from pypbr_b200.models import CookTorranceBRDF
 
     maps, view, lights, inten = config1_fixture()
@@ -650,24 +694,30 @@ def measure_c1(args, ctx):
 
     def fwd_bwd():
         out = brdf(mat, view_d, lights_d, inten_d, 1.0)
-        torch.autograd.grad(out, leaves, go)
+        return out, torch.autograd.grad(out, leaves, go)
 
-    res = {}
-    n = 200
+    res, last = {}, None
     launches0 = ctx.cabi.launch_count()
     with ClockSampler(ctx.local) as clk:
         for key, fn in (("fwd_us", fwd), ("fwd_bwd_us", fwd_bwd)):
-            for _ in range(20):
+            for _ in range(warmup):
                 fn()
             ctx.barrier()
             a, b = ev(), ev()
             a.record()
-            for _ in range(n):
-                fn()
+            for i in range(steps):
+                r = fn()
+                if dump_dir is not None and fn is fwd_bwd and i == steps - 1:
+                    last = r
+                del r
             b.record()
             torch.cuda.synchronize()
-            res[key] = ctx.max_over_ranks(a.elapsed_time(b)) / n * 1e3
+            res[key] = ctx.max_over_ranks(a.elapsed_time(b)) / steps * 1e3
     launches = ctx.cabi.launch_count() - launches0
+    if last is not None and ctx.rank == 0:
+        out, grads = last
+        dump_outputs(dump_dir, {"out": out, **{"grad_" + k: t for k, t in zip(maps, grads)}}, 1, C1["H"], C1["W"])
+    del last
     # the kernels alone (CUDA graph replay of the same two launches: no host time between them)
     graph_us = None
     try:
@@ -679,23 +729,24 @@ def measure_c1(args, ctx):
         gr = torch.cuda.CUDAGraph()
         with torch.cuda.graph(gr):
             fwd_bwd()
-        for _ in range(5):
+        for _ in range(warmup):
             gr.replay()
         torch.cuda.synchronize()
         a, b = ev(), ev()
         a.record()
-        for _ in range(n):
+        for _ in range(steps):
             gr.replay()
         b.record()
         torch.cuda.synchronize()
-        graph_us = a.elapsed_time(b) / n * 1e3
+        graph_us = a.elapsed_time(b) / steps * 1e3
     except Exception as e:  # pragma: no cover
         graph_us = f"capture failed: {str(e)[:80]}"
     texels = C1["H"] * C1["W"]
     return {"value": texels * ctx.world / (res["fwd_bwd_us"] * 1e-6) / 1e9, "unit": UNIT, "ms_per_step": res["fwd_bwd_us"] * 1e-3,
-            "steps": n, "warmup": 20, **res, "fwd_bwd_cuda_graph_us": graph_us,
+            "steps": steps, "warmup": warmup, **res, "fwd_bwd_cuda_graph_us": graph_us,
             "config": {"workload": C1["workload"], "H": C1["H"], "W": C1["W"], "lights": 1,
-                       "inputs": "tests/golden/config1_tiles_256.npz (the reference's tests/data/tiles material, its own loader + resize)",
+                       "inputs": "tests/golden/config1_tiles_256.npz + config1_tiles_256.in_normal.npz (the reference's tests/data/tiles "
+                                 "material, its own loader + resize)",
                        "l2": "2 MB of maps: L2-resident by nature of the config (a single small material); the number is launch latency, not bandwidth"},
             "roofline": {"bound": "launch latency", "note": "0.26 Mtexel per call: 120 B/texel x 65536 texels = 7.9 MB per fwd+bwd, ~1.2 us at the HBM roof"},
             "gpu_launches": int(launches), "clocks": clk.summary()}
@@ -728,13 +779,14 @@ class _Pipe:
         self.used[slot] = True
 
 
-def measure_e2e(args, ctx, cfg, tgt_brdf_inputs):
+def measure_e2e(ctx, cfg, steps, warmup):
     """End to end through the public API with HOST buffers (C2 shape).  Three legs, all chunk-pipelined (H2D of the next
     chunk overlaps the kernels of the current one), wall clock between two device synchronisations, max over ranks:
       primary      : uint8 textures (B,H,W,C) in pinned memory -> H2D -> pbr_ingest_image -> brdf() (K1) -> autograd backward
                      (K2) -> D2H of d(light intensity), the reduction the backward delivers (12 bytes)
       f32_maps_grads_to_host : float32 maps in pinned memory -> H2D -> K1 -> K2 -> D2H of every map gradient (32 B/texel)
       fit_uint8    : uint8 textures -> H2D -> ingest -> fused loss kernel (K3: render + MSE + backward) -> D2H of the loss
+    Each leg: `warmup` steps, then `steps` timed steps.
     """
     from pypbr_b200.fit import fused_loss_step
     from pypbr_b200.materials import BasecolorMetallicMaterial
@@ -754,10 +806,9 @@ def measure_e2e(args, ctx, cfg, tgt_brdf_inputs):
     g = torch.Generator(device=dev).manual_seed(123 + rank)
     grad_out = torch.rand(chunk, 3, H, W, generator=g, device=dev)      # upstream gradient: resident, like in `value`
     target = torch.rand(chunk, 3, H, W, generator=g, device=dev)
-    n_steps = max(3, min(args.steps, 10))
 
     def timed(run_step, finish, n):
-        for s in range(2):
+        for s in range(warmup):
             run_step(s)
         finish()
         ctx.barrier()
@@ -833,14 +884,14 @@ def measure_e2e(args, ctx, cfg, tgt_brdf_inputs):
         unit[0] = 0
         pipe.used = [False, False]
 
-    dt = timed(step_render_grad_u8, finish, n_steps)
-    primary = {"value": texel_lights_per_step * n_steps / dt / 1e9, "unit": UNIT, "h2d_bytes_per_step": h2d8, "d2h_bytes_per_step": 12,
-               "steps": n_steps, "ms_per_step": dt / n_steps * 1e3,
+    dt = timed(step_render_grad_u8, finish, steps)
+    primary = {"value": texel_lights_per_step * steps / dt / 1e9, "unit": UNIT, "h2d_bytes_per_step": h2d8, "d2h_bytes_per_step": 12,
+               "steps": steps, "warmup": warmup, "ms_per_step": dt / steps * 1e3,
                "path": "pinned host uint8 (B,H,W,C) textures -> H2D in chunks of 8 materials (copy stream, double-buffered) -> pbr_ingest_image x4 -> "
                        "CookTorranceBRDF.__call__ (pbr_ct_forward) -> torch.autograd.grad (pbr_ct_backward; map gradients stay in HBM for the optimiser) -> "
                        "D2H of d(light_intensity) (12 bytes)",
-               "h2d_gbs": h2d8 / (dt / n_steps) / 1e9, "h2d_ceiling_gbs": h2d_ceiling,
-               "frac_of_h2d_ceiling": h2d8 / (dt / n_steps) / 1e9 / h2d_ceiling,
+               "h2d_gbs": h2d8 / (dt / steps) / 1e9, "h2d_ceiling_gbs": h2d_ceiling,
+               "frac_of_h2d_ceiling": h2d8 / (dt / steps) / 1e9 / h2d_ceiling,
                "bound": "host->device copy rate of this host at this many ranks (h2d_ceiling_gbs: the same buffers copied with no kernels "
                         "running, all ranks at once, measured in this run)", "numa": ctx.numa}
 
@@ -861,9 +912,9 @@ def measure_e2e(args, ctx, cfg, tgt_brdf_inputs):
         loss_acc.zero_()
 
     fit_bufs, loss_acc = {}, torch.zeros(1, device=dev)
-    dt = timed(step_fit_u8, finish, n_steps)
-    legs["fit_uint8"] = {"value": texel_lights_per_step * n_steps / dt / 1e9, "unit": UNIT, "h2d_bytes_per_step": h2d8, "d2h_bytes_per_step": 4,
-                         "ms_per_step": dt / n_steps * 1e3, "h2d_gbs": h2d8 / (dt / n_steps) / 1e9,
+    dt = timed(step_fit_u8, finish, steps)
+    legs["fit_uint8"] = {"value": texel_lights_per_step * steps / dt / 1e9, "unit": UNIT, "h2d_bytes_per_step": h2d8, "d2h_bytes_per_step": 4,
+                         "steps": steps, "ms_per_step": dt / steps * 1e3, "h2d_gbs": h2d8 / (dt / steps) / 1e9,
                          "path": "pinned host uint8 textures -> H2D (chunked, overlapped) -> pbr_ingest_image x4 -> pypbr_b200.fit.fused_loss_step "
                                  "(pbr_ct_loss_fwd_bwd: render + MSE + backward in one launch) -> D2H of the loss (4 bytes)"}
     del host8, stage8
@@ -874,7 +925,6 @@ def measure_e2e(args, ctx, cfg, tgt_brdf_inputs):
     host_grads = {k: torch.empty(v.shape, dtype=torch.float32).pin_memory() for k, v in host.items()}
     stage = [{k: torch.empty((chunk, *v.shape[1:]), dtype=torch.float32, device=dev) for k, v in host.items()} for _ in range(2)]
     d2h_stream = torch.cuda.Stream(device=dev)
-    n_steps32 = max(2, min(args.steps, 4))
 
     def upload32(i):
         slot, c = i % 2, i % n_chunks
@@ -901,10 +951,10 @@ def measure_e2e(args, ctx, cfg, tgt_brdf_inputs):
                     gt.record_stream(d2h_stream)
             unit[0] += 1
 
-    dt = timed(step_f32, finish, n_steps32)
+    dt = timed(step_f32, finish, steps)
     legs["f32_maps_grads_to_host"] = {
-        "value": texel_lights_per_step * n_steps32 / dt / 1e9, "unit": UNIT, "h2d_bytes_per_step": h2d, "d2h_bytes_per_step": h2d,
-        "ms_per_step": dt / n_steps32 * 1e3, "h2d_gbs": h2d / (dt / n_steps32) / 1e9,
+        "value": texel_lights_per_step * steps / dt / 1e9, "unit": UNIT, "h2d_bytes_per_step": h2d, "d2h_bytes_per_step": h2d,
+        "steps": steps, "ms_per_step": dt / steps * 1e3, "h2d_gbs": h2d / (dt / steps) / 1e9,
         "path": "pinned host float32 maps -> H2D (chunked, overlapped) -> pbr_ct_forward -> pbr_ct_backward -> D2H of all four map gradients "
                 "into pinned host memory (third stream; PCIe full duplex)"}
     primary["legs"] = legs
@@ -916,9 +966,9 @@ def run_ours(args):
     name = args.config
     steps, warmup = args.steps, max(args.warmup, 3)
     if name == "c1":
-        res = measure_c1(args, ctx)
+        res = measure_c1(ctx, steps, warmup, dump_dir=args.dump_outputs)
     else:
-        res = measure_shading(name, args, ctx, steps, warmup)
+        res = measure_shading(name, args, ctx, steps, warmup, dump_dir=args.dump_outputs)
     line = {"metric": METRIC, "value": res["value"], "unit": UNIT, "n_gpus": ctx.world, "steps": res["steps"], "warmup": res["warmup"],
             "ms_per_step": res["ms_per_step"], "higher_is_better": True, "scaling": "weak", "vs_baseline": None, "dtype": "f32",
             "data": "synthetic", "config": res["config"], "roofline": res["roofline"]}
@@ -929,7 +979,7 @@ def run_ours(args):
     solo = ctx.rank == 0 and ctx.world == 1
     line["cpu_baseline"] = cpu_baseline_for(name) if (solo and not args.no_cpu) else None
     line["gpu_eager_baseline"] = gpu_eager_baseline(name, ctx.dev, res["value"]) if (solo and not args.no_eager) else None
-    line["e2e"] = measure_e2e(args, ctx, CONFIGS["c2"], None) if (name == "c2" and not args.no_e2e) else None
+    line["e2e"] = measure_e2e(ctx, CONFIGS["c2"], steps, warmup) if (name == "c2" and not args.no_e2e) else None
     torch.cuda.empty_cache()
     line["gpu_launches"] = res["gpu_launches"]
     line["clocks"] = res["clocks"]
@@ -938,7 +988,7 @@ def run_ours(args):
         # path with a collective must be in the driver-run line, at every N)
         cfgs = {}
         for k in ("c1", "c3", "c5"):
-            r = measure_c1(args, ctx) if k == "c1" else measure_shading(k, args, ctx, steps, warmup)
+            r = measure_c1(ctx, steps, warmup) if k == "c1" else measure_shading(k, args, ctx, steps, warmup)
             if solo and not args.no_cpu:
                 r["cpu_baseline"] = cpu_baseline_for(k, reps=2, budget_s=6.0)
             if solo and not args.no_eager and k == "c1":
@@ -962,7 +1012,7 @@ def run_ours(args):
 
 
 # ---------------------------------------------------------------------------------------------- config 4
-def run_c4(args, emit=True):
+def run_c4(args, emit=True, dump_dir=None):
     """
     BASELINE.json configs[3] (SURVEY.md §8d "C4"): two 4096x4096 metallic materials (albedo, normal, roughness,
     metallic, height) -> to_diffuse_specular_material() on each -> blend_materials(d1, d2, "mask", mask) ->
@@ -971,6 +1021,8 @@ def run_c4(args, emit=True):
                  read-back happens inside: the stream is never drained), CUDA-event time per pipeline
       kernels  : every kernel on its own through the C ABI on preallocated buffers (launches back to back between
                  two CUDA events), algorithmic bytes / time against the measured HBM peak
+    Each: warm-up, then --steps timed repetitions.  dump_dir: write what the last timed pipeline returned there
+    (dump_outputs): the maps of both blended materials and the height blend's mask.
     """
     from pypbr_b200 import _cabi
     from pypbr_b200.blending import blend_materials
@@ -1007,35 +1059,45 @@ def run_c4(args, emit=True):
         return b1, b2, mk
 
     ev = lambda: torch.cuda.Event(enable_timing=True)
-    for _ in range(max(args.warmup, 3)):
+    steps, warmup = args.steps, max(args.warmup, 3)
+    for _ in range(warmup):
         pipeline()
     torch.cuda.synchronize()
     l0 = _cabi.launch_count()
     e0, e1 = ev(), ev()
     with ClockSampler(local) as clk:
         e0.record()
-        for _ in range(args.steps):
-            pipeline()
+        for i in range(steps):
+            r = pipeline()
+            if dump_dir is not None and i == steps - 1:
+                last = r
+            del r
         e1.record()
         torch.cuda.synchronize()
     launches = _cabi.launch_count() - l0
-    pipe_ms = e0.elapsed_time(e1) / args.steps
+    pipe_ms = e0.elapsed_time(e1) / steps
+    if dump_dir is not None:
+        b1, b2, mk = last
+        out = {f"mask_blend_{k}": t for k, t in b1._maps.items() if t is not None}
+        out.update({f"height_blend_{k}": t for k, t in b2._maps.items() if t is not None}, height_mask=mk)
+        dump_outputs(dump_dir, out, 1, H, W)
+        del last, b1, b2, mk, out
 
     # kernel-only legs through the C ABI
     d1 = m1.to_diffuse_specular_material()
     d2 = m2.to_diffuse_specular_material()
 
-    def timed(fn, reps=10):
-        for _ in range(3):
+    def timed(fn):
+        for _ in range(warmup):
             fn()
         torch.cuda.synchronize()
         a, b = ev(), ev()
         a.record()
-        for _ in range(reps):
+        for _ in range(steps):
             fn()
         b.record()
         torch.cuda.synchronize()
-        return a.elapsed_time(b) / reps
+        return a.elapsed_time(b) / steps
 
     kernels = {}
 
@@ -1086,7 +1148,7 @@ def run_c4(args, emit=True):
     dom = max(kernels.items(), key=lambda kv: kv[1]["ms"])
     line = {
         "metric": "Gtexel/s conversion + blend pipeline", "value": texels / (pipe_ms * 1e-3) / 1e9, "unit": "Gtexel/s",
-        "n_gpus": 1, "steps": args.steps, "warmup": max(args.warmup, 3), "ms_per_step": pipe_ms, "higher_is_better": True,
+        "n_gpus": 1, "steps": steps, "warmup": warmup, "ms_per_step": pipe_ms, "higher_is_better": True,
         "scaling": "weak", "vs_baseline": None, "dtype": "f32", "data": "synthetic",
         "config": {"workload": C4["workload"], "H": H, "W": W,
                    "pipeline": "2 x to_diffuse_specular_material + blend_materials(mask) + blend_materials(height), public API",
@@ -1106,7 +1168,8 @@ def run_c4(args, emit=True):
 
 # ---------------------------------------------------------------------------------------------- aux rows (SURVEY.md 8f)
 def run_aux(args):
-    """Kernel-only timings of the rows either side of the shading path: image ingestion, index transforms, Adam."""
+    """Kernel-only timings of the rows either side of the shading path: image ingestion, index transforms, Adam.  Each
+    kernel: warm-up, then --steps timed launches."""
     from pypbr_b200 import _cabi
     from pypbr_b200.fit import FusedAdam
     from pypbr_b200.materials import BasecolorMetallicMaterial
@@ -1122,18 +1185,19 @@ def run_aux(args):
     texels = B * H * W
     peak, peak_src = measured_peak()
     ev = lambda: torch.cuda.Event(enable_timing=True)
+    steps, warmup = args.steps, max(args.warmup, 3)
 
-    def timed(fn, reps=10):
-        for _ in range(3):
+    def timed(fn):
+        for _ in range(warmup):
             fn()
         torch.cuda.synchronize()
         a, b = ev(), ev()
         a.record()
-        for _ in range(reps):
+        for _ in range(steps):
             fn()
         b.record()
         torch.cuda.synchronize()
-        return a.elapsed_time(b) / reps
+        return a.elapsed_time(b) / steps
 
     kernels = {}
 
@@ -1192,7 +1256,7 @@ def run_aux(args):
     dom = max(kernels.items(), key=lambda kv: kv[1]["ms"])
     line = {
         "metric": "GB/s of the ingestion / index-transform / optimiser kernels", "value": dom[1]["achieved"], "unit": "GB/s",
-        "n_gpus": 1, "steps": 10, "warmup": 3, "ms_per_step": dom[1]["ms"], "higher_is_better": True, "scaling": "weak",
+        "n_gpus": 1, "steps": steps, "warmup": warmup, "ms_per_step": dom[1]["ms"], "higher_is_better": True, "scaling": "weak",
         "vs_baseline": None, "dtype": "f32", "data": "synthetic",
         "config": {"workload": f"SURVEY 8f rows on {B} materials {H}x{W}: image ingestion, index transforms, Adam step, normal utilities",
                    "l2": "every kernel streams 1-15 GB, far above the 126 MB L2; no flush needed"},
@@ -1219,13 +1283,20 @@ def main():
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--no-eager", action="store_true")
     ap.add_argument("--no-configs", action="store_true", help="c2: skip the c1 / c3 / c5 block of the line")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="c1-c5: after the timed steps, write what the last one returned as DIR/<name>.npy (a fixed "
+                         "sample of texel positions, under 64 MB in all); the inputs are the same on every run")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs is not None and (args.impl != "ours" or args.config == "aux"):
+        ap.error("--dump-outputs covers the timed paths of --config c1-c5 (--impl ours)")
     if args.impl == "reference":
         if args.config == "aux":
             raise SystemExit("bench.py: the reference arm is defined for c1-c5")
         return run_reference_arm(args)
     if args.config == "c4":
-        return run_c4(args)
+        return run_c4(args, dump_dir=args.dump_outputs)
     if args.config == "aux":
         return run_aux(args)
     run_ours(args)

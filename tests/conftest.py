@@ -29,12 +29,16 @@ def pytest_collection_modifyitems(config, items):
 
 
 def golden_ct_cases():
-    return sorted(os.path.basename(p)[:-4] for p in glob.glob(os.path.join(GOLDEN, "ct_*.npz")))
+    names = (os.path.basename(p)[:-4] for p in glob.glob(os.path.join(GOLDEN, "ct_*.npz")))
+    return sorted(n for n in names if "." not in n)   # <name>.<array>.npz is a part of <name> (load_golden)
 
 
 def load_golden(name):
-    z = np.load(os.path.join(GOLDEN, name + ".npz"))
-    d = {k: z[k] for k in z.files}
+    """The arrays of tests/golden/<name>.npz, and of <name>.<array>.npz beside it where a fixture over 1 MB is split."""
+    d = {}
+    for path in [os.path.join(GOLDEN, name + ".npz")] + sorted(glob.glob(os.path.join(GOLDEN, glob.escape(name) + ".*.npz"))):
+        z = np.load(path)
+        d.update({k: z[k] for k in z.files})
     if "params" in d:
         d["params"] = json.loads(str(d["params"]))
     return d

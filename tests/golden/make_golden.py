@@ -341,7 +341,11 @@ def make_config1_fixture():
     arrs = {f"in_{k}": v.numpy() for k, v in maps.items()}
     arrs.update(view=view.numpy(), lights=light.numpy(), intensity=inten.numpy(), out32=out.numpy(),
                 params=np.array(json.dumps(p)))
-    np.savez_compressed(os.path.join(HERE, "config1_tiles_256.npz"), **arrs)
+    # three files, none over 1 MB: the normal map and the output each in config1_tiles_256.<array>.npz
+    split = ("in_normal", "out32")
+    np.savez_compressed(os.path.join(HERE, "config1_tiles_256.npz"), **{k: v for k, v in arrs.items() if k not in split})
+    for k in split:
+        np.savez_compressed(os.path.join(HERE, f"config1_tiles_256.{k}.npz"), **{k: arrs[k]})
     print(f"config1_tiles_256: ok  mean {out.mean():.7f} min {out.min():.5f} max {out.max():.5f}")
 
 

@@ -1,14 +1,16 @@
 """
 pypbr_b200.io: folder loading / saving with the reference's naming conventions and workflow selection (pypbr/io.py:22-230).
-Host maps against the unmodified reference when it is on this machine; CUDA loading (8-bit bytes uploaded, converted by
-pbr_ingest_image) bit-equal to host loading.
+Host maps against a regression snapshot in tests/golden (recorded from this package's loader where it had been checked
+equal to the reference's); CUDA loading (8-bit bytes uploaded, converted by pbr_ingest_image) bit-equal to host loading.
 """
+import json
 import os
 import warnings
 
 import numpy as np
 import pytest
 import torch
+from conftest import load_golden
 from PIL import Image
 
 from pypbr_b200.io import load_material_from_folder, save_material_to_folder, select_material_class
@@ -87,27 +89,27 @@ def test_save_and_reload_round_trip(tmp_path):
     assert "albedo.png" in os.listdir(str(tmp_path / "out2"))
 
 
+REFERENCE_FOLDER_SEED = 3
+REFERENCE_WORKFLOWS = {"metallic": "metallic", "specular": "specular", "auto": None}   # fixture tag -> preferred_workflow
+
+
 def test_same_maps_as_the_reference(tmp_path):
-    from test_transforms import _reference
-
-    if _reference() is None:
-        pytest.skip("reference sources not on this machine")
-    from pypbr.io import load_material_from_folder as ref_load
-
-    folder = _write_folder(str(tmp_path), seed=3)
-    for pref in ("metallic", "specular", None):
+    """Against a regression snapshot of the maps loaded from _write_folder(seed=REFERENCE_FOLDER_SEED),
+    tests/golden/io_folder_24x40.npz: recorded from this package's loader at a commit where it had been checked equal to
+    the reference's loader (tests/golden/make_host_golden.py).  Not an independent comparison with the reference: a
+    snapshot re-recorded from this package carries no reference parity of its own."""
+    z = load_golden("io_folder_24x40")
+    meta = json.loads(str(z["meta"]))
+    folder = _write_folder(str(tmp_path), seed=REFERENCE_FOLDER_SEED)
+    for tag, pref in REFERENCE_WORKFLOWS.items():
         ours = _quiet(load_material_from_folder, folder, preferred_workflow=pref)
-        theirs = _quiet(ref_load, folder, preferred_workflow=pref)
-        assert type(ours).__name__ == type(theirs).__name__
-        assert set(ours._maps) == set(theirs._maps)
-        for k, t in theirs._maps.items():
+        theirs = meta[tag]
+        assert type(ours).__name__ == theirs["class"]
+        assert set(ours._maps) == set(theirs["maps"])
+        for k, present in theirs["maps"].items():
+            t = torch.from_numpy(z[f"{tag}_{k}"]) if present else None
             assert (t is None) == (ours._maps[k] is None) and (t is None or torch.equal(ours._maps[k], t)), (pref, k)
-        assert ours.albedo_is_srgb == theirs.albedo_is_srgb
-    data = "/root/reference/tests/data/tiles"
-    if os.path.isdir(data):
-        ours, theirs = _quiet(load_material_from_folder, data, preferred_workflow="metallic"), _quiet(ref_load, data, preferred_workflow="metallic")
-        for k, t in theirs._maps.items():
-            assert torch.equal(ours._maps[k], t), k
+        assert ours.albedo_is_srgb == theirs["albedo_is_srgb"]
 
 
 @pytest.mark.gpu

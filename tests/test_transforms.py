@@ -3,16 +3,16 @@ pypbr_b200.transforms against the reference's own test strategy (tests/test_tran
 sizes, flips equal tensor.flip, normal signs, colour round trip) - on CPU maps (the host branches of the material methods)
 and, marked gpu, on CUDA maps where every map of a material moves in one pbr_index_transform launch - plus what the
 reference's tests do not pin: the source material is never modified, the result never aliases it, seeded pipelines draw
-the same parameters as the reference, and (when the reference is present on this machine) the results are identical.
+the same parameters as the reference, and a seeded pipeline still gives the results stored in tests/golden (a regression
+snapshot of this package's host path, recorded where that path had been checked equal to the reference's; see
+tests/golden/make_host_golden.py).
 """
-import os
+import json
 import random
-import shutil
-import sys
-import tempfile
 
 import pytest
 import torch
+from conftest import load_golden
 
 from pypbr_b200.materials import BasecolorMetallicMaterial
 from pypbr_b200.transforms import (AdjustNormalStrength, CenterCrop, Compose, Crop, FlipHorizontal, FlipVertical, InvertNormal,
@@ -145,55 +145,39 @@ def test_functional_names_and_signatures_match_the_reference_interface():
         RandomRotate(padding_mode="edge")
 
 
-def _reference():
-    """The unmodified reference package, when this machine has it (the build container; never the GPU box)."""
-    root = "/root/reference/pypbr"
-    if not os.path.isdir(root):
-        return None
-    if "pypbr" not in sys.modules:
-        tmp = tempfile.mkdtemp(prefix="pypbr_ref_")
-        shutil.copytree(root, os.path.join(tmp, "pypbr"))
-        with open(os.path.join(tmp, "pypbr", "_version.py"), "w") as f:   # git-ignored file pypbr/__init__.py imports
-            f.write('__version__ = version = "0+reference"\n')
-        sys.path.insert(0, tmp)
-    import pypbr   # noqa: F401
+SEEDED_PIPELINE_SEED = 11
 
-    return sys.modules["pypbr"]
+
+def seeded_pipeline(T):
+    """The pipeline whose results on the maps of tests/golden/transforms_pipeline_24x40.npz are stored there, run after
+    random.seed(SEEDED_PIPELINE_SEED); `T` is the transforms module."""
+    return T.Compose([T.RandomCrop(16, 32), T.FlipHorizontal(), T.Roll((3, -5)), T.Tile(2), T.RandomResize(20, 30),
+                      T.RandomRotate(0.0, 90.0), T.FlipVertical(), T.InvertNormal(), T.CenterCrop(12, 12)])
 
 
 def test_same_results_as_the_reference_on_a_seeded_pipeline():
-    ref = _reference()
-    if ref is None:
-        pytest.skip("reference sources not on this machine")
-    import pypbr.transforms as RT
-    from pypbr.materials import BasecolorMetallicMaterial as RefMaterial
-
-    maps = _maps(H=24, W=40, seed=5)
-    ours = BasecolorMetallicMaterial(device=torch.device("cpu"))
-    theirs = RefMaterial()
-    for k, v in maps.items():
-        ours._maps[k] = v.clone()
-        theirs._maps[k] = v.clone()
-
-    def pipeline(T):
-        return T.Compose([T.RandomCrop(16, 32), T.FlipHorizontal(), T.Roll((3, -5)), T.Tile(2), T.RandomResize(20, 30),
-                          T.RandomRotate(0.0, 90.0), T.FlipVertical(), T.InvertNormal(), T.CenterCrop(12, 12)])
-
+    """Against a regression snapshot of the seeded pipeline: results recorded from this package's host path at a commit where
+    that path had been checked equal to the reference's (tests/golden/make_host_golden.py).  Not an independent comparison
+    with the reference: a snapshot re-recorded from this package carries no reference parity of its own."""
     import pypbr_b200.transforms as OT
 
-    random.seed(11)
-    a = pipeline(OT)(ours)
-    random.seed(11)
-    b = pipeline(RT)(theirs)
-    assert a.size == b.size
-    for k in maps:
+    z = load_golden("transforms_pipeline_24x40")
+    meta = json.loads(str(z["meta"]))
+    ours = BasecolorMetallicMaterial(device=torch.device("cpu"))
+    for k in meta["maps"]:
+        ours._maps[k] = torch.from_numpy(z["in_" + k])
+    random.seed(SEEDED_PIPELINE_SEED)
+    a = seeded_pipeline(OT)(ours)
+    assert list(a.size) == meta["size"]
+    for k in meta["maps"]:
+        want = torch.from_numpy(z["out_" + k])
         if k == "normal":
             # rotate_normals is a 2 x 2 matmul in the reference (utils/functions.py:98, BLAS: the FMA order is its own) -
             # the rotated vectors agree to an ulp, the resampling (which texel goes where) exactly
-            assert torch.allclose(a._maps[k], b._maps[k], rtol=0, atol=3e-7), k
+            assert torch.allclose(a._maps[k], want, rtol=0, atol=3e-7), k
         else:
-            assert torch.equal(a._maps[k], b._maps[k]), k
-    assert a.normal_convention.name == b.normal_convention.name
+            assert torch.equal(a._maps[k], want), k
+    assert a.normal_convention.name == meta["normal_convention"]
 
 
 # ------------------------------------------------------------------------------------------------------------ CUDA maps
