@@ -357,6 +357,14 @@ int pbr_ct_loss_fwd_bwd(const PbrCtDesc* desc, const PbrCtLoss* loss, const PbrC
 /* d_intensity: device, L*3, accumulated with atomics (caller zero-fills); may be NULL */
 int pbr_ct_fit_step(const PbrCtDesc* desc, const PbrCtLoss* loss, const PbrCtAdam* adam, float* d_intensity,
                     pbr_stream_t stream);
+/* Camera at a finite position: the same three calls with desc->view read as the camera POSITION c (same frame as a
+ * point light's position; host or device memory according to params_on_device) instead of the view direction.  Texel
+ * (i, j) sits at P = (x_j, -y_i, 0) on the plane of side s = light_size (> 0, else 1) - for both light types - and is
+ * shaded with the view vector F.normalize(c - P).  grads->d_view receives the gradient w.r.t. c.  force_generic and
+ * fwd_out are ignored; the argument checks and error codes are those of pbr_ct_forward / _backward / _loss_fwd_bwd. */
+int pbr_ct_forward_camera(const PbrCtDesc* desc, pbr_stream_t stream);
+int pbr_ct_backward_camera(const PbrCtDesc* desc, const PbrCtGrads* grads, pbr_stream_t stream);
+int pbr_ct_loss_fwd_bwd_camera(const PbrCtDesc* desc, const PbrCtLoss* loss, const PbrCtGrads* grads, pbr_stream_t stream);
 
 int pbr_convert_m2s(const PbrConvDesc* desc, pbr_stream_t stream);
 int pbr_convert_s2m(const PbrConvDesc* desc, pbr_stream_t stream);

@@ -187,6 +187,7 @@ EXPORTS = (
     "pbr_convert_m2s", "pbr_convert_s2m", "pbr_blend", "pbr_color_convert", "pbr_normal_min",
     "pbr_normal_ingest", "pbr_ingest_image", "pbr_index_transform", "pbr_adam_step", "pbr_normal_op", "pbr_launch_count", "pbr_sizeof",
     "pbr_convert_m2s_backward", "pbr_convert_s2m_backward", "pbr_blend_backward", "pbr_normal_ingest_backward",
+    "pbr_ct_forward_camera", "pbr_ct_backward_camera", "pbr_ct_loss_fwd_bwd_camera",
 )
 
 
@@ -216,6 +217,9 @@ def load():
     lib.pbr_ct_backward.argtypes = [POINTER(PbrCtDesc), POINTER(PbrCtGrads), c_void_p]
     lib.pbr_ct_loss_fwd_bwd.argtypes = [POINTER(PbrCtDesc), POINTER(PbrCtLoss), POINTER(PbrCtGrads), c_void_p]
     lib.pbr_ct_fit_step.argtypes = [POINTER(PbrCtDesc), POINTER(PbrCtLoss), POINTER(PbrCtAdam), c_void_p, c_void_p]
+    lib.pbr_ct_forward_camera.argtypes = [POINTER(PbrCtDesc), c_void_p]
+    lib.pbr_ct_backward_camera.argtypes = [POINTER(PbrCtDesc), POINTER(PbrCtGrads), c_void_p]
+    lib.pbr_ct_loss_fwd_bwd_camera.argtypes = [POINTER(PbrCtDesc), POINTER(PbrCtLoss), POINTER(PbrCtGrads), c_void_p]
     lib.pbr_convert_m2s.argtypes = [POINTER(PbrConvDesc), c_void_p]
     lib.pbr_convert_s2m.argtypes = [POINTER(PbrConvDesc), c_void_p]
     lib.pbr_blend.argtypes = [POINTER(PbrBlendDesc), c_void_p]

@@ -940,6 +940,183 @@ __global__ void __launch_bounds__(kCtThreads, kGeom ? 2 : bwd_min_ctas(kLight)) 
   }
 }
 
+// ------------------------------------------------------------------------------------------------
+// Camera at a finite position (pbr_ct_*_camera): the view vector of a texel is F.normalize(c - P) with c = PbrCtDesc.view
+// and P = (x, -y, 0) its plane position, instead of the one CTA-uniform direction of the ct_* kernels.
+// The design of the generic kernels: V = f2, kCtThreads threads, a walk over up to kHoistMats materials, element-access
+// loads and stores (any alignment and width).  The view vectors - and, for one point light, its geometry - are computed
+// once per texel and reused by every material of the walk (they do not depend on the material).  Light modes:
+// kLightDirectional (l is image-constant, h and (1 - h.v)^5 per texel), kLightPointHoisted (L == 1) and kLightPoint.
+// The backward always computes the geometry adjoints (the camera gradient runs through h, N.V and the Fresnel term).
+// ------------------------------------------------------------------------------------------------
+template <int kLight>
+__device__ __forceinline__ void cam_setup(const CtKParams& p, const CtStage& S, const Where& w, V (&x)[kSlots], float& y,
+                                          LaneViews<V, kSlots>& cv, LightGeomT<V> (&hg)[kSlots]) {
+  GeomCache<V> gc;
+  grid_coords<kLightPoint>(S, w, p.flags.L, x, y, hg, gc);   // the plane coordinates only
+  const float* cam = p.view_dev ? p.view_dev : p.view;
+  const float c[3] = {cam[0], cam[1], cam[2]};
+#pragma unroll
+  for (int i = 0; i < kSlots; ++i) {
+    camera_view(c, x[i], y, cv.x[i], cv.y[i], cv.z[i], cv.len[i]);
+    if (kLight == kLightPointHoisted)
+      point_light_geom(S.light[0].p[0], S.light[0].p[1], S.light[0].p[2], x[i], y, cv.x[i], cv.y[i], cv.z[i], hg[i]);
+  }
+}
+
+template <int WF, int kLight>
+__global__ void __launch_bounds__(kCtThreads, PBR_FWD_MIN_CTAS) cam_forward_kernel(const __grid_constant__ CtKParams p) {
+  __shared__ CtStage S;
+  stage_params(p, S);
+  const Where w = locate_ct<false>(p);
+  if (!w.active) return;
+  const CtFlags& F = p.flags;
+  const bool has_normal = p.normal.ptr != nullptr;
+  V x[kSlots];
+  float y;
+  LaneViews<V, kSlots> cv;
+  LightGeomT<V> hg[kSlots];
+  cam_setup<kLight>(p, S, w, x, y, cv, hg);
+
+  const int b0 = blockIdx.z * p.mats_per_cta;
+  const int b1 = min(b0 + p.mats_per_cta, p.B);
+  for (int b = b0; b < b1; ++b) {
+    float araw[3][kCtTexels], nraw[3][kCtTexels], rough[kCtTexels], mraw[3][kCtTexels];
+    load_material<WF, false>(p, w, b, araw, nraw, rough, mraw, has_normal);
+    if (b + 1 < b1) prefetch_material<WF, false>(p, w, b + 1, has_normal);
+    V a[3][kSlots], n[3][kSlots], r[kSlots], m[3][kSlots];
+    pairs_of3<kSlots>(araw, 0, a); pairs_of3<kSlots>(nraw, 0, n); pairs_of3<kSlots>(mraw, 0, m); pairs_of<kSlots>(rough, 0, r);
+    auto emit = [&](int l, const V(&v)[3][kSlots]) {   // light l (per-light mode) or the accumulated image (l = 0)
+#pragma unroll
+      for (int c = 0; c < 3; ++c) {
+        float tv[kCtTexels];
+        unpair_to<kSlots>(v[c], 0, tv);
+        store_seg<kCtTexels>(at<false>(p.out, b, c, w) + (F.per_light ? (int64_t)l * p.out_sl : 0), w.vec, w.valid, tv);
+      }
+    };
+    ct_forward_group<WF, kLight, V, kSlots, decltype(emit), kFwdUnroll, LaneViews<V, kSlots>>(S, F, a, n, r, m, x, y, hg, emit,
+                                                                                                GeomCache<V>(), cv);
+  }
+}
+
+// Backward / fused loss (p.is_loss), with d_intensity, d_lights and d_view (= d camera position) when their pointers are
+// set.  Accumulate mode with L > 1 runs the two-pass backward (the summed image is recomputed).  The shared-parameter
+// gradients go warp shuffle -> shared atomics per light, and one global atomic per CTA and value.
+template <int WF, int kLight>
+__global__ void __launch_bounds__(kCtThreads, 2) cam_backward_kernel(const __grid_constant__ CtKParams p) {
+  __shared__ CtStage S;
+  __shared__ float s_int[PBR_MAX_LIGHTS * 3];
+  __shared__ float s_geo[(PBR_MAX_LIGHTS + 1) * 3];
+  __shared__ float s_loss[kCtThreads / 32];
+  const int tid = threadIdx.y * blockDim.x + threadIdx.x;
+  const CtFlags& F = p.flags;
+  const bool int_grad = p.d_intensity != nullptr;
+  const bool is_loss = p.is_loss != 0;
+  const bool has_normal = p.normal.ptr != nullptr;
+  for (int i = tid; i < F.L * 3; i += kCtThreads) s_int[i] = 0.0f;
+  for (int i = tid; i < (F.L + 1) * 3; i += kCtThreads) s_geo[i] = 0.0f;
+  stage_params(p, S);  // ends with __syncthreads()
+  const Where w = locate_ct<false>(p);
+  const float live = w.active ? 1.0f : 0.0f;   // edge threads stay for the warp-wide reductions
+
+  V x[kSlots];
+  float y;
+  LaneViews<V, kSlots> cv;
+  LightGeomT<V> hg[kSlots];
+  cam_setup<kLight>(p, S, w, x, y, cv, hg);
+
+  float loss_local = 0.0f;
+  const int b0 = blockIdx.z * p.mats_per_cta;
+  const int b1 = min(b0 + p.mats_per_cta, p.B);
+  for (int b = b0; b < b1; ++b) {
+    float araw[3][kCtTexels], nraw[3][kCtTexels], rough[kCtTexels], mraw[3][kCtTexels];
+    load_material<WF, false>(p, w, b, araw, nraw, rough, mraw, has_normal);
+    if (b + 1 < b1) prefetch_material<WF, false>(p, w, b + 1, has_normal);
+    V a[3][kSlots], n[3][kSlots], r[kSlots], m[3][kSlots];
+    pairs_of3<kSlots>(araw, 0, a); pairs_of3<kSlots>(nraw, 0, n); pairs_of3<kSlots>(mraw, 0, m); pairs_of<kSlots>(rough, 0, r);
+    // dLoss/d out of light l (per-light mode) or of the accumulated image: grad_out, or 2 * loss_scale * (out - target)
+    auto gout = [&](int l, const V(&outv)[3][kSlots], V(&g)[3][kSlots]) {
+#pragma unroll
+      for (int c = 0; c < 3; ++c) {
+        float src[kCtTexels], ov[kCtTexels], gv[kCtTexels];
+        load_seg<kCtTexels>(at<false>(p.gsrc, b, c, w) + (F.per_light ? (int64_t)l * p.gsrc_sl : 0), w.vec, w.valid, src);
+        unpair_to<kSlots>(outv[c], 0, ov);
+#pragma unroll
+        for (int i = 0; i < kCtTexels; ++i) {
+          if (is_loss) {
+            const float diff = (i < w.valid) ? ov[i] - src[i] : 0.0f;
+            loss_local += diff * diff;
+            gv[i] = 2.0f * p.loss_scale * diff;
+          } else {
+            gv[i] = (i < w.valid) ? src[i] : 0.0f;
+          }
+        }
+        pairs_of<kSlots>(gv, 0, g[c]);
+      }
+    };
+    auto int_sink = [&](int l, const float(&gi)[3]) {
+#pragma unroll
+      for (int c = 0; c < 3; ++c) {
+        const float sum = warp_sum(gi[c] * live);
+        if ((tid & 31) == 0) atomicAdd(&s_int[3 * l + c], sum);
+      }
+    };
+    V da[3][kSlots], dn[3][kSlots], dr[kSlots], dm[3][kSlots];
+    ct_backward_group<WF, kLight, V, kSlots, decltype(gout), decltype(int_sink), NoFetch, CtaGeomSink, NoSavedOut, kBwdUnroll,
+                      LaneViews<V, kSlots>>(S, F, a, n, r, m, x, y, hg, gout, int_sink, da, dn, dr, dm, NoFetch(), GeomCache<V>(),
+                                            CtaGeomSink{s_geo, F.L, tid, live, nullptr}, NoSavedOut(), int_grad, cv);
+    if (w.active) {
+      float d_albedo[3][kCtTexels], d_normal[3][kCtTexels], d_rough[kCtTexels], d_met[3][kCtTexels];
+#pragma unroll
+      for (int c = 0; c < 3; ++c) { unpair_to<kSlots>(da[c], 0, d_albedo[c]); unpair_to<kSlots>(dn[c], 0, d_normal[c]); unpair_to<kSlots>(dm[c], 0, d_met[c]); }
+      unpair_to<kSlots>(dr, 0, d_rough);
+      if (p.d_albedo.ptr) {
+#pragma unroll
+        for (int c = 0; c < 3; ++c) store_seg<kCtTexels>(at<false>(p.d_albedo, b, c, w), w.vec, w.valid, d_albedo[c]);
+      }
+      if (has_normal && p.d_normal.ptr) {
+#pragma unroll
+        for (int c = 0; c < 3; ++c) store_seg<kCtTexels>(at<false>(p.d_normal, b, c, w), w.vec, w.valid, d_normal[c]);
+      }
+      if (p.d_roughness.ptr) store_seg<kCtTexels>(at<false>(p.d_roughness, b, 0, w), w.vec, w.valid, d_rough);
+      if (p.d_metspec.ptr) {
+#pragma unroll
+        for (int c = 0; c < (WF == 0 ? 1 : 3); ++c) store_seg<kCtTexels>(at<false>(p.d_metspec, b, c, w), w.vec, w.valid, d_met[c]);
+      }
+    }
+  }
+
+  if (is_loss) {
+    const float sum = warp_sum(loss_local * live);
+    if ((tid & 31) == 0) s_loss[tid >> 5] = sum;
+  }
+  __syncthreads();
+  if (tid <= F.L) {
+    // the camera sum is already d/d c (camera_view_bwd per texel); a directional light's sum is w.r.t. its UNIT
+    // direction, whose Jacobian is image-constant and applied here, once
+    const float g[3] = {s_geo[3 * tid], s_geo[3 * tid + 1], s_geo[3 * tid + 2]};
+    float o[3] = {g[0], g[1], g[2]};
+    float* dst = p.d_view;
+    if (tid < F.L) {
+      const float* lights = p.lights_dev ? p.lights_dev : p.lights;
+      if (!F.point) normalize_bwd(lights + 3 * tid, g, o);
+      dst = p.d_lights ? p.d_lights + 3 * tid : nullptr;
+    }
+    if (dst) {
+#pragma unroll
+      for (int c = 0; c < 3; ++c) atomicAdd(dst + c, o[c]);
+    }
+  }
+  if (is_loss && tid == 0) {
+    float sum = 0.0f;
+    for (int i = 0; i < kCtThreads / 32; ++i) sum += s_loss[i];
+    atomicAdd(p.loss_sum, sum);
+  }
+  if (int_grad) {
+    for (int i = tid; i < F.L * 3; i += kCtThreads) atomicAdd(&p.d_intensity[i], s_int[i]);
+  }
+}
+
 }  // namespace pbr
 
 #include "pbr_ct_stream.cuh"
@@ -1520,6 +1697,38 @@ void launch_wf1(CtKParams& k, dim3 grid, dim3 block, bool stream, bool backward,
 void launch_wf2(CtKParams& k, dim3 grid, dim3 block, bool stream, bool backward, cudaStream_t st) { launch_wf<2>(k, grid, block, stream, backward, st); }
 #endif
 
+// the camera kernels of one workflow (pbr_ct_*_camera): directional lights, one point light (hoisted), several point lights
+template <int WF>
+static void launch_cam(const CtKParams& k, dim3 grid, dim3 block, bool backward, cudaStream_t st) {
+  const int lm = !k.flags.point ? kLightDirectional : (k.flags.L == 1 ? kLightPointHoisted : kLightPoint);
+  switch (lm) {
+    case kLightDirectional:
+      if (backward) cam_backward_kernel<WF, kLightDirectional><<<grid, block, 0, st>>>(k);
+      else cam_forward_kernel<WF, kLightDirectional><<<grid, block, 0, st>>>(k);
+      break;
+    case kLightPointHoisted:
+      if (backward) cam_backward_kernel<WF, kLightPointHoisted><<<grid, block, 0, st>>>(k);
+      else cam_forward_kernel<WF, kLightPointHoisted><<<grid, block, 0, st>>>(k);
+      break;
+    default:
+      if (backward) cam_backward_kernel<WF, kLightPoint><<<grid, block, 0, st>>>(k);
+      else cam_forward_kernel<WF, kLightPoint><<<grid, block, 0, st>>>(k);
+      break;
+  }
+}
+void launch_cam_wf0(const CtKParams& k, dim3 grid, dim3 block, bool backward, cudaStream_t st);
+void launch_cam_wf1(const CtKParams& k, dim3 grid, dim3 block, bool backward, cudaStream_t st);
+void launch_cam_wf2(const CtKParams& k, dim3 grid, dim3 block, bool backward, cudaStream_t st);
+#if PBR_HAS_WF(0)
+void launch_cam_wf0(const CtKParams& k, dim3 grid, dim3 block, bool backward, cudaStream_t st) { launch_cam<0>(k, grid, block, backward, st); }
+#endif
+#if PBR_HAS_WF(1)
+void launch_cam_wf1(const CtKParams& k, dim3 grid, dim3 block, bool backward, cudaStream_t st) { launch_cam<1>(k, grid, block, backward, st); }
+#endif
+#if PBR_HAS_WF(2)
+void launch_cam_wf2(const CtKParams& k, dim3 grid, dim3 block, bool backward, cudaStream_t st) { launch_cam<2>(k, grid, block, backward, st); }
+#endif
+
 #if PBR_MAIN_PART
 // shared tail of the three Cook-Torrance entry points
 // every in-plane offset (row * sh + col) of a plane fits 32 bits
@@ -1549,6 +1758,24 @@ static int ct_dispatch(CtKParams& k, int wf, bool backward, cudaStream_t st) {
     default: launch_wf2(k, grid, block, stream, backward, st); break;
   }
   return launch_result();
+}
+
+// the same for the camera kernels: every material walk spans up to kHoistMats materials (the views are per texel)
+static int cam_dispatch(CtKParams& k, int wf, bool backward, cudaStream_t st) {
+  dim3 grid, block;
+  launch_shape(k.B, k.H, k.W, grid, block, kCtThreads, kCtTexels);
+  k.mats_per_cta = k.B < kHoistMats ? k.B : kHoistMats;
+  grid.z = (k.B + k.mats_per_cta - 1) / k.mats_per_cta;
+  switch (wf) {
+    case 0: launch_cam_wf0(k, grid, block, backward, st); break;
+    case 1: launch_cam_wf1(k, grid, block, backward, st); break;
+    default: launch_cam_wf2(k, grid, block, backward, st); break;
+  }
+  return launch_result();
+}
+
+static int dispatch(CtKParams& k, int wf, bool backward, bool camera, cudaStream_t st) {
+  return camera ? cam_dispatch(k, wf, backward, st) : ct_dispatch(k, wf, backward, st);
 }
 #endif   // PBR_MAIN_PART
 
@@ -1601,15 +1828,16 @@ uint64_t pbr_sizeof(int which) {
 
 uint64_t pbr_launch_count(void) { return g_launches.load(std::memory_order_relaxed); }
 
-int pbr_ct_forward(const PbrCtDesc* desc, pbr_stream_t stream) {
+// camera: desc->view is the camera position (cam_* kernels) instead of the view direction (ct_* kernels)
+static int ct_forward(const PbrCtDesc* desc, bool camera, pbr_stream_t stream) {
   CtKParams k{};
   if (int rc = fill_ct_params(desc, k)) return rc;
   if (!desc->out.ptr) return PBR_E_NULL;
   k.vec_ok = k.vec_ok && plane_vec_ok(desc->out) && (desc->out_sl % kTexels == 0);
-  return ct_dispatch(k, kernel_workflow(desc), false, (cudaStream_t)stream);
+  return dispatch(k, kernel_workflow(desc), false, camera, (cudaStream_t)stream);
 }
 
-int pbr_ct_backward(const PbrCtDesc* desc, const PbrCtGrads* grads, pbr_stream_t stream) {
+static int ct_backward(const PbrCtDesc* desc, const PbrCtGrads* grads, bool camera, pbr_stream_t stream) {
   CtKParams k{};
   if (int rc = fill_ct_params(desc, k)) return rc;
   if (int rc = fill_grads(grads, k)) return rc;
@@ -1617,14 +1845,15 @@ int pbr_ct_backward(const PbrCtDesc* desc, const PbrCtGrads* grads, pbr_stream_t
   k.gsrc = grads->grad_out; k.gsrc_sl = grads->grad_out_sl;
   k.is_loss = 0;
   k.vec_ok = k.vec_ok && plane_vec_ok(grads->grad_out) && (grads->grad_out_sl % kTexels == 0);
-  if (!desc->per_light && desc->L > 1) {   // only the accumulate-mode backward of several lights has a use for it
+  if (!camera && !desc->per_light && desc->L > 1) {   // only the accumulate-mode backward of several lights has a use for it
     k.fout = grads->fwd_out;
     k.vec_ok = k.vec_ok && plane_vec_ok(grads->fwd_out);
   }
-  return ct_dispatch(k, kernel_workflow(desc), true, (cudaStream_t)stream);
+  return dispatch(k, kernel_workflow(desc), true, camera, (cudaStream_t)stream);
 }
 
-int pbr_ct_loss_fwd_bwd(const PbrCtDesc* desc, const PbrCtLoss* loss, const PbrCtGrads* grads, pbr_stream_t stream) {
+static int ct_loss_fwd_bwd(const PbrCtDesc* desc, const PbrCtLoss* loss, const PbrCtGrads* grads, bool camera,
+                           pbr_stream_t stream) {
   CtKParams k{};
   if (int rc = fill_ct_params(desc, k)) return rc;
   if (int rc = fill_grads(grads, k)) return rc;
@@ -1633,7 +1862,20 @@ int pbr_ct_loss_fwd_bwd(const PbrCtDesc* desc, const PbrCtLoss* loss, const PbrC
   k.is_loss = 1;
   k.loss_scale = loss->loss_scale; k.loss_sum = loss->loss_sum;
   k.vec_ok = k.vec_ok && plane_vec_ok(loss->target) && (loss->target_sl % kTexels == 0);
-  return ct_dispatch(k, kernel_workflow(desc), true, (cudaStream_t)stream);
+  return dispatch(k, kernel_workflow(desc), true, camera, (cudaStream_t)stream);
+}
+
+int pbr_ct_forward(const PbrCtDesc* desc, pbr_stream_t stream) { return ct_forward(desc, false, stream); }
+int pbr_ct_backward(const PbrCtDesc* desc, const PbrCtGrads* grads, pbr_stream_t stream) { return ct_backward(desc, grads, false, stream); }
+int pbr_ct_loss_fwd_bwd(const PbrCtDesc* desc, const PbrCtLoss* loss, const PbrCtGrads* grads, pbr_stream_t stream) {
+  return ct_loss_fwd_bwd(desc, loss, grads, false, stream);
+}
+int pbr_ct_forward_camera(const PbrCtDesc* desc, pbr_stream_t stream) { return ct_forward(desc, true, stream); }
+int pbr_ct_backward_camera(const PbrCtDesc* desc, const PbrCtGrads* grads, pbr_stream_t stream) {
+  return ct_backward(desc, grads, true, stream);
+}
+int pbr_ct_loss_fwd_bwd_camera(const PbrCtDesc* desc, const PbrCtLoss* loss, const PbrCtGrads* grads, pbr_stream_t stream) {
+  return ct_loss_fwd_bwd(desc, loss, grads, true, stream);
 }
 
 int pbr_ct_fit_step(const PbrCtDesc* desc, const PbrCtLoss* loss, const PbrCtAdam* adam, float* d_intensity,

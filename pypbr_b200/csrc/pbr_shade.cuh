@@ -152,17 +152,47 @@ PBR_HD void geom_cache_load(const GeomCache<V>& gc, int l, int i, const float p[
   }
 }
 
-template <int kLight, class V, int N>
+// The view direction the group functions below shade with (template parameter View):
+//   OrthoView : the CTA-uniform unit vector staged in CtStage (S.vx, S.vy, S.vz), the orthographic camera of the
+//               reference - every ct_* kernel;
+//   LaneViews : a camera at a finite position - the unit view vector of every lane-value and |c - P| for its adjoint
+//               (camera_view in pbr_math.cuh), computed once per texel by the cam_* kernels.
+struct OrthoView {};
+template <class V, int N>
+struct LaneViews {
+  V x[N], y[N], z[N], len[N];
+};
+PBR_HD float view_x(const CtStage& S, const OrthoView&, int) { return S.vx; }
+PBR_HD float view_y(const CtStage& S, const OrthoView&, int) { return S.vy; }
+PBR_HD float view_z(const CtStage& S, const OrthoView&, int) { return S.vz; }
+template <class V, int N> PBR_HD V view_x(const CtStage&, const LaneViews<V, N>& v, int i) { return v.x[i]; }
+template <class V, int N> PBR_HD V view_y(const CtStage&, const LaneViews<V, N>& v, int i) { return v.y[i]; }
+template <class V, int N> PBR_HD V view_z(const CtStage&, const LaneViews<V, N>& v, int i) { return v.z[i]; }
+// directional light: l is image-constant, but with a per-texel view the half vector and (1 - h.v)^5 are per texel too
+template <class V> PBR_HD void dir_view_geom(const OrthoView&, int, LightGeomT<V>&) {}
+template <class V, int N> PBR_HD void dir_view_geom(const LaneViews<V, N>& v, int i, LightGeomT<V>& g) {
+  half_vector(v.x[i], v.y[i], v.z[i], g);
+}
+// d/d unit view vector of lane-value i -> d/d camera position (in place); the orthographic view's Jacobian is applied
+// once per CTA by the caller instead (it is image-constant)
+template <class V> PBR_HD void view_bwd(const OrthoView&, int, V*) {}
+template <class V, int N> PBR_HD void view_bwd(const LaneViews<V, N>& v, int i, V* g) {
+  camera_view_bwd(v.x[i], v.y[i], v.z[i], v.len[i], g);
+}
+
+template <int kLight, class V, int N, class View = OrthoView>
 PBR_HD void light_geom(const CtStage& S, int l, const V (&x)[N], float y, const LightGeomT<V> (&hoisted)[N], int i,
-                       const GeomCache<V>& gc, LightGeomT<V>& g) {
-  if (is_cached(kLight)) {
+                       const GeomCache<V>& gc, LightGeomT<V>& g, const View& view = View()) {
+  if (is_cached(kLight)) {   // (orthographic view only)
     geom_cache_load<geom_fields(kLight), V>(gc, l, i, S.light[l].p, x[i], y, S.vx, S.vy, S.vz, g);
   } else if (kLight == kLightPoint) {
-    point_light_geom(S.light[l].p[0], S.light[l].p[1], S.light[l].p[2], x[i], y, S.vx, S.vy, S.vz, g);
+    point_light_geom(S.light[l].p[0], S.light[l].p[1], S.light[l].p[2], x[i], y, view_x(S, view, i), view_y(S, view, i),
+                     view_z(S, view, i), g);
   } else if (kLight == kLightPointHoisted) {
     g = hoisted[i];
   } else {
     g = splat_geom<V>(S.light[l].geom);
+    dir_view_geom(view, i, g);
   }
 }
 
@@ -191,17 +221,19 @@ PBR_HD V encode_out_d(V c, bool return_srgb, V* d) {
 // forward: N lane-values of one row.  emit(l, out[3][N]) receives the encoded colour of light l
 // (per-light mode) or, once, of the accumulated image (l = 0).
 // ------------------------------------------------------------------------------------------------
-template <int kWorkflow, int kLight, class V, int N, class Emit, int kUnroll = kFwdUnroll>
+template <int kWorkflow, int kLight, class V, int N, class Emit, int kUnroll = kFwdUnroll, class View = OrthoView>
 PBR_HD void ct_forward_group(const CtStage& S, const CtFlags& F, const V (&araw)[3][N], const V (&nraw)[3][N],
                              const V (&rough)[N], const V (&mraw)[3][N], const V (&x)[N], float y,
-                             const LightGeomT<V> (&hoisted)[N], Emit emit, GeomCache<V> gc = GeomCache<V>()) {
+                             const LightGeomT<V> (&hoisted)[N], Emit emit, GeomCache<V> gc = GeomCache<V>(),
+                             const View& view = View()) {
   Texel<kWorkflow, V> t[N];
 #pragma unroll
   for (int i = 0; i < N; ++i) {
     const V a3[3] = {araw[0][i], araw[1][i], araw[2][i]};
     const V n3[3] = {nraw[0][i], nraw[1][i], nraw[2][i]};
     const V m3[3] = {mraw[0][i], mraw[1][i], mraw[2][i]};
-    texel_setup<kWorkflow, false>(a3, n3, rough[i], m3, F.albedo_is_srgb, F.specular_is_srgb, S.vx, S.vy, S.vz, t[i]);
+    texel_setup<kWorkflow, false>(a3, n3, rough[i], m3, F.albedo_is_srgb, F.specular_is_srgb, view_x(S, view, i),
+                                  view_y(S, view, i), view_z(S, view, i), t[i]);
   }
   V acc[3][N];
 #pragma unroll
@@ -216,7 +248,7 @@ PBR_HD void ct_forward_group(const CtStage& S, const CtFlags& F, const V (&araw)
 #pragma unroll
     for (int i = 0; i < N; ++i) {
       LightGeomT<V> g;
-      light_geom<kLight, V, N>(S, l, x, y, hoisted, i, gc, g);
+      light_geom<kLight, V, N>(S, l, x, y, hoisted, i, gc, g, view);
       LightFwd<V> f;
       V col[3];
       shade_light_fwd<kWorkflow, false>(t[i], g, S.light[l].inten, f, col);
@@ -256,7 +288,8 @@ struct NoFetch {
 };
 //   geom_sink.light(l, g[3])    : (GeomSink != NoGeomSink only) gradient w.r.t. the position of point light l, or
 //        w.r.t. the UNIT direction of directional light l, summed over the texels of the group;
-//   geom_sink.view(g[3])        : gradient w.r.t. the UNIT view direction, summed over the group's texels and lights.
+//   geom_sink.view(g[3])        : gradient w.r.t. the UNIT view direction (OrthoView) or w.r.t. the camera position
+//        (LaneViews), summed over the group's texels and lights.
 struct NoGeomSink {
   static constexpr bool kOn = false;
   PBR_HD void light(int, const float (&)[3]) const {}
@@ -291,16 +324,17 @@ PBR_HD V encode_slope_from_out(V out, bool return_srgb) {
 }
 
 template <int kWorkflow, int kLight, class V, int N, class Gout, class IntSink, class Fetch = NoFetch,
-          class GeomSink = NoGeomSink, class SavedOut = NoSavedOut, int kUnroll = kBwdUnroll>
+          class GeomSink = NoGeomSink, class SavedOut = NoSavedOut, int kUnroll = kBwdUnroll, class View = OrthoView>
 PBR_HD void ct_backward_group(const CtStage& S, const CtFlags& F, const V (&araw)[3][N], const V (&nraw)[3][N],
                               const V (&rough)[N], const V (&mraw)[3][N], const V (&x)[N], float y,
                               const LightGeomT<V> (&hoisted)[N], Gout gout, IntSink int_sink, V (&d_albedo)[3][N],
                               V (&d_normal)[3][N], V (&d_rough)[N], V (&d_met)[3][N], Fetch fetch = Fetch(),
                               GeomCache<V> gc = GeomCache<V>(), GeomSink geom_sink = GeomSink(),
-                              SavedOut saved_out = SavedOut(), bool want_int = true) {
+                              SavedOut saved_out = SavedOut(), bool want_int = true, const View& view = View()) {
   constexpr bool kGeom = GeomSink::kOn;
-  static_assert(!kGeom || kLight == kLightDirectional || kLight == kLightPoint || kLight == kLightPointCached,
-                "geometry gradients: directional, per-texel point lights, or the 6-field geometry cache");
+  static_assert(!kGeom || kLight == kLightDirectional || kLight == kLightPoint || kLight == kLightPointHoisted ||
+                    kLight == kLightPointCached,
+                "geometry gradients: directional, per-texel or hoisted point lights, or the 6-field geometry cache");
   V g_view[kGeom ? N : 1][3];
   if (kGeom) {
 #pragma unroll
@@ -313,7 +347,8 @@ PBR_HD void ct_backward_group(const CtStage& S, const CtFlags& F, const V (&araw
     const V a3[3] = {araw[0][i], araw[1][i], araw[2][i]};
     const V n3[3] = {nraw[0][i], nraw[1][i], nraw[2][i]};
     const V m3[3] = {mraw[0][i], mraw[1][i], mraw[2][i]};
-    texel_setup<kWorkflow, true>(a3, n3, rough[i], m3, F.albedo_is_srgb, F.specular_is_srgb, S.vx, S.vy, S.vz, t[i]);
+    texel_setup<kWorkflow, true>(a3, n3, rough[i], m3, F.albedo_is_srgb, F.specular_is_srgb, view_x(S, view, i),
+                                 view_y(S, view, i), view_z(S, view, i), t[i]);
     texel_grad_zero(tg[i]);
   }
 
@@ -351,7 +386,7 @@ PBR_HD void ct_backward_group(const CtStage& S, const CtFlags& F, const V (&araw
 #pragma unroll
         for (int i = 0; i < N; ++i) {
           LightGeomT<V> g;
-          light_geom<kLight, V, N>(S, l, x, y, hoisted, i, gc, g);
+          light_geom<kLight, V, N>(S, l, x, y, hoisted, i, gc, g, view);
           LightFwd<V> f;
           V col[3];
           shade_light_fwd<kWorkflow, false>(t[i], g, S.light[l].inten, f, col);
@@ -386,7 +421,7 @@ PBR_HD void ct_backward_group(const CtStage& S, const CtFlags& F, const V (&araw
     V outv[3][N], slope[3][N], gl[3][N];
 #pragma unroll
     for (int i = 0; i < N; ++i) {
-      light_geom<kLight, V, N>(S, l, x, y, hoisted, i, gc, g[i]);
+      light_geom<kLight, V, N>(S, l, x, y, hoisted, i, gc, g[i], view);
       V col[3];
       shade_light_fwd<kWorkflow>(t[i], g[i], S.light[l].inten, f[i], col);
       if (!two_pass) {
@@ -416,7 +451,8 @@ PBR_HD void ct_backward_group(const CtStage& S, const CtFlags& F, const V (&araw
       }
       if (kGeom) {
         V glt[3];
-        light_geom_bwd<kLight != kLightDirectional>(g[i], gg, S.light[l].p, x[i], y, S.vx, S.vy, S.vz, glt, g_view[i]);
+        light_geom_bwd<kLight != kLightDirectional>(g[i], gg, S.light[l].p, x[i], y, view_x(S, view, i), view_y(S, view, i),
+                                                    view_z(S, view, i), glt, g_view[i]);
 #pragma unroll
         for (int c = 0; c < 3; ++c) glt_sum[c] += lane_sum(glt[c]);
       }
@@ -429,7 +465,8 @@ PBR_HD void ct_backward_group(const CtStage& S, const CtFlags& F, const V (&araw
 #pragma unroll
   for (int i = 0; i < N; ++i) {
     V da[3], dn[3], dm[3], dr, g_ndv;
-    texel_finish_grad<kWorkflow>(t[i], tg[i], rough[i], S.vx, S.vy, S.vz, da, dn, &dr, dm, kGeom ? &g_ndv : nullptr);
+    texel_finish_grad<kWorkflow>(t[i], tg[i], rough[i], view_x(S, view, i), view_y(S, view, i), view_z(S, view, i), da, dn,
+                                 &dr, dm, kGeom ? &g_ndv : nullptr);
     if (kGeom) {
       g_view[i][0] += g_ndv * t[i].nx; g_view[i][1] += g_ndv * t[i].ny; g_view[i][2] += g_ndv * t[i].nz;
     }
@@ -444,9 +481,11 @@ PBR_HD void ct_backward_group(const CtStage& S, const CtFlags& F, const V (&araw
   if (kGeom) {
     float gv[3] = {0.0f, 0.0f, 0.0f};
 #pragma unroll
-    for (int i = 0; i < N; ++i)
+    for (int i = 0; i < N; ++i) {
+      view_bwd(view, i, g_view[i]);
 #pragma unroll
       for (int c = 0; c < 3; ++c) gv[c] += lane_sum(g_view[i][c]);
+    }
     geom_sink.view(gv);
   }
 }

@@ -23,7 +23,7 @@ import torch.nn as nn
 
 from . import _cabi
 from .materials import MaterialBase
-from .models.cooktorrance import _fill_desc, _out_plane, _prepare
+from .models.cooktorrance import _fill_desc, _out_plane, _prepare, check_view_type
 
 
 def shard_range(total: int, rank: int, world: int) -> Tuple[int, int]:
@@ -49,6 +49,7 @@ def fused_loss_step(
     want_geometry_grad: bool = False,
     want_map_grads: bool = True,
     device=None,
+    view_type: str = "directional",
 ):
     """
     One fused forward + MSE + backward pass over a (batched) material.
@@ -61,13 +62,15 @@ def fused_loss_step(
          parameters of a fit with unknown lighting); buf then has 1 + 6L + 3 floats.
     want_map_grads: False -> loss (and shared-parameter gradients) only: no gradient buffer is allocated or written.
     device: where to shade (default material.device; maps living elsewhere are moved, like CookTorranceBRDF's override_device).
+    view_type: as CookTorranceBRDF's; "point" reads view_dir as the camera position, and the last 3 floats of buf (with
+         want_geometry_grad) are then the gradient w.r.t. that position.
     Returns (buf, grads): buf is a device tensor [loss_sum, d_intensity(L*3)..., (d_lights(L*3)..., d_view(3))]
     (loss_sum is the UNscaled sum of squared errors; multiply by loss_scale for the mean), grads a dict of tensors.
     """
     lib = _cabi.load()
     cfg, (albedo, normal, roughness, metspec), _leaf, device = _prepare(
         material, device if device is not None else material.device, view_dir, lights, intensity, light_type, light_size,
-        return_srgb, multi_light
+        return_srgb, multi_light, view_type
     )
     _cabi.require_cuda(target, "target")
     target = target.contiguous()
@@ -108,11 +111,9 @@ def fused_loss_step(
     ls.target, ls.target_sl = _out_plane(target, cfg.per_light, cfg.batched)
     ls.loss_scale = float(loss_scale)
     ls.loss_sum = red.data_ptr()
+    fn = "pbr_ct_loss_fwd_bwd_camera" if cfg.camera else "pbr_ct_loss_fwd_bwd"
     with torch.cuda.device(device):
-        _cabi.check(
-            lib.pbr_ct_loss_fwd_bwd(_cabi.byref(d), _cabi.byref(ls), _cabi.byref(g), _cabi.stream_ptr(device)),
-            "pbr_ct_loss_fwd_bwd",
-        )
+        _cabi.check(getattr(lib, fn)(_cabi.byref(d), _cabi.byref(ls), _cabi.byref(g), _cabi.stream_ptr(device)), fn)
     grads = {"albedo": d_albedo, "normal": d_normal, "roughness": d_rough,
              ("metallic" if cfg.workflow == _cabi.WORKFLOW_METALLIC else "specular"): d_met}
     return red, grads
@@ -277,6 +278,12 @@ class FusedAdam:
         self.step_count = t_step
 
 
+def _no_camera(view_type: str) -> None:
+    if check_view_type(view_type) == "point":
+        raise ValueError("the one-launch fit step has no camera at a finite position (view_type='point'): "
+                         "use fit_step(fused=False)")
+
+
 def fused_fit_step(
     material: MaterialBase,
     optimizer: FusedAdam,
@@ -291,6 +298,7 @@ def fused_fit_step(
     loss_scale: Optional[float] = None,
     want_intensity_grad: bool = False,
     scratch: Optional[Dict[str, torch.Tensor]] = None,
+    view_type: str = "directional",
 ) -> torch.Tensor:
     """
     Render + MSE + backward + Adam + projection in ONE kernel launch (pbr_ct_fit_step): the map gradients stay in
@@ -300,8 +308,10 @@ def fused_fit_step(
     The optimiser must own exactly the maps the kernel shades (albedo, roughness, metallic | specular, and normal
     if the material has one) - the very tensors stored in the material, contiguous, not batch-broadcast - with the
     default projection for all of them or none at all.  Anything else: use `fit_step(..., fused=False)`.
+    The one-launch kernel shades with the view direction only: view_type="point" (a camera position) raises ValueError.
     Returns the device buffer [sum of squared errors, d_intensity(L*3)...] (not all-reduced).
     """
+    _no_camera(view_type)
     lib = _cabi.load()
     cfg, (albedo, normal, roughness, metspec), _leaf, device = _prepare(
         material, material.device, view_dir, lights, intensity, light_type, light_size, return_srgb, multi_light
@@ -367,7 +377,7 @@ def fused_fit_step(
 def fit_step(material: MaterialBase, optimizer: FusedAdam, target: torch.Tensor, view_dir, lights, intensity,
              light_type: str = "point", light_size: Optional[float] = None, multi_light: str = "per_light",
              scratch: Optional[Dict[str, torch.Tensor]] = None, global_numel: Optional[int] = None,
-             fused: bool = False, async_loss: bool = False, timing: Optional[list] = None):
+             fused: bool = False, async_loss: bool = False, timing: Optional[list] = None, view_type: str = "directional"):
     """
     One step of the sharded inverse-rendering fit on this rank's materials: fused render + MSE + backward
     (pbr_ct_loss_fwd_bwd), ONE all-reduce of the loss buffer, fused Adam + projection (pbr_adam_step).
@@ -376,11 +386,13 @@ def fit_step(material: MaterialBase, optimizer: FusedAdam, target: torch.Tensor,
     call returns a PendingLoss; the loss buffers alternate between two slots of `scratch`, and a slot is only reused
     after its all-reduce of two steps ago has completed.
     `global_numel`: element count of the target over ALL ranks (the MSE denominator); default: this rank's.
+    `view_type`: as CookTorranceBRDF's ("point": view_dir is the camera position); "point" needs fused=False.
     Returns the all-reduced buffer [sum of squared errors, ...] (device tensor; multiply [0] by 1/global_numel), or
     the PendingLoss that will deliver it.
     """
     numel = global_numel if global_numel is not None else target.numel()
     if fused:
+        _no_camera(view_type)
         if async_loss:
             scratch = scratch if scratch is not None else {}
             ring = scratch.setdefault("loss_ring", [None, None])
@@ -397,7 +409,7 @@ def fit_step(material: MaterialBase, optimizer: FusedAdam, target: torch.Tensor,
             return pend[i]
         return allreduce_loss_and_shared(buf)
     buf, grads = fused_loss_step(material, target, view_dir, lights, intensity, light_type, light_size,
-                                 multi_light=multi_light, loss_scale=1.0 / numel, out=scratch)
+                                 multi_light=multi_light, loss_scale=1.0 / numel, out=scratch, view_type=view_type)
     allreduce_loss_and_shared(buf)
     optimizer.step({k: grads[k] for k in optimizer.params})
     return buf
@@ -411,12 +423,14 @@ class RenderingLoss(nn.Module):
     """
 
     def __init__(self, light_type="point", view_dir=torch.tensor([0.0, 0.0, 1.0]), light_dir=torch.tensor([0.1, 0.1, 1.0]),
-                 light_intensity=torch.tensor([1.0, 1.0, 1.0]), light_size: Optional[float] = None):
+                 light_intensity=torch.tensor([1.0, 1.0, 1.0]), light_size: Optional[float] = None,
+                 view_type: str = "directional"):
         super().__init__()
         from .models import CookTorranceBRDF
 
         self.light_type = light_type
-        self.brdf = CookTorranceBRDF(light_type=light_type, multi_light="per_light")
+        self.brdf = CookTorranceBRDF(light_type=light_type, multi_light="per_light", view_type=view_type)
+        self.view_type = self.brdf.view_type
         self.view_dir = view_dir
         self.light_dir = light_dir
         self.light_intensity = light_intensity
@@ -439,7 +453,7 @@ class RenderingLoss(nn.Module):
         want_geo = grad_on and (shared[1].requires_grad or shared[2].requires_grad)
         kw = dict(light_type=self.light_type, light_size=self.light_size, multi_light="per_light",
                   want_map_grads=want_maps, want_intensity_grad=want_int, want_geometry_grad=want_geo,
-                  device=self.brdf.override_device)
+                  device=self.brdf.override_device, view_type=self.view_type)
         L = shared[1].shape[0] if shared[1].dim() == 2 else 1
 
         class _Fn(torch.autograd.Function):

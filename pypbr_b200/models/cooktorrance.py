@@ -12,7 +12,9 @@ Extensions over the reference (which is single-material, single-light, cooktorra
   * `light_dir_or_position` / `light_intensity` may be (L, 3):
       multi_light="accumulate" -> encode(clamp(sum_l clamp(shade_l, 0, 1), 0, 1)), shape (..., 3, H, W)
       multi_light="per_light"  -> one image per light, shape (..., L, 3, H, W)
-    both reduce to the reference for L = 1.
+    both reduce to the reference for L = 1;
+  * view_type="point": `view_dir` is the position of a camera at a finite distance, and every texel is shaded with its own
+    view vector F.normalize(camera - P) (texel (i, j) at P = (x_j, -y_i, 0) on the plane of side `light_size or 1.0`).
 """
 
 from __future__ import annotations
@@ -51,7 +53,7 @@ class _ShadeCfg:
     """Everything about one shading call that is not a texture map."""
 
     __slots__ = ("workflow", "metallic_channels", "light_type", "albedo_is_srgb", "specular_is_srgb", "return_srgb",
-                 "per_light", "light_size", "L", "view", "lights", "intensity", "on_device", "batched", "multi")
+                 "per_light", "light_size", "L", "view", "lights", "intensity", "on_device", "batched", "multi", "camera")
 
 
 def _fill_desc(cfg: _ShadeCfg, albedo, normal, roughness, metspec, keep: list) -> "_cabi.PbrCtDesc":
@@ -103,6 +105,13 @@ def _out_shape(cfg: _ShadeCfg, albedo: Tensor):
     return (*shape, 3, albedo.shape[-2], albedo.shape[-1])
 
 
+def check_view_type(view_type: str) -> str:
+    view_type = view_type.lower()
+    if view_type not in ("directional", "point"):
+        raise ValueError(f"Unsupported view_type: {view_type}. Must be 'directional' or 'point'.")
+    return view_type
+
+
 class _CookTorranceFn(torch.autograd.Function):
     @staticmethod
     def forward(ctx, cfg: _ShadeCfg, albedo, normal, roughness, metspec, intensity_leaf, lights_leaf=None, view_leaf=None):
@@ -111,15 +120,16 @@ class _CookTorranceFn(torch.autograd.Function):
         d = _fill_desc(cfg, albedo, normal, roughness, metspec, keep)
         out = torch.empty(_out_shape(cfg, albedo), dtype=torch.float32, device=albedo.device)
         d.out, d.out_sl = _out_plane(out, cfg.per_light, cfg.batched)
+        fn = "pbr_ct_forward_camera" if cfg.camera else "pbr_ct_forward"
         with _cabi.device_guard(albedo.device):
-            _cabi.check(lib.pbr_ct_forward(_cabi.byref(d), _cabi.stream_ptr(albedo.device)), "pbr_ct_forward")
+            _cabi.check(getattr(lib, fn)(_cabi.byref(d), _cabi.stream_ptr(albedo.device)), fn)
         ctx.cfg = cfg
         ctx.has_normal = normal is not None
         # the shared parameters may live on another device than the maps (the reference moves them with .to(device))
         ctx.leaf_meta = [(t.device, tuple(t.shape)) if t is not None else None for t in (intensity_leaf, lights_leaf, view_leaf)]
         # accumulate mode with several lights: the output (which the caller holds anyway) lets the backward skip its
-        # first pass, the recomputation of the summed image (PbrCtGrads.fwd_out)
-        ctx.keep_out = cfg.L > 1 and not cfg.per_light
+        # first pass, the recomputation of the summed image (PbrCtGrads.fwd_out; the camera kernels do not use it)
+        ctx.keep_out = cfg.L > 1 and not cfg.per_light and not cfg.camera
         ctx.save_for_backward(albedo, normal if normal is not None else albedo.new_empty(0), roughness, metspec,
                               out if ctx.keep_out else albedo.new_empty(0))
         return out
@@ -155,8 +165,9 @@ class _CookTorranceFn(torch.autograd.Function):
         d_view = torch.zeros(3, dtype=torch.float32, device=dev) if need[7] else None
         g.d_lights = d_lights.data_ptr() if d_lights is not None else None
         g.d_view = d_view.data_ptr() if d_view is not None else None
+        fn = "pbr_ct_backward_camera" if cfg.camera else "pbr_ct_backward"
         with _cabi.device_guard(dev):
-            _cabi.check(lib.pbr_ct_backward(_cabi.byref(d), _cabi.byref(g), _cabi.stream_ptr(dev)), "pbr_ct_backward")
+            _cabi.check(getattr(lib, fn)(_cabi.byref(d), _cabi.byref(g), _cabi.stream_ptr(dev)), fn)
         shared = []
         for t, meta in zip((d_int, d_lights, d_view), ctx.leaf_meta):
             shared.append(t.reshape(meta[1]).to(meta[0]) if (t is not None and meta is not None) else None)
@@ -164,13 +175,15 @@ class _CookTorranceFn(torch.autograd.Function):
 
 
 def _prepare(material: MaterialBase, device, view_dir, light, intensity, light_type: str, light_size, return_srgb: bool,
-             multi_light: str):
+             multi_light: str, view_type: str = "directional"):
     """Host-side validation in the reference's order (cooktorrance.py:92-118); returns (cfg, maps, shared-parameter
-    leaves (intensity, lights, view - None where no gradient is wanted), device)."""
+    leaves (intensity, lights, view - None where no gradient is wanted), device).  view_type="point": view_dir is the
+    camera position."""
     # attribute / workflow errors first, exactly where the reference raises them (cooktorrance.py:99-118)
     roughness = material.roughness  # AttributeError if the map was never set
     normal = material.normal  # AttributeError unless the key exists (None selects the +Z default)
     cfg = _ShadeCfg()
+    cfg.camera = check_view_type(view_type) == "point"
     cfg.specular_is_srgb = True
     cfg.metallic_channels = 1
     if hasattr(material, "metallic") and material.metallic is not None:
@@ -234,7 +247,8 @@ def _prepare(material: MaterialBase, device, view_dir, light, intensity, light_t
         metspec = fit(metspec, (3,), "specular")
 
     cfg.light_type = _cabi.LIGHT_POINT if light_type == "point" else _cabi.LIGHT_DIRECTIONAL
-    cfg.light_size = float(light_size or 1.0) if light_type == "point" else 0.0
+    # the plane's size places the texels: a point light's position, or a camera's, is relative to it
+    cfg.light_size = float(light_size or 1.0) if (light_type == "point" or cfg.camera) else 0.0
     cfg.return_srgb = bool(return_srgb)
 
     view = torch.as_tensor(view_dir, dtype=torch.float32) if not isinstance(view_dir, Tensor) else view_dir
@@ -282,12 +296,18 @@ class CookTorranceBRDF(BRDFModel):
     """
     Cook-Torrance BRDF (GGX D, Smith-Schlick G, Schlick F) for directional and point lights.
 
+    view_type: "directional" (the reference: `view_dir` is one view direction for the whole image) or "point"
+    (`view_dir` is the position of a camera at a finite distance, in the frame of a point light's position; each
+    texel is shaded with its own view vector).
+
     Example:
         brdf = CookTorranceBRDF(light_type="point")
         color = brdf(material, view_dir, light_pos, light_intensity, light_size)   # (3, H, W)
+        color = CookTorranceBRDF(light_type="point", view_type="point")(material, camera_pos, light_pos, light_intensity)
     """
 
-    def __init__(self, light_type: str = "point", override_device: torch.device = None, multi_light: str = "accumulate"):
+    def __init__(self, light_type: str = "point", override_device: torch.device = None, multi_light: str = "accumulate",
+                 view_type: str = "directional"):
         super().__init__()
         self.light_type = light_type.lower()
         if self.light_type not in ["directional", "point"]:
@@ -296,6 +316,7 @@ class CookTorranceBRDF(BRDFModel):
             raise ValueError(f"Unsupported multi_light: {multi_light}. Must be 'accumulate' or 'per_light'.")
         self.override_device = override_device
         self.multi_light = multi_light
+        self.view_type = check_view_type(view_type)
 
     def forward(
         self,
@@ -315,7 +336,7 @@ class CookTorranceBRDF(BRDFModel):
         device = self.override_device or material.device
         cfg, (albedo, normal, roughness, metspec), shared_leaves, _ = _prepare(
             material, device, view_dir, light_dir_or_position, light_intensity, self.light_type, light_size,
-            return_srgb, self.multi_light,
+            return_srgb, self.multi_light, self.view_type,
         )
         # the shared-parameter leaves are views of the caller's tensors, so e.g. the (L, 3) intensity gradient reaches
         # the caller's (3,) or (L, 3) tensor through autograd's view tracking.
