@@ -23,19 +23,11 @@ __device__ __forceinline__ void mbar_arrive_expect_tx(uint64_t* bar, uint32_t by
   asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_u32(bar)), "r"(bytes) : "memory");
 }
 
-// plain arrival (consumer -> producer "stage is free")
-__device__ __forceinline__ void mbar_arrive(uint64_t* bar) {
-  asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(smem_u32(bar)) : "memory");
-}
-
 // try_wait suspends the warp in hardware until the phase completes or a time limit expires; with the default limit a warp
 // whose tile is late came back ~18 times per tile (YIELD + TRYWAIT + BRA: 4.6 % of the streamed backward's instructions,
-// issued in competition with the warps that have work).  PBR_WAIT_HINT_NS raises the limit (0: the default limit).
-#ifndef PBR_WAIT_HINT_NS
-#define PBR_WAIT_HINT_NS 20000
-#endif
+// issued in competition with the warps that have work).  So the wait passes a time hint that raises the limit.
+constexpr uint32_t kWaitHintNs = 20000;
 __device__ __forceinline__ void mbar_wait(uint64_t* bar, uint32_t parity) {
-#if PBR_WAIT_HINT_NS > 0
   asm volatile(
       "{\n"
       ".reg .pred p;\n"
@@ -45,21 +37,8 @@ __device__ __forceinline__ void mbar_wait(uint64_t* bar, uint32_t parity) {
       "bra PBR_WAIT_%=;\n"
       "PBR_DONE_%=:\n"
       "}\n" ::"r"(smem_u32(bar)),
-      "r"(parity), "r"((uint32_t)PBR_WAIT_HINT_NS)
+      "r"(parity), "r"(kWaitHintNs)
       : "memory");
-#else
-  asm volatile(
-      "{\n"
-      ".reg .pred p;\n"
-      "PBR_WAIT_%=:\n"
-      "mbarrier.try_wait.parity.shared::cta.b64 p, [%0], %1;\n"
-      "@p bra PBR_DONE_%=;\n"
-      "bra PBR_WAIT_%=;\n"
-      "PBR_DONE_%=:\n"
-      "}\n" ::"r"(smem_u32(bar)),
-      "r"(parity)
-      : "memory");
-#endif
 }
 
 // L2 policy for data that is read exactly once

@@ -10,12 +10,10 @@
 //   tile    = blockDim.y rows x (blockDim.x * kST) texels of ONE material: every input plane of the tile
 //             (albedo x3, roughness, metallic | specular, normal x3, and grad_out | target x3 for the
 //             backward) is kTileFloats contiguous floats of shared memory per stage, in image order;
-//   producer= every warp for itself (per-warp pipelines, the default for both kernels): a warp owns 32 x kST contiguous texels
+//   producer= every warp for itself (per-warp pipelines): a warp owns 32 x kST contiguous texels
 //             of the tile row, i.e. one cp.async.bulk of 512 B per plane and stage, completion counted in bytes on the
 //             warp's own mbarrier (pbr_async.cuh); right after it has read a stage into registers one lane per plane
 //             re-arms the barrier and issues the copies of the tile kStages ahead.  No cross-warp synchronisation at all.
-//             (PBR_STREAM_PER_WARP_*=0 builds the CTA-level pipeline instead: warp 0 feeds the whole CTA, one copy per
-//             (plane, row), and waits on an "empty" mbarrier the other warps arrive on after their last read.)
 //   consumer= all threads.  A thread owns kSSlots lane-values (texel pairs) of one tile row, INTERLEAVED
 //             with the other threads of the row: slot j of thread tx covers the texels
 //             j*(bx*kLanes) + tx*kLanes ... + kLanes-1 of the row.  So one warp-level LDS.64 / STG.64
@@ -29,8 +27,8 @@
 // per-texel light geometry (material independent) is computed once and reused - as in the generic
 // kernels - and the pipeline stays full for the whole walk.
 //
-// Measured floor of this data-movement design with the shading math compiled out (-DPBR_DBG_NOMATH,
-// tools/build_variants.py): 6.4-6.6 TB/s forward and backward, i.e. 98-100 % of the measured copy peak;
+// Measured floor of this data-movement design with the shading math compiled out (a debug build, DESIGN §3.1):
+// 6.4-6.6 TB/s forward and backward, i.e. 98-100 % of the measured copy peak;
 // whatever the real kernels lose against that is instruction issue, not memory.  With the kFast flavour (below) they
 // lose almost nothing: forward 0.446-0.451 ms (100 %), backward 0.783-0.807 ms (96-99 %) at 64 x 1024^2.
 #pragma once
@@ -39,55 +37,25 @@
 
 namespace pbr {
 
-#ifndef PBR_STREAM_STAGES
-#define PBR_STREAM_STAGES 2
-#endif
-#ifndef PBR_STREAM_THREADS
-#define PBR_STREAM_THREADS 128
-#endif
-#ifndef PBR_STREAM_TEXELS
-#define PBR_STREAM_TEXELS 4   // texels per thread: 4 (two packed pairs) or 2 (one pair)
-#endif
-#ifndef PBR_STREAM_FWD_MIN_CTAS
-#define PBR_STREAM_FWD_MIN_CTAS 4   // 128 registers
-#endif
-#ifndef PBR_STREAM_BWD_MIN_CTAS
-#define PBR_STREAM_BWD_MIN_CTAS 3   // 168 registers
-#endif
-constexpr int kStreamThreads = PBR_STREAM_THREADS;
-constexpr int kStages = PBR_STREAM_STAGES;
-constexpr int kST = PBR_STREAM_TEXELS;
-static_assert((kST == 2 || kST == 4) && kST % kLanes == 0, "stream kernels: 2 or 4 texels per thread");
+constexpr int kStages = 2;
+constexpr int kStreamThreads = 128;
+constexpr int kST = 4;   // texels per thread: two packed pairs
+constexpr int kStreamFwdMinCtas = 4;   // 128 registers
+constexpr int kStreamBwdMinCtas = 3;   // 168 registers
+static_assert(kST % kLanes == 0, "stream kernels: whole lane-values per thread");
 constexpr int kSSlots = kST / kLanes;               // lane-values per thread
 constexpr int kTileFloats = kStreamThreads * kST;   // floats of one plane in one stage (2 KB at 128 threads x 4 texels)
-// PBR_STREAM_PER_WARP: every warp runs its OWN copy pipeline over its own 32 x kST texels of a tile row (plane stride
+// Per-warp pipelines: every warp runs its OWN copy pipeline over its own 32 x kST texels of a tile row (plane stride
 // inside a stage = one warp segment) instead of warp 0 feeding the whole CTA: a warp refills a stage right after its own
 // last read of it, without waiting for the other warps or for its own arithmetic.
-// Measured (C2 shape, tools/tune.py): forward 0.499 -> 0.474 ms (95 % of the HBM copy peak).  The backward used to be
+// Measured (C2 shape, bare C ABI): forward 0.499 -> 0.474 ms (95 % of the HBM copy peak).  The backward used to be
 // 1.5 % slower that way (0.944 -> 0.959 ms): the per-warp issue of 11 small copies per tile cost what the decoupling gave.
 // With the kFast flavour (below) the balance flips - CTA-level 0.852 ms, per-warp 0.807 ms at 64 x 1024^2
 // (profiles/r2_tune_c2_kfast_variants.json) - so both kernels run per-warp pipelines.  Deeper pipelines (3, 4 stages) are
-// slower in both.
-#ifndef PBR_STREAM_PER_WARP_FWD
-#define PBR_STREAM_PER_WARP_FWD 1
-#endif
-#ifndef PBR_STREAM_PER_WARP_BWD
-#define PBR_STREAM_PER_WARP_BWD 1
-#endif
-#ifndef PBR_STREAM_BWD_LATE_REFILL
-#define PBR_STREAM_BWD_LATE_REFILL 0   // per-warp backward: refill after the whole tile instead of after the last read
-#endif
-constexpr bool kPerWarpFwd = PBR_STREAM_PER_WARP_FWD != 0, kPerWarpBwd = PBR_STREAM_PER_WARP_BWD != 0;
-constexpr bool kLateRefill = PBR_STREAM_BWD_LATE_REFILL != 0;
-// CTA-level backward: the warp that reads a stage LAST refills it at once (a shared-memory counter elects it) instead of
-// warp 0 doing so after it has shaded its own second pair and waited for the other warps on the `empty` barrier.
-#ifndef PBR_STREAM_BWD_LAST_REFILL
-#define PBR_STREAM_BWD_LAST_REFILL 0
-#endif
-constexpr bool kLastRefill = PBR_STREAM_BWD_LAST_REFILL != 0 && !kPerWarpBwd;
-constexpr int kWarpSeg = 32 * kST;                                  // floats of one plane a warp owns per tile row
-constexpr int kMaxPipes = kStreamThreads / 32;                      // independent copy pipelines per CTA (per-warp mode)
-PBR_HDC int plane_stride(bool per_warp) { return per_warp ? kWarpSeg : kStreamThreads * kST; }   // floats between two planes of a stage
+// slower in both, and so were a backward that refills after the whole tile instead of after its last read (0.808 ms) and
+// a CTA-level backward in which the warp that reads a stage last refills it (0.860 ms; DESIGN §3.1).
+constexpr int kWarpSeg = 32 * kST;                  // floats of one plane a warp owns per tile row = floats between two planes of a stage
+constexpr int kPipes = kStreamThreads / 32;         // independent copy pipelines per CTA
 constexpr int kMaxSrcPlanes = 13;                   // albedo 3 + roughness 1 + metallic|specular 3 + normal 3 + grad_out|target 3
 
 // backward flavours (compile-time, so the plain backward carries no reduction code)
@@ -102,9 +70,7 @@ struct StreamSrc {
 };
 
 struct StreamShared {
-  uint64_t full[kStages * kMaxPipes];   // producer -> consumers: the copies of the stage have landed (transaction bytes)
-  uint64_t empty[kStages];   // consumers -> producer: one arrival per warp after its last read of the stage
-  int readers[kStages];      // kLastRefill: warps that have read the stage's current tile
+  uint64_t full[kStages * kPipes];   // producer -> consumers: the copies of the stage have landed (transaction bytes)
   StreamSrc src[kMaxSrcPlanes];
   int n_src;
 };
@@ -141,20 +107,6 @@ __device__ __forceinline__ void stream_build_table(const CtKParams& p, int row0,
   sh.n_src = n;
 }
 
-// warp 0: enqueue the copies of material `b` into `stage` (floats) and arm its barrier
-__device__ __forceinline__ void stream_issue(const StreamShared& sh, uint64_t* bar, float* stage, int b, int rows_valid,
-                                             int seg_bytes, int row_floats, uint64_t policy, int lane) {
-  const int items = sh.n_src * rows_valid;
-  if (lane == 0) mbar_arrive_expect_tx(bar, (uint32_t)(items * seg_bytes));
-  __syncwarp();
-  for (int it = lane; it < items; it += 32) {
-    const int pl = it / rows_valid, r = it - pl * rows_valid;
-    const StreamSrc& s = sh.src[pl];
-    bulk_g2s(stage + s.slot * kTileFloats + r * row_floats, s.base + (int64_t)b * s.sb + (int64_t)r * s.sh,
-             (uint32_t)seg_bytes, bar, policy);
-  }
-}
-
 // per-warp pipeline: the calling warp enqueues ITS segment (32 x kST texels of its row) of every plane of material `b`
 __device__ __forceinline__ void warp_issue(const StreamShared& sh, uint64_t* bar, float* stage, int b, int64_t row_in_tile,
                                            int col_in_tile, int seg_bytes, uint64_t policy) {
@@ -172,53 +124,35 @@ __device__ __forceinline__ void fence_proxy_async() { asm volatile("fence.proxy.
 
 // one lane-value (kLanes consecutive floats) from shared memory / to global memory
 __device__ __forceinline__ V lds_v(const float* p) {
-#if defined(PBR_SCALAR_LANES)
-  return *p;
-#else
   const float2 v = *reinterpret_cast<const float2*>(p);
   return V{v.x, v.y};
-#endif
 }
-__device__ __forceinline__ void stg_v(float* p, V v) {
-#if defined(PBR_SCALAR_LANES)
-  __stcs(p, v);
-#else
-  __stcs(reinterpret_cast<float2*>(p), make_float2(v.x, v.y));
-#endif
-}
+__device__ __forceinline__ void stg_v(float* p, V v) { __stcs(reinterpret_cast<float2*>(p), make_float2(v.x, v.y)); }
 
 // Geometry of the tile this CTA owns and of the thread inside it.
 struct StreamWhere {
   int row0, col0;       // tile origin
   int row, col;         // this thread's row and the first texel of its slot 0
-  int slot_stride;      // texels between a thread's consecutive slots (= blockDim.x * kLanes)
-  int toff;             // offset of slot 0 inside a tile plane (floats)
-  int rows_valid, seg_bytes, row_floats;
-  int wcol;             // per-warp pipelines: offset of the warp's segment inside the tile row
+  int slot_stride;      // texels between a thread's consecutive slots (= 32 * kLanes)
+  int toff;             // offset of slot 0 inside the warp's segment of a plane (floats)
+  int seg_bytes;        // bytes of the warp's segment of one plane row (0: the warp has nothing to copy or shade)
+  int wcol;             // offset of the warp's segment inside the tile row
   bool row_ok;
 };
-template <bool kPerWarp>
+// blockDim.x is a multiple of 32: a warp sits inside one tile row and owns kWarpSeg contiguous texels of it
 __device__ __forceinline__ StreamWhere stream_locate(int H, int W) {
   StreamWhere w;
-  w.row_floats = blockDim.x * kST;
-  w.slot_stride = blockDim.x * kLanes;
+  const int lane = threadIdx.x & 31;
   w.row0 = blockIdx.y * blockDim.y;
-  w.col0 = blockIdx.x * w.row_floats;
+  w.col0 = blockIdx.x * (blockDim.x * kST);
   w.row = w.row0 + threadIdx.y;
-  w.col = w.col0 + threadIdx.x * kLanes;
-  w.toff = threadIdx.y * w.row_floats + threadIdx.x * kLanes;
-  w.rows_valid = min((int)blockDim.y, H - w.row0);
-  w.seg_bytes = min(w.row_floats, W - w.col0) * 4;
   w.row_ok = w.row < H;
-  if (kPerWarp) {   // blockDim.x is a multiple of 32: a warp sits inside one tile row and owns kWarpSeg contiguous texels of it
-    const int lane = threadIdx.x & 31;
-    w.wcol = (threadIdx.x >> 5) * kWarpSeg;           // first texel of the warp's segment inside the tile row
-    w.slot_stride = 32 * kLanes;
-    w.col = w.col0 + w.wcol + lane * kLanes;
-    w.toff = lane * kLanes;
-    const int left = W - (w.col0 + w.wcol);
-    w.seg_bytes = (w.row_ok && left > 0) ? min(kWarpSeg, left) * 4 : 0;   // 0: the warp has nothing to copy or shade
-  }
+  w.wcol = (threadIdx.x >> 5) * kWarpSeg;           // first texel of the warp's segment inside the tile row
+  w.slot_stride = 32 * kLanes;
+  w.col = w.col0 + w.wcol + lane * kLanes;
+  w.toff = lane * kLanes;
+  const int left = W - (w.col0 + w.wcol);
+  w.seg_bytes = (w.row_ok && left > 0) ? min(kWarpSeg, left) * 4 : 0;
   return w;
 }
 // kFast flavour of the streamed kernels (round 2).  The host picks it when the launch is the plain case: blockDim = (kStreamThreads, 1),
@@ -231,33 +165,18 @@ __device__ __forceinline__ StreamWhere stream_locate(int H, int W) {
 // Measured at 64 x 1024^2 (bare C ABI): backward 0.923 -> 0.852 ms (586 M -> 519 M warp-instructions), with per-warp
 // pipelines 0.807 ms = 96 % of the measured copy peak (floor with the math compiled out: 0.775 ms); forward
 // 0.461 -> 0.446 ms = the copy peak.
-#ifndef PBR_STREAM_FAST
-#define PBR_STREAM_FAST 1
-#endif
-constexpr bool kStreamFast = PBR_STREAM_FAST != 0;
-template <bool kPerWarp>
 __device__ __forceinline__ StreamWhere stream_locate_fast() {
   StreamWhere w;
-  w.row_floats = kTileFloats;
+  const int lane = threadIdx.x & 31;
   w.row0 = blockIdx.y;
   w.col0 = blockIdx.x * kTileFloats;
   w.row = w.row0;
-  w.rows_valid = 1;
   w.row_ok = true;
-  if (kPerWarp) {
-    const int lane = threadIdx.x & 31;
-    w.wcol = (threadIdx.x >> 5) * kWarpSeg;
-    w.slot_stride = 32 * kLanes;
-    w.col = w.col0 + w.wcol + lane * kLanes;
-    w.toff = lane * kLanes;
-    w.seg_bytes = kWarpSeg * 4;
-  } else {
-    w.wcol = 0;
-    w.slot_stride = kStreamThreads * kLanes;
-    w.col = w.col0 + threadIdx.x * kLanes;
-    w.toff = threadIdx.x * kLanes;
-    w.seg_bytes = kTileFloats * 4;
-  }
+  w.wcol = (threadIdx.x >> 5) * kWarpSeg;
+  w.slot_stride = 32 * kLanes;
+  w.col = w.col0 + w.wcol + lane * kLanes;
+  w.toff = lane * kLanes;
+  w.seg_bytes = kWarpSeg * 4;
   return w;
 }
 // kFast also fixes the colour handling to the reference's defaults (sRGB albedo / specular in, sRGB out), which the host checks
@@ -293,21 +212,17 @@ __device__ __forceinline__ void stream_coords(const CtStage& S, const StreamWher
 // forward
 // ------------------------------------------------------------------------------------------------
 template <int WF, int kLight, bool kFast = false>
-__global__ void __launch_bounds__(kStreamThreads, PBR_STREAM_FWD_MIN_CTAS) ct_forward_stream(const __grid_constant__ CtKParams p) {
+__global__ void __launch_bounds__(kStreamThreads, kStreamFwdMinCtas) ct_forward_stream(const __grid_constant__ CtKParams p) {
   using SL = Slots<WF, false>;
   constexpr int G = kSSlots;   // all of the thread's pairs are shaded together
-  constexpr bool kPerWarp = kPerWarpFwd;
-  constexpr int kPlaneStride = plane_stride(kPerWarp), kPipes = kPerWarp ? kMaxPipes : 1;
   extern __shared__ __align__(128) float stream_smem[];
   __shared__ CtStage S;
   __shared__ StreamShared sh;
   const int tid = kFast ? threadIdx.x : threadIdx.y * blockDim.x + threadIdx.x;
-  const StreamWhere w = kFast ? stream_locate_fast<kPerWarp>() : stream_locate<kPerWarp>(p.H, p.W);
+  const StreamWhere w = kFast ? stream_locate_fast() : stream_locate(p.H, p.W);
   const int row_in_tile = kFast ? 0 : threadIdx.y;
   if (tid == 0) {
     stream_build_table<WF, false>(p, w.row0, w.col0, sh);
-#pragma unroll
-    for (int s = 0; s < kStages; ++s) mbar_init(&sh.empty[s], kStreamThreads / 32);
 #pragma unroll
     for (int s = 0; s < kStages * kPipes; ++s) mbar_init(&sh.full[s], 1);
     mbar_init_fence();
@@ -317,22 +232,15 @@ __global__ void __launch_bounds__(kStreamThreads, PBR_STREAM_FWD_MIN_CTAS) ct_fo
   const int b0 = blockIdx.z * p.mats_per_cta;
   const int ntiles = min(b0 + p.mats_per_cta, p.B) - b0;
   const int stage_floats = ((kFast || p.normal.ptr) ? SL::count : SL::count_no_normal) * kTileFloats;
-  uint64_t policy = 0;
-  // per-warp pipelines: this warp's barriers and stage buffers (planes x kWarpSeg floats per stage)
-  const int pipe = kPerWarp ? (tid >> 5) : 0;
+  // this warp's barriers and stage buffers (planes x kWarpSeg floats per stage)
+  const int pipe = tid >> 5;
   uint64_t* const full = sh.full + pipe * kStages;
-  float* const my_stages = stream_smem + (kPerWarp ? pipe * kStages * (stage_floats / (kTileFloats / kWarpSeg)) : 0);
-  const int my_stage_floats = kPerWarp ? stage_floats / (kTileFloats / kWarpSeg) : stage_floats;
-  if (kPerWarp) {
-    policy = l2_evict_first_policy();
-    if (w.seg_bytes > 0)
-      for (int k = 0; k < kStages && k < ntiles; ++k)
-        warp_issue(sh, &full[k], my_stages + k * my_stage_floats, b0 + k, row_in_tile, w.wcol, w.seg_bytes, policy);
-  } else if (tid < 32) {
-    policy = l2_evict_first_policy();
+  float* const my_stages = stream_smem + pipe * kStages * (stage_floats / (kTileFloats / kWarpSeg));
+  const int my_stage_floats = stage_floats / (kTileFloats / kWarpSeg);
+  const uint64_t policy = l2_evict_first_policy();
+  if (w.seg_bytes > 0)
     for (int k = 0; k < kStages && k < ntiles; ++k)
-      stream_issue(sh, &sh.full[k], stream_smem + k * stage_floats, b0 + k, w.rows_valid, w.seg_bytes, w.row_floats, policy, tid);
-  }
+      warp_issue(sh, &full[k], my_stages + k * my_stage_floats, b0 + k, row_in_tile, w.wcol, w.seg_bytes, policy);
 
   V x[kSSlots];
   float y;
@@ -350,29 +258,24 @@ __global__ void __launch_bounds__(kStreamThreads, PBR_STREAM_FWD_MIN_CTAS) ct_fo
   for (int k = 0; k < ntiles; ++k) {
     const int s = k % kStages;
     const float* st = my_stages + s * my_stage_floats + w.toff;
-    if (!kPerWarp || w.seg_bytes > 0) mbar_wait(&full[s], (k / kStages) & 1);
+    if (w.seg_bytes > 0) mbar_wait(&full[s], (k / kStages) & 1);
     V a[3][G], n[3][G], r[G], m[3][G];
 #pragma unroll
     for (int j = 0; j < G; ++j) {
       const float* sj = st + j * w.slot_stride;
 #pragma unroll
-      for (int c = 0; c < 3; ++c) a[c][j] = lds_v(sj + (SL::albedo + c) * kPlaneStride);
-      r[j] = lds_v(sj + SL::rough * kPlaneStride);
+      for (int c = 0; c < 3; ++c) a[c][j] = lds_v(sj + (SL::albedo + c) * kWarpSeg);
+      r[j] = lds_v(sj + SL::rough * kWarpSeg);
 #pragma unroll
-      for (int c = 0; c < 3; ++c) m[c][j] = c < SL::mc ? lds_v(sj + (SL::met + c) * kPlaneStride) : splat<V>(0.0f);
+      for (int c = 0; c < 3; ++c) m[c][j] = c < SL::mc ? lds_v(sj + (SL::met + c) * kWarpSeg) : splat<V>(0.0f);
 #pragma unroll
-      for (int c = 0; c < 3; ++c) n[c][j] = has_normal ? lds_v(sj + (SL::normal + c) * kPlaneStride) : splat<V>(c == 2 ? 1.0f : 0.0f);
+      for (int c = 0; c < 3; ++c) n[c][j] = has_normal ? lds_v(sj + (SL::normal + c) * kWarpSeg) : splat<V>(c == 2 ? 1.0f : 0.0f);
     }
-    // this warp holds its texels in registers: refill its own stage (per-warp pipelines), or tell the producer
-    // (no CTA-wide barrier - warps drift freely)
+    // this warp holds its texels in registers: refill its own stage (no CTA-wide barrier - warps drift freely)
     __syncwarp();
-    if (kPerWarp) {
-      if (w.seg_bytes > 0 && k + kStages < ntiles) {
-        fence_proxy_async();
-        warp_issue(sh, &full[s], my_stages + s * my_stage_floats, b0 + k + kStages, row_in_tile, w.wcol, w.seg_bytes, policy);
-      }
-    } else if ((tid & 31) == 0) {
-      mbar_arrive(&sh.empty[s]);
+    if (w.seg_bytes > 0 && k + kStages < ntiles) {
+      fence_proxy_async();
+      warp_issue(sh, &full[s], my_stages + s * my_stage_floats, b0 + k + kStages, row_in_tile, w.wcol, w.seg_bytes, policy);
     }
     if (any) {
       V outv[3][G];
@@ -382,15 +285,7 @@ __global__ void __launch_bounds__(kStreamThreads, PBR_STREAM_FWD_MIN_CTAS) ct_fo
 #pragma unroll
           for (int j = 0; j < G; ++j) outv[c][j] = v[c][j];
       };
-#if defined(PBR_DBG_NOMATH)   // memory pipeline only (tools/build_variants.py "nomath"): results are meaningless
-#pragma unroll
-      for (int j = 0; j < G; ++j)
-#pragma unroll
-        for (int c = 0; c < 3; ++c) outv[c][j] = a[c][j] + n[c][j] + m[c][j] * r[j] + hg[j].lx + x[j];
-      (void)emit;
-#else
       ct_forward_group<WF, kLight, V, G>(S, stream_flags<kFast>(p.flags), a, n, r, m, x, y, hg, emit);
-#endif
 #pragma unroll
       for (int j = 0; j < G; ++j)
         if (act[j]) {
@@ -399,12 +294,6 @@ __global__ void __launch_bounds__(kStreamThreads, PBR_STREAM_FWD_MIN_CTAS) ct_fo
         }
     }
     o += p.out.sb;
-    // producer: by the time warp 0 has shaded tile k every warp has long since read stage s
-    if (!kPerWarp && tid < 32 && k + kStages < ntiles) {
-      mbar_wait(&sh.empty[s], (k / kStages) & 1);
-      stream_issue(sh, &sh.full[s], stream_smem + s * stage_floats, b0 + k + kStages, w.rows_valid, w.seg_bytes,
-                   w.row_floats, policy, tid);
-    }
   }
 }
 
@@ -412,10 +301,8 @@ __global__ void __launch_bounds__(kStreamThreads, PBR_STREAM_FWD_MIN_CTAS) ct_fo
 // backward / fused loss
 // ------------------------------------------------------------------------------------------------
 template <int WF, int kLight, int kMode, bool kFast = false>
-__global__ void __launch_bounds__(kStreamThreads, PBR_STREAM_BWD_MIN_CTAS) ct_backward_stream(const __grid_constant__ CtKParams p) {
+__global__ void __launch_bounds__(kStreamThreads, kStreamBwdMinCtas) ct_backward_stream(const __grid_constant__ CtKParams p) {
   using SL = Slots<WF, true>;
-  constexpr bool kPerWarp = kPerWarpBwd;
-  constexpr int kPlaneStride = plane_stride(kPerWarp), kPipes = kPerWarp ? kMaxPipes : 1;
   constexpr bool kLoss = (kMode & kModeLoss) != 0;
   constexpr bool kIntGrad = (kMode & kModeIntGrad) != 0;
   extern __shared__ __align__(128) float stream_smem[];
@@ -423,11 +310,9 @@ __global__ void __launch_bounds__(kStreamThreads, PBR_STREAM_BWD_MIN_CTAS) ct_ba
   __shared__ StreamShared sh;
   __shared__ float s_red[kStreamThreads / 32][4];
   const int tid = kFast ? threadIdx.x : threadIdx.y * blockDim.x + threadIdx.x;
-  const StreamWhere w = kFast ? stream_locate_fast<kPerWarp>() : stream_locate<kPerWarp>(p.H, p.W);
+  const StreamWhere w = kFast ? stream_locate_fast() : stream_locate(p.H, p.W);
   if (tid == 0) {
     stream_build_table<WF, true>(p, w.row0, w.col0, sh);
-#pragma unroll
-    for (int s = 0; s < kStages; ++s) { mbar_init(&sh.empty[s], kStreamThreads / 32); sh.readers[s] = 0; }
 #pragma unroll
     for (int s = 0; s < kStages * kPipes; ++s) mbar_init(&sh.full[s], 1);
     mbar_init_fence();
@@ -437,24 +322,16 @@ __global__ void __launch_bounds__(kStreamThreads, PBR_STREAM_BWD_MIN_CTAS) ct_ba
   const int b0 = blockIdx.z * p.mats_per_cta;
   const int ntiles = min(b0 + p.mats_per_cta, p.B) - b0;
   const int stage_floats = ((kFast || p.normal.ptr) ? SL::count : SL::count_no_normal) * kTileFloats;
-  uint64_t policy = 0;
-  if (kLastRefill) policy = l2_evict_first_policy();
-  // per-warp pipelines: this warp's barriers and stage buffers (planes x kWarpSeg floats per stage)
-  const int pipe = kPerWarp ? (tid >> 5) : 0;
+  // this warp's barriers and stage buffers (planes x kWarpSeg floats per stage)
+  const int pipe = tid >> 5;
   uint64_t* const full = sh.full + pipe * kStages;
-  float* const my_stages = stream_smem + (kPerWarp ? pipe * kStages * (stage_floats / (kTileFloats / kWarpSeg)) : 0);
-  const int my_stage_floats = kPerWarp ? stage_floats / (kTileFloats / kWarpSeg) : stage_floats;
+  float* const my_stages = stream_smem + pipe * kStages * (stage_floats / (kTileFloats / kWarpSeg));
+  const int my_stage_floats = stage_floats / (kTileFloats / kWarpSeg);
   const int row_in_tile = kFast ? 0 : threadIdx.y;
-  if (kPerWarp) {
-    policy = l2_evict_first_policy();
-    if (w.seg_bytes > 0)
-      for (int k = 0; k < kStages && k < ntiles; ++k)
-        warp_issue(sh, &full[k], my_stages + k * my_stage_floats, b0 + k, row_in_tile, w.wcol, w.seg_bytes, policy);
-  } else if (tid < 32) {
-    policy = l2_evict_first_policy();
+  const uint64_t policy = l2_evict_first_policy();
+  if (w.seg_bytes > 0)
     for (int k = 0; k < kStages && k < ntiles; ++k)
-      stream_issue(sh, &sh.full[k], stream_smem + k * stage_floats, b0 + k, w.rows_valid, w.seg_bytes, w.row_floats, policy, tid);
-  }
+      warp_issue(sh, &full[k], my_stages + k * my_stage_floats, b0 + k, row_in_tile, w.wcol, w.seg_bytes, policy);
 
   V x[kSSlots];
   float y;
@@ -472,46 +349,26 @@ __global__ void __launch_bounds__(kStreamThreads, PBR_STREAM_BWD_MIN_CTAS) ct_ba
   for (int k = 0; k < ntiles; ++k) {
     const int s = k % kStages;
     const float* st = my_stages + s * my_stage_floats + w.toff;
-    if (!kPerWarp || w.seg_bytes > 0) mbar_wait(&full[s], (k / kStages) & 1);
+    if (w.seg_bytes > 0) mbar_wait(&full[s], (k / kStages) & 1);
 #pragma unroll
     for (int j = 0; j < kSSlots; ++j) {
       const float* sj = st + j * w.slot_stride;
       V a[3][1], n[3][1], r[1], m[3][1], gs[3];
 #pragma unroll
-      for (int c = 0; c < 3; ++c) a[c][0] = lds_v(sj + (SL::albedo + c) * kPlaneStride);
-      r[0] = lds_v(sj + SL::rough * kPlaneStride);
+      for (int c = 0; c < 3; ++c) a[c][0] = lds_v(sj + (SL::albedo + c) * kWarpSeg);
+      r[0] = lds_v(sj + SL::rough * kWarpSeg);
 #pragma unroll
-      for (int c = 0; c < 3; ++c) m[c][0] = c < SL::mc ? lds_v(sj + (SL::met + c) * kPlaneStride) : splat<V>(0.0f);
+      for (int c = 0; c < 3; ++c) m[c][0] = c < SL::mc ? lds_v(sj + (SL::met + c) * kWarpSeg) : splat<V>(0.0f);
 #pragma unroll
-      for (int c = 0; c < 3; ++c) gs[c] = lds_v(sj + (SL::gsrc + c) * kPlaneStride);   // grad_out, or the target image in loss mode
+      for (int c = 0; c < 3; ++c) gs[c] = lds_v(sj + (SL::gsrc + c) * kWarpSeg);   // grad_out, or the target image in loss mode
 #pragma unroll
-      for (int c = 0; c < 3; ++c) n[c][0] = has_normal ? lds_v(sj + (SL::normal + c) * kPlaneStride) : splat<V>(c == 2 ? 1.0f : 0.0f);
+      for (int c = 0; c < 3; ++c) n[c][0] = has_normal ? lds_v(sj + (SL::normal + c) * kWarpSeg) : splat<V>(c == 2 ? 1.0f : 0.0f);
       if (j == kSSlots - 1) {
-        // last read of the stage by this warp: refill it (per-warp pipelines) or tell the producer (no CTA-wide
-        // barrier - warps drift freely)
+        // last read of the stage by this warp: refill it (no CTA-wide barrier - warps drift freely)
         __syncwarp();
-        if (kPerWarp) {
-          if (!kLateRefill && w.seg_bytes > 0 && k + kStages < ntiles) {
-            fence_proxy_async();
-            warp_issue(sh, &full[s], my_stages + s * my_stage_floats, b0 + k + kStages, row_in_tile, w.wcol, w.seg_bytes, policy);
-          }
-        } else if (kLastRefill) {
-          int last = 0;
-          if ((tid & 31) == 0) {
-            __threadfence_block();
-            last = atomicAdd(&sh.readers[s], 1) == kStreamThreads / 32 - 1;
-          }
-          last = __shfl_sync(0xffffffffu, last, 0);
-          if (last) {   // warp-uniform: every warp has read the stage
-            if ((tid & 31) == 0) sh.readers[s] = 0;
-            if (k + kStages < ntiles) {
-              fence_proxy_async();
-              stream_issue(sh, &sh.full[s], stream_smem + s * stage_floats, b0 + k + kStages, w.rows_valid, w.seg_bytes,
-                           w.row_floats, policy, tid & 31);
-            }
-          }
-        } else if ((tid & 31) == 0) {
-          mbar_arrive(&sh.empty[s]);
+        if (w.seg_bytes > 0 && k + kStages < ntiles) {
+          fence_proxy_async();
+          warp_issue(sh, &full[s], my_stages + s * my_stage_floats, b0 + k + kStages, row_in_tile, w.wcol, w.seg_bytes, policy);
         }
       }
       if (kFast || slot_active(w, j, p.W)) {
@@ -536,15 +393,8 @@ __global__ void __launch_bounds__(kStreamThreads, PBR_STREAM_BWD_MIN_CTAS) ct_ba
           }
         };
         V da[3][1], dn[3][1], dr[1], dm[3][1];
-#if defined(PBR_DBG_NOMATH)   // memory pipeline only (tools/build_variants.py "nomath"): results are meaningless
-#pragma unroll
-        for (int c = 0; c < 3; ++c) { da[c][0] = a[c][0] + gs[c]; dn[c][0] = n[c][0] + hgs[0].lx; dm[c][0] = m[c][0] + xs[0]; }
-        dr[0] = r[0];
-        (void)gout; (void)int_sink;
-#else
         ct_backward_group<WF, kLight, V, 1>(S, stream_flags<kFast>(p.flags), a, n, r, m, xs, y, hgs, gout, int_sink, da, dn, dr, dm, NoFetch(), GeomCache<V>(),
                                             NoGeomSink(), NoSavedOut(), kIntGrad);
-#endif
         const int jo = j * w.slot_stride;
         if (kFast || o_a) {
 #pragma unroll
@@ -561,21 +411,10 @@ __global__ void __launch_bounds__(kStreamThreads, PBR_STREAM_BWD_MIN_CTAS) ct_ba
         }
       }
     }
-    if (kPerWarp && kLateRefill && w.seg_bytes > 0 && k + kStages < ntiles) {
-      __syncwarp();
-      fence_proxy_async();
-      warp_issue(sh, &full[s], my_stages + s * my_stage_floats, b0 + k + kStages, row_in_tile, w.wcol, w.seg_bytes, policy);
-    }
     if (kFast || o_a) o_a += p.d_albedo.sb;
     if (kFast || o_n) o_n += p.d_normal.sb;
     if (kFast || o_r) o_r += p.d_roughness.sb;
     if (kFast || o_m) o_m += p.d_metspec.sb;
-    // producer: by the time warp 0 has shaded tile k every warp has long since read stage s
-    if (!kPerWarp && !kLastRefill && tid < 32 && k + kStages < ntiles) {
-      mbar_wait(&sh.empty[s], (k / kStages) & 1);
-      stream_issue(sh, &sh.full[s], stream_smem + s * stage_floats, b0 + k + kStages, w.rows_valid, w.seg_bytes,
-                   w.row_floats, policy, tid);
-    }
   }
 
   // CTA-level reductions: warp shuffle -> shared -> ONE atomic per CTA and value

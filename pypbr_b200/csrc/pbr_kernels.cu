@@ -12,7 +12,6 @@
 
 #include <atomic>
 #include <climits>
-#include <cstdlib>
 
 #include "../../include/pbrcuda.h"
 #include "pbr_shade.cuh"
@@ -29,27 +28,11 @@
 
 namespace pbr {
 
-#ifndef PBR_THREADS
-#define PBR_THREADS 256
-#endif
-#ifndef PBR_FWD_MIN_CTAS
-#define PBR_FWD_MIN_CTAS 4   // __launch_bounds__ minBlocksPerSM hints (register caps), tuned on the GPU (profiles/)
-#endif
-#ifndef PBR_BWD_MIN_CTAS
-#define PBR_BWD_MIN_CTAS 3
-#endif
-#ifndef PBR_HOIST_MATS
-#define PBR_HOIST_MATS 16    // materials a thread walks over when the light geometry is hoisted
-#endif
-#ifndef PBR_TEXELS
-#define PBR_TEXELS 4         // texels per thread: 4 (float4 per plane), 2 (float2) or 1 (scalar, coalesced per warp)
-#endif
-constexpr int kTexels = PBR_TEXELS;     // texels per thread
-constexpr int kThreads = PBR_THREADS;   // threads per CTA of the streaming kernels (conversions, blend, colour, normals)
-#ifndef PBR_CT_THREADS
-#define PBR_CT_THREADS 128   // threads per CTA of the generic Cook-Torrance kernels (168 registers x 3 CTAs per SM in the backward)
-#endif
-constexpr int kCtThreads = PBR_CT_THREADS;
+constexpr int kFwdMinCtas = 4;   // __launch_bounds__ minBlocksPerSM hints (register caps), tuned on the GPU (profiles/)
+constexpr int kBwdMinCtas = 3;
+constexpr int kTexels = 4;       // texels per thread of the streaming kernels (float4 per plane)
+constexpr int kThreads = 256;    // threads per CTA of the streaming kernels (conversions, blend, colour, normals)
+constexpr int kCtThreads = 128;  // threads per CTA of the generic Cook-Torrance kernels (168 registers x 3 CTAs per SM in the backward)
 
 static std::atomic<uint64_t> g_launches{0};
 
@@ -114,25 +97,13 @@ __device__ __forceinline__ Where locate(int H, int W, bool vec_ok) { return loca
 // ------------------------------------------------------------------------------------------------
 // A thread of the generic kernels owns kCtTexels consecutive texels of one row, shaded as kSlots = kCtTexels/2
 // packed pairs (V = f2: FFMA2/FMUL2/FADD2).  One pair per thread keeps the adjoint's working set in registers.
-#ifndef PBR_CT_TEXELS
-#define PBR_CT_TEXELS 2
-#endif
-constexpr int kCtTexels = PBR_CT_TEXELS;
-// -DPBR_SCALAR_LANES builds the one-texel-per-lane flavour (V = float) for A/B accuracy and speed checks.
-#if defined(PBR_SCALAR_LANES)
-typedef float V;
-#else
+constexpr int kCtTexels = 2;
 typedef f2 V;
-#endif
 constexpr int kLanes = Lanes<V>::n;
 static_assert(kCtTexels % kLanes == 0, "texels per thread must be a multiple of the lane count");
 constexpr int kSlots = kCtTexels / kLanes;
-#ifndef PBR_FWD_GROUP
-#define PBR_FWD_GROUP 1   // pairs shaded together (ILP) by the generic forward kernel
-#endif
-#ifndef PBR_BWD_GROUP
-#define PBR_BWD_GROUP 1   // ... by the generic backward kernel (register pressure)
-#endif
+constexpr int kFwdGroup = 1;   // pairs shaded together (ILP) by the generic forward kernel
+constexpr int kBwdGroup = 1;   // ... by the generic backward kernel (register pressure)
 
 // torch.optim.Adam (single-tensor path): m = lerp(m, g, 1-b1); v = v*b2 + (1-b2)*g*g;
 // p -= (lr / (1-b1^t)) * m / (sqrt(v)/sqrt(1-b2^t) + eps).  Shared by adam_kernel and the fused fit epilogue.
@@ -274,22 +245,11 @@ __device__ __forceinline__ void load_material(const CtKParams& p, const Where& w
 // The maps of the NEXT material of the walk are pulled into L2 while the current one is shaded (one request per 128-byte
 // line: a warp's row segment of a plane is 256 bytes), so the loads at the top of the next iteration hit L2 instead of
 // waiting for HBM.  No registers, no shared memory (the multi-light kernels have neither to spare).
-#ifndef PBR_BWD_LATE_PREFETCH
-#define PBR_BWD_LATE_PREFETCH 0   // measured: +1.6 % on C3, -3 % on the C5 fit kernel (same instantiation, per-light mode) -> off
-#endif
-constexpr bool kBwdLatePrefetch = PBR_BWD_LATE_PREFETCH != 0;
-#ifndef PBR_FWD_REG_PREFETCH
-#define PBR_FWD_REG_PREFETCH 1
-#endif
-constexpr bool kFwdRegPrefetch = PBR_FWD_REG_PREFETCH != 0;
-#ifndef PBR_PREFETCH_NEXT
-#define PBR_PREFETCH_NEXT 1
-#endif
 __device__ __forceinline__ void prefetch_l2(const float* p) { asm volatile("prefetch.global.L2 [%0];" ::"l"(p)); }
 
 template <int WF, bool kVec>
 __device__ __forceinline__ void prefetch_material(const CtKParams& p, const Where& w, int b, bool has_normal) {
-  if (!PBR_PREFETCH_NEXT || ((threadIdx.x * kCtTexels) & 31) != 0) return;   // first thread of every 128-byte line
+  if (((threadIdx.x * kCtTexels) & 31) != 0) return;   // first thread of every 128-byte line
 #pragma unroll
   for (int c = 0; c < 3; ++c) prefetch_l2(at<kVec>(p.albedo, b, c, w));
   if (has_normal) {
@@ -359,12 +319,9 @@ __device__ __forceinline__ void grid_coords(const CtStage& S, const Where& w, in
 }
 
 // Register budget of the generic forward: the cached multi-light flavours take the full budget (2 CTAs per SM): registers buy
-// them more than occupancy does (tools/tune.py, 16 x 1024^2: L = 16 0.810 -> 0.771 ms, L = 8 0.403 -> 0.390, L = 4 0.227 -> 0.222;
+// them more than occupancy does (bare C ABI, 16 x 1024^2: L = 16 0.810 -> 0.771 ms, L = 8 0.403 -> 0.390, L = 4 0.227 -> 0.222;
 // unrolling the light loop on top of it is slower again), the memory-bound single-light / uncached flavours keep 4 CTAs.
-#ifndef PBR_FWD_CACHED_MIN_CTAS
-#define PBR_FWD_CACHED_MIN_CTAS 2
-#endif
-constexpr int fwd_min_ctas(int light_mode) { return is_cached(light_mode) ? PBR_FWD_CACHED_MIN_CTAS : PBR_FWD_MIN_CTAS; }
+constexpr int fwd_min_ctas(int light_mode) { return is_cached(light_mode) ? 2 : kFwdMinCtas; }
 
 // Plain-case flavours of the generic kernels (template parameter kFM, round 2): like kFast of the streamed kernels, the host picks
 // them when the launch is what the reference's defaults produce - sRGB albedo and output, a normal map, 64-bit accesses - and
@@ -378,14 +335,7 @@ constexpr int fwd_min_ctas(int light_mode) { return is_cached(light_mode) ? PBR_
 // kernel waits on the per-light encode / slope chains (MUFU) at 8 warps per SM, not on instruction issue: not kept.)
 
 enum { kFmGeneric = 0, kFmAccum = 1 };
-#ifndef PBR_GENERIC_FAST
-#define PBR_GENERIC_FAST 1
-#endif
-constexpr bool kGenericFast = PBR_GENERIC_FAST != 0;
-#ifndef PBR_PLAIN_UNROLL
-#define PBR_PLAIN_UNROLL 2   // light-loop unrolling of the plain-case flavours
-#endif
-constexpr int kPlainUnroll = PBR_PLAIN_UNROLL;
+constexpr int kPlainUnroll = 2;   // light-loop unrolling of the plain-case flavours
 template <int kFM>
 __device__ __forceinline__ CtFlags plain_flags(const CtFlags& f) {
   CtFlags F = f;
@@ -399,7 +349,7 @@ __device__ __forceinline__ CtFlags plain_flags(const CtFlags& f) {
 
 template <int WF, int kLight, bool kVec = true, int kFM = kFmGeneric>
 __global__ void __launch_bounds__(kCtThreads, fwd_min_ctas(kLight)) ct_forward_kernel(const __grid_constant__ CtKParams p) {
-  constexpr int G = PBR_FWD_GROUP;
+  constexpr int G = kFwdGroup;
   __shared__ CtStage S;
   stage_params(p, S);
   const Where w = locate_ct<kVec>(p);
@@ -419,21 +369,16 @@ __global__ void __launch_bounds__(kCtThreads, fwd_min_ctas(kLight)) ct_forward_k
   // are loaded into a second register set while the current one is shaded (the backward, at 235 registers, prefetches
   // into L2 instead).
   float nx_a[3][kCtTexels], nx_n[3][kCtTexels], nx_r[kCtTexels], nx_m[3][kCtTexels];
-  if (kFwdRegPrefetch) load_material<WF, kVec>(p, w, b0, nx_a, nx_n, nx_r, nx_m, has_normal);
+  load_material<WF, kVec>(p, w, b0, nx_a, nx_n, nx_r, nx_m, has_normal);
   for (int b = b0; b < b1; ++b) {
     float araw[3][kCtTexels], nraw[3][kCtTexels], rough[kCtTexels], mraw[3][kCtTexels];
-    if (kFwdRegPrefetch) {
 #pragma unroll
-      for (int i = 0; i < kCtTexels; ++i) {
+    for (int i = 0; i < kCtTexels; ++i) {
 #pragma unroll
-        for (int c = 0; c < 3; ++c) { araw[c][i] = nx_a[c][i]; nraw[c][i] = nx_n[c][i]; mraw[c][i] = nx_m[c][i]; }
-        rough[i] = nx_r[i];
-      }
-      if (b + 1 < b1) load_material<WF, kVec>(p, w, b + 1, nx_a, nx_n, nx_r, nx_m, has_normal);
-    } else {
-      load_material<WF, kVec>(p, w, b, araw, nraw, rough, mraw, has_normal);
-      if (b + 1 < b1) prefetch_material<WF, kVec>(p, w, b + 1, has_normal);
+      for (int c = 0; c < 3; ++c) { araw[c][i] = nx_a[c][i]; nraw[c][i] = nx_n[c][i]; mraw[c][i] = nx_m[c][i]; }
+      rough[i] = nx_r[i];
     }
+    if (b + 1 < b1) load_material<WF, kVec>(p, w, b + 1, nx_a, nx_n, nx_r, nx_m, has_normal);
     float outv[3][kCtTexels];
 #pragma unroll
     for (int s = 0; s < kSlots; s += G) {
@@ -471,14 +416,7 @@ __global__ void __launch_bounds__(kCtThreads, fwd_min_ctas(kLight)) ct_forward_k
   }
 }
 
-#ifndef PBR_COLD_UNROLL
-#define PBR_COLD_UNROLL 4   // measured: branching over the cold path (1) is not faster than predicating it
-#endif
-#ifndef PBR_PACKED_LOSS
-#define PBR_PACKED_LOSS 1
-#endif
-constexpr int kColdUnroll = PBR_COLD_UNROLL;
-constexpr bool kPackedLoss = PBR_PACKED_LOSS != 0;
+constexpr int kColdUnroll = 4;   // measured: branching over the cold path (1) is not faster than predicating it
 
 // per-thread asynchronous copies global -> shared (LDGSTS) for the backward kernel's grad_out / target ring
 constexpr int kRing = 4;
@@ -504,20 +442,14 @@ __device__ __forceinline__ float warp_sum(float v) {
 //   p.d_intensity : per-light intensity gradients, reduced the same way.
 // CTAs per SM the backward's register budget is sized for.  With the 6-field cache the shared memory already caps
 // the SM at 2-3 CTAs and the light loop is long: the full 255-register budget (no spills) beats a third CTA
-// (tools/tune.py, L = 8: 3.29 vs 3.80 ms; L = 16: 2.53 vs 2.99 ms).
-#ifndef PBR_BWD_CACHED_MIN_CTAS
-#define PBR_BWD_CACHED_MIN_CTAS 2
-#endif
+// (bare C ABI, L = 8: 3.29 vs 3.80 ms; L = 16: 2.53 vs 2.99 ms).
 constexpr int bwd_min_ctas(int light_mode) {
-  return (light_mode == kLightPointCached || light_mode == kLightPointCachedAllBig) ? PBR_BWD_CACHED_MIN_CTAS : PBR_BWD_MIN_CTAS;
+  return (light_mode == kLightPointCached || light_mode == kLightPointCachedAllBig) ? 2 : kBwdMinCtas;
 }
 // Light-loop unrolling of the general backward: by two where the full register budget is available (per-light loss kernel,
 // 32 x 1024^2: L = 8 2.654 -> 2.571 ms, L = 16 2.470 -> 2.393 ms; the 168-register flavours spill over it: L = 4 1.624 -> 1.794 ms).
-#ifndef PBR_BWD_BIG_UNROLL
-#define PBR_BWD_BIG_UNROLL 2
-#endif
 PBR_HDC int bwd_unroll(int light_mode) {
-  return (light_mode == kLightPointCached || light_mode == kLightPointCachedAllBig) ? PBR_BWD_BIG_UNROLL : kBwdUnroll;
+  return (light_mode == kLightPointCached || light_mode == kLightPointCachedAllBig) ? 2 : kBwdUnroll;
 }
 
 // The saved forward output of the row segment being back-propagated (PbrCtGrads.fwd_out).  It travels through slot 1 of
@@ -572,12 +504,12 @@ struct CtaGeomSink {
 template <int WF, int kLight, bool kGeom = false, bool kVec = true, int kFM = kFmGeneric>
 __global__ void __launch_bounds__(kCtThreads, kGeom ? 2 : bwd_min_ctas(kLight)) ct_backward_kernel(const __grid_constant__ CtKParams p) {
   static_assert(kFM == kFmGeneric || (!kGeom && kVec), "plain-case flavours: map gradients, 64-bit accesses");
-  constexpr int G = PBR_BWD_GROUP;
+  constexpr int G = kBwdGroup;
   __shared__ CtStage S;
   __shared__ float s_int[PBR_MAX_LIGHTS * 3];
   __shared__ float s_geo[kGeom ? (PBR_MAX_LIGHTS + 1) * 3 : 1];
   __shared__ float s_loss[kCtThreads / 32];
-  __shared__ __align__(16) float s_ring[kRing * 3 * kCtThreads * kLanes * PBR_BWD_GROUP];
+  __shared__ __align__(16) float s_ring[kRing * 3 * kCtThreads * kLanes * kBwdGroup];
   const int tid = threadIdx.y * blockDim.x + threadIdx.x;
   const CtFlags F = plain_flags<kFM>(p.flags);
   const bool int_grad = kFM != kFmGeneric ? false : p.d_intensity != nullptr;
@@ -618,24 +550,12 @@ __global__ void __launch_bounds__(kCtThreads, kGeom ? 2 : bwd_min_ctas(kLight)) 
   V loss_v = splat<V>(0.0f);   // squared error of the vector path, one partial sum per lane
   const int b0 = blockIdx.z * p.mats_per_cta;
   const int b1 = min(b0 + p.mats_per_cta, p.B);
-  // The maps of material b + 1 are requested when the light loop of material b is over - its ~70 registers are free by
-  // then - and land (from L2, where prefetch_material sent them) while the gradients of b are finished and stored.
-  // Only where it was measured to pay: the 255-register flavour in accumulate mode (L = 16: 2.49 -> 2.45 ms per
-  // 16 x 1024^2); the 168-register flavours spill over it (L = 4: 0.83 -> 1.02 ms), the per-light loss kernel is neutral.
-  const bool late_prefetch = kBwdLatePrefetch && kLight == kLightPointCached && !F.per_light;
-  float nx_a[3][kCtTexels], nx_n[3][kCtTexels], nx_r[kCtTexels], nx_m[3][kCtTexels];
+  // (Loading the maps of material b + 1 into registers once the light loop of b is over was measured for the 255-register
+  // cached flavour: +1.6 % on C3, -3 % on the C5 fit kernel, which runs the same instantiation in per-light mode; the
+  // 168-register flavours spill over it.  Not kept: the L2 prefetch below is all the backward does ahead.)
   for (int b = b0; b < b1; ++b) {
     float araw[3][kCtTexels], nraw[3][kCtTexels], rough[kCtTexels], mraw[3][kCtTexels];
-    if (late_prefetch && b > b0) {
-#pragma unroll
-      for (int i = 0; i < kCtTexels; ++i) {
-#pragma unroll
-        for (int c = 0; c < 3; ++c) { araw[c][i] = nx_a[c][i]; nraw[c][i] = nx_n[c][i]; mraw[c][i] = nx_m[c][i]; }
-        rough[i] = nx_r[i];
-      }
-    } else {
-      load_material<WF, kVec>(p, w, b, araw, nraw, rough, mraw, has_normal);
-    }
+    load_material<WF, kVec>(p, w, b, araw, nraw, rough, mraw, has_normal);
     if (b + 1 < b1) prefetch_material<WF, kVec>(p, w, b + 1, has_normal);
     if (adam_on) {
       // Fused fit step: what the Adam epilogue of THIS material needs (parameters and both moments of every channel)
@@ -712,10 +632,7 @@ __global__ void __launch_bounds__(kCtThreads, kGeom ? 2 : bwd_min_ctas(kLight)) 
         cp_async_commit();   // always: keeps the group count uniform
       };
       auto fetch = [&](int l) {
-        if (l < 0) {   // after the light loop
-          if (late_prefetch && s + G >= kSlots && b + 1 < b1) load_material<WF, kVec>(p, w, b + 1, nx_a, nx_n, nx_r, nx_m, has_normal);
-          return;
-        }
+        if (l < 0) return;   // after the light loop
         if (l == 0) {
 #pragma unroll
           for (int q = 0; q < kRing - 1; ++q) issue(q);
@@ -733,7 +650,7 @@ __global__ void __launch_bounds__(kCtThreads, kGeom ? 2 : bwd_min_ctas(kLight)) 
       };
       auto gout = [&](int l, const V(&outv)[3][G], V(&g)[3][G]) {
         take(l);
-        if (kPackedLoss && (kVec || w.vec)) {   // every lane is a live texel (uniform over the grid): packed arithmetic, no masks
+        if (kVec || w.vec) {   // every lane is a live texel (uniform over the grid): packed arithmetic, no masks
 #pragma unroll
           for (int c = 0; c < 3; ++c) {
             V t[G];
@@ -965,7 +882,7 @@ __device__ __forceinline__ void cam_setup(const CtKParams& p, const CtStage& S, 
 }
 
 template <int WF, int kLight>
-__global__ void __launch_bounds__(kCtThreads, PBR_FWD_MIN_CTAS) cam_forward_kernel(const __grid_constant__ CtKParams p) {
+__global__ void __launch_bounds__(kCtThreads, kFwdMinCtas) cam_forward_kernel(const __grid_constant__ CtKParams p) {
   __shared__ CtStage S;
   stage_params(p, S);
   const Where w = locate_ct<false>(p);
@@ -1404,46 +1321,32 @@ static int launch_result() {
 
 // Point light with L == 1: the light geometry of a texel is shared by every material of the batch,
 // so a thread walks over up to kHoistMats materials and computes it once.
-constexpr int kHoistMats = PBR_HOIST_MATS;
+constexpr int kHoistMats = 16;
 
 // Point lights with L > 1: the geometry of every light is computed once per texel pair, parked in shared memory
 // (GeomCache, pbr_shade.cuh) and reused by every material of the walk - it is ~55 % of the forward arithmetic of a
 // texel-light.  Worth it from two materials on, and while the cache leaves room for enough CTAs per SM.
-#ifndef PBR_GC_MAX_BYTES
-#define PBR_GC_MAX_BYTES (100 * 1024)   // L <= 16 with the 6-field cache: at least 2 CTAs per SM
-#endif
-#ifndef PBR_GC_ALL_MAX_LIGHTS
-#define PBR_GC_ALL_MAX_LIGHTS 4   // up to here all 8 geometry fields are cached and the backward keeps 3 CTAs per SM
-#endif
+constexpr size_t kGcMaxBytes = 100 * 1024;   // L <= 16 with the 6-field cache: at least 2 CTAs per SM
+constexpr int kGcAllMaxLights = 4;   // up to here all 8 geometry fields are cached and the backward keeps 3 CTAs per SM
+constexpr int kGcBigMaxLights = 8;   // backward, 4 < L <= 8: all 8 fields cached, full register budget (2 CTAs per SM by registers anyway)
 static size_t geom_cache_bytes(int L, int light_mode) { return (size_t)L * geom_fields(light_mode) * kSlots * kCtThreads * sizeof(V); }
-static bool vec_fast_disabled() {   // A/B and test switch: run the element-access flavour on shapes the fast one would take
-  static const bool off = [] { const char* e = getenv("PBR_DISABLE_VEC_FAST"); return e && e[0] && e[0] != '0'; }();
-  return off;
-}
-static bool geom_cache_disabled() {
-  static const bool off = [] { const char* e = getenv("PBR_DISABLE_GEOM_CACHE"); return e && e[0] && e[0] != '0'; }();
-  return off;
-}
 
-#ifndef PBR_GC_BIG_MAX_LIGHTS
-#define PBR_GC_BIG_MAX_LIGHTS 8   // backward, 4 < L <= 8: all 8 fields cached, full register budget (2 CTAs per SM by registers anyway)
-#endif
 static int light_mode(const CtKParams& k, bool backward) {
   if (!k.flags.point) return kLightDirectional;
   if (!k.vec_fast) return kLightPoint;              // the element-access flavour only exists for the uncached light modes
   if (k.d_lights || k.d_view) {
     // geometry gradients (shared parameters of a fit with unknown lighting): the 6-field cache when a walk over several
     // materials pays for it, else the per-texel geometry
-    if (backward && k.flags.L > 1 && k.B >= 2 && !geom_cache_disabled() &&
-        geom_cache_bytes(k.flags.L, kLightPointCached) <= (size_t)PBR_GC_MAX_BYTES) return kLightPointCached;
+    if (backward && k.flags.L > 1 && k.B >= 2 && geom_cache_bytes(k.flags.L, kLightPointCached) <= kGcMaxBytes)
+      return kLightPointCached;
     return kLightPoint;
   }
   if (k.flags.L == 1) return kLightPointHoisted;
-  if (k.B >= 2 && !geom_cache_disabled()) {
-    if (k.flags.L <= PBR_GC_ALL_MAX_LIGHTS) return kLightPointCachedAll;
+  if (k.B >= 2) {
+    if (k.flags.L <= kGcAllMaxLights) return kLightPointCachedAll;
     // (not under the Adam epilogue: with its 30 KB of staging the two CTAs would leave the SM almost no L1, 12.21 -> 12.35 ms on C5)
-    if (backward && !k.adam_on && k.flags.L <= PBR_GC_BIG_MAX_LIGHTS) return kLightPointCachedAllBig;
-    if (geom_cache_bytes(k.flags.L, kLightPointCached) <= (size_t)PBR_GC_MAX_BYTES) return kLightPointCached;
+    if (backward && !k.adam_on && k.flags.L <= kGcBigMaxLights) return kLightPointCachedAllBig;
+    if (geom_cache_bytes(k.flags.L, kLightPointCached) <= kGcMaxBytes) return kLightPointCached;
   }
   return kLightPoint;
 }
@@ -1456,7 +1359,7 @@ static void ct_launch_shape(CtKParams& k, dim3& grid, dim3& block, bool backward
 }
 
 // most dynamic shared memory a generic kernel is ever launched with: geometry cache + Adam staging (or the partial-sum slots)
-constexpr size_t kMaxDynSmem = (size_t)PBR_GC_MAX_BYTES + 30 * kCtThreads * kCtTexels * 4;
+constexpr size_t kMaxDynSmem = kGcMaxBytes + 30 * kCtThreads * kCtTexels * 4;
 // launch with `smem` bytes of dynamic shared memory (opt-in above 48 KB, once per kernel instantiation and device)
 template <void (*Kern)(CtKParams)>
 static void launch_dyn(const CtKParams& k, dim3 grid, dim3 block, size_t smem, cudaStream_t st) {
@@ -1479,14 +1382,9 @@ static int kernel_workflow(const PbrCtDesc* d) {
 
 // what the plain-case flavour (kFmAccum) assumes besides its own mode: the reference's default colour handling and a
 // normal map, on the 64-bit-access flavour
-static bool generic_fast_disabled() {   // A/B and test switch: run the general flavour where a plain-case one would be picked
-  static const bool off = [] { const char* e = getenv("PBR_DISABLE_GENERIC_FAST"); return e && e[0] && e[0] != '0'; }();
-  return off;
-}
 template <int WF>
 static bool plain_case(const CtKParams& k) {
-  return kGenericFast && !generic_fast_disabled() && k.vec_fast && k.flags.albedo_is_srgb && k.flags.return_srgb && (WF != 1 || k.flags.specular_is_srgb) &&
-         k.normal.ptr != nullptr;
+  return k.vec_fast && k.flags.albedo_is_srgb && k.flags.return_srgb && (WF != 1 || k.flags.specular_is_srgb) && k.normal.ptr != nullptr;
 }
 
 template <int WF>
@@ -1591,23 +1489,15 @@ static int fill_grads(const PbrCtGrads* g, CtKParams& k) {
 // ------------------------------------------------------------------------------------------------
 // streamed (TMA-fed) fast path: one light, 16-byte aligned planes, W % 4 == 0 (pbr_ct_stream.cuh)
 // ------------------------------------------------------------------------------------------------
-static bool stream_disabled() {
-  static const bool off = [] { const char* e = getenv("PBR_DISABLE_STREAM"); return e && e[0] && e[0] != '0'; }();
-  return off;
-}
-
 static bool fits_i32(const PbrPlane& pl, int H, int W) {
   return !pl.ptr || ((int64_t)(H - 1) * pl.sh + W) < (int64_t)INT32_MAX;
 }
 
-static bool stream_shape(const CtKParams& k, dim3& grid, dim3& block, int& mats, bool per_warp) {
-  if (stream_disabled() || k.force_generic || k.flags.L != 1 || !k.vec_ok || (k.W % 4) != 0) return false;
-  static const int min_bx = [] { const char* e = getenv("PBR_STREAM_MIN_BX"); int v = e ? atoi(e) : 1; return v < 1 ? 1 : v; }();
-  int groups = k.W / kST, bx = min_bx < 4 / kST ? 4 / kST : min_bx;   // a row segment is a multiple of 16 bytes
-  if (per_warp) {   // per-warp copy pipelines: a warp must sit inside one tile row
-    if (groups < 32) return false;   // narrower than one warp segment: the generic kernels take it
-    if (bx < 32) bx = 32;
-  }
+static bool stream_shape(const CtKParams& k, dim3& grid, dim3& block, int& mats) {
+  if (k.force_generic || k.flags.L != 1 || !k.vec_ok || (k.W % 4) != 0) return false;
+  const int groups = k.W / kST;
+  if (groups < 32) return false;   // narrower than one warp segment: the generic kernels take it
+  int bx = 32;                     // per-warp copy pipelines: a warp must sit inside one tile row
   while (bx < groups && bx < kStreamThreads) bx <<= 1;
   int by = kStreamThreads / bx;
   int64_t gy = ((int64_t)k.H + by - 1) / by;
@@ -1635,7 +1525,7 @@ static void stream_launch(const CtKParams& k, dim3 grid, dim3 block, int planes,
 template <int WF>
 static void launch_fwd_stream(const CtKParams& k, dim3 grid, dim3 block, cudaStream_t st) {
   const int planes = k.normal.ptr ? Slots<WF, false>::count : Slots<WF, false>::count_no_normal;
-  const bool fast = kStreamFast && block.x == (unsigned)kStreamThreads && block.y == 1 && (k.W % kTileFloats) == 0 && k.normal.ptr &&
+  const bool fast = block.x == (unsigned)kStreamThreads && block.y == 1 && (k.W % kTileFloats) == 0 && k.normal.ptr &&
                     k.flags.albedo_is_srgb && k.flags.return_srgb && (WF != 1 || k.flags.specular_is_srgb);
   if (fast) {
     if (k.flags.point) stream_launch<ct_forward_stream<WF, kLightPointHoisted, true>>(k, grid, block, planes, st);
@@ -1650,7 +1540,7 @@ template <int WF, int kMode>
 static void launch_bwd_stream_m(const CtKParams& k, dim3 grid, dim3 block, cudaStream_t st) {
   const int planes = k.normal.ptr ? Slots<WF, true>::count : Slots<WF, true>::count_no_normal;
   // the plain case (full tiles of one row, a normal map, every gradient requested) runs the kFast flavour (pbr_ct_stream.cuh)
-  const bool fast = kStreamFast && block.x == (unsigned)kStreamThreads && block.y == 1 && (k.W % kTileFloats) == 0 && k.normal.ptr &&
+  const bool fast = block.x == (unsigned)kStreamThreads && block.y == 1 && (k.W % kTileFloats) == 0 && k.normal.ptr &&
                     k.flags.albedo_is_srgb && k.flags.return_srgb && (WF != 1 || k.flags.specular_is_srgb) &&
                     k.d_albedo.ptr && k.d_normal.ptr && k.d_roughness.ptr && k.d_metspec.ptr;
   if (fast) {
@@ -1744,8 +1634,8 @@ static bool planes_fit_i32(const CtKParams& k) {
 static int ct_dispatch(CtKParams& k, int wf, bool backward, cudaStream_t st) {
   dim3 grid, block;
   int mats = 1;
-  k.vec_fast = k.vec_ok && (k.W % kCtTexels) == 0 && planes_fit_i32(k) && !vec_fast_disabled();
-  bool stream = stream_shape(k, grid, block, mats, backward ? kPerWarpBwd : kPerWarpFwd);
+  k.vec_fast = k.vec_ok && (k.W % kCtTexels) == 0 && planes_fit_i32(k);
+  bool stream = stream_shape(k, grid, block, mats);
   if (stream) {
     if (backward) stream = fits_i32(k.d_albedo, k.H, k.W) && fits_i32(k.d_normal, k.H, k.W) && fits_i32(k.d_roughness, k.H, k.W) && fits_i32(k.d_metspec, k.H, k.W);
     else stream = fits_i32(k.out, k.H, k.W);

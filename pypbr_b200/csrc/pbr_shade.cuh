@@ -6,22 +6,10 @@
 
 #include "pbr_math.cuh"
 
-// light-loop unrolling of the forward evaluation (independent chains for the scheduler), tuned on the GPU
-#ifndef PBR_FWD_UNROLL
-#define PBR_FWD_UNROLL 1
-#endif
-#ifndef PBR_P1_UNROLL
-#define PBR_P1_UNROLL 2
-#endif
-#ifndef PBR_BWD_UNROLL
-#define PBR_BWD_UNROLL 1   // main light loop of the backward
-#endif
-#ifndef PBR_BOUNDARY_RECOMPUTE
-#define PBR_BOUNDARY_RECOMPUTE 1   // one-pass accumulate backward: texels whose saved output sits at the clamp's upper end recompute the sum
-#endif
 namespace pbr {
-constexpr int kFwdUnroll = PBR_FWD_UNROLL, kP1Unroll = PBR_P1_UNROLL, kBwdUnroll = PBR_BWD_UNROLL;
-constexpr bool kBoundaryRecompute = PBR_BOUNDARY_RECOMPUTE != 0;
+// light-loop unrolling (independent chains for the scheduler), tuned on the GPU: the forward evaluation, pass 1 of the
+// two-pass backward, and the main light loop of the backward
+constexpr int kFwdUnroll = 1, kP1Unroll = 2, kBwdUnroll = 1;
 }
 #ifndef PBR_MAX_LIGHTS
 #define PBR_MAX_LIGHTS 64
@@ -202,7 +190,7 @@ PBR_HD void light_geom(const CtStage& S, int l, const V (&x)[N], float y, const 
 //   out within 5e-7 of the knee's image (sRGB only): the two branches of linear_to_srgb do not meet exactly at 0.0031308 -
 //                the power branch starts 7e-8 BELOW 12.92 * knee - so a sum just above the knee encodes to a value the
 //                linear branch also produces, and their slopes differ by 1.8 % (seen once in 12.6 M texels at the C3 shape).
-// Those texels recompute the sum (kBoundaryRecompute); everything else reads the slope off the output.
+// Those texels recompute the sum; everything else reads the slope off the output.
 constexpr float kKneeImage = 12.92f * kSrgbEncKnee;   // 0.040449936
 PBR_HD bool at_boundary(float v, float top, bool srgb) { return v >= top || (srgb && fabsf(v - kKneeImage) < 5e-7f); }
 PBR_HD bool at_boundary(f2 v, float top, bool srgb) { return at_boundary(v.x, top, srgb) || at_boundary(v.y, top, srgb); }
@@ -309,7 +297,7 @@ struct NoSavedOut {
 // d encode(clamp(acc)) / d acc from out = encode(clamp(acc)) (utils/functions.py:50-66 inverted on its upper branch:
 // t^(1/2.4 - 1) = u^-1.4 with u = (out + 0.055)/1.055).  out >= encode(1) - which is 0.99999994, not 1, in fp32:
 // 1.055 - 0.055 rounds down, in the reference too - is read as "the sum was clamped" here; the caller recomputes the sum
-// for exactly those texels (kBoundaryRecompute), because a sum of exactly 1 (torch.clamp's gate is inclusive) and the one
+// for exactly those texels (at_boundary), because a sum of exactly 1 (torch.clamp's gate is inclusive) and the one
 // or two fp32 sums just below it encode to the same number.
 template <class V>
 PBR_HD V encode_slope_from_out(V out, bool return_srgb) {
@@ -371,7 +359,7 @@ PBR_HD void ct_backward_group(const CtStage& S, const CtFlags& F, const V (&araw
 #pragma unroll
         for (int i = 0; i < N; ++i) {
           slope[c][i] = encode_slope_from_out(outv[c][i], F.return_srgb);
-          if (kBoundaryRecompute) recompute = recompute || at_boundary(outv[c][i], top, F.return_srgb);
+          recompute = recompute || at_boundary(outv[c][i], top, F.return_srgb);
         }
     }
     if (recompute) {
