@@ -12,6 +12,7 @@
 
 #include <atomic>
 #include <climits>
+#include <type_traits>
 
 #include "../../include/pbrcuda.h"
 #include "pbr_shade.cuh"
@@ -137,6 +138,7 @@ struct CtKParams {
   int vec_fast;          // host: the kVec = true flavour of the generic kernels applies (see locate_ct)
   int is_loss;           // backward: grad_out is derived from (render - target)
   int force_generic;     // PbrCtDesc.force_generic
+  int camera;            // host: `view` is a camera position (pbr_ct_*_camera): cam_forward_kernel / cam_backward_kernel
   PbrPlane albedo, normal, roughness, metspec, out;
   int64_t out_sl;
   // backward: `gsrc` is grad_out, or the target image when is_loss
@@ -285,13 +287,25 @@ __device__ __forceinline__ void unpair_to(const V (&src)[G], int s0, float (&dst
 // dynamic shared memory of the kLightPointCached* kernels: the geometry cache, L * geom_fields * kSlots * kCtThreads V's
 extern __shared__ __align__(16) unsigned char s_dyn[];
 
-template <int kLight>
-__device__ __forceinline__ void grid_coords(const CtStage& S, const Where& w, int L, V (&x)[kSlots], float& y,
-                                            LightGeomT<V> (&hg)[kSlots], GeomCache<V>& gc) {
+// The view a thread's lane-values are shaded with (pbr_shade.cuh).  OrthoView: the CTA-uniform direction of the stage,
+// nothing to fill.  LaneViews (kCam, pbr_ct_*_camera): a camera at a finite position c = PbrCtDesc.view, each texel's unit
+// view vector F.normalize(c - P) with P = (x, -y, 0) its plane position, and |c - P| for the adjoint.
+__device__ __forceinline__ void fill_views(const CtKParams&, const V (&)[kSlots], float, OrthoView&) {}
+__device__ __forceinline__ void fill_views(const CtKParams& p, const V (&x)[kSlots], float y, LaneViews<V, kSlots>& v) {
+  const float* cam = p.view_dev ? p.view_dev : p.view;
+  const float c[3] = {cam[0], cam[1], cam[2]};
+#pragma unroll
+  for (int i = 0; i < kSlots; ++i) camera_view(c, x[i], y, v.x[i], v.y[i], v.z[i], v.len[i]);
+}
+
+// Per-texel set-up of the generic kernels: plane coordinates, views, and the light geometry that does not depend on the
+// material, computed once and reused by every material of the walk.
+template <int kLight, class View>
+__device__ __forceinline__ void grid_coords(const CtKParams& p, const CtStage& S, const Where& w, V (&x)[kSlots], float& y,
+                                            View& views, LightGeomT<V> (&hg)[kSlots], GeomCache<V>& gc) {
   gc.base = reinterpret_cast<V*>(s_dyn) + (threadIdx.y * blockDim.x + threadIdx.x);
   gc.stride = kCtThreads;
   gc.fstride = kSlots * kCtThreads;
-  (void)L;
 #pragma unroll
   for (int i = 0; i < kSlots; ++i)
 #pragma unroll
@@ -300,14 +314,16 @@ __device__ __forceinline__ void grid_coords(const CtStage& S, const Where& w, in
       lane_set(x[i], k, linspace_at(S.lsx, col < S.lsx.n ? col : S.lsx.n - 1));
     }
   y = linspace_at(S.lsy, w.row);
+  fill_views(p, x, y, views);
   if (kLight == kLightPointHoisted) {
 #pragma unroll
     for (int i = 0; i < kSlots; ++i)
-      point_light_geom(S.light[0].p[0], S.light[0].p[1], S.light[0].p[2], x[i], y, S.vx, S.vy, S.vz, hg[i]);
+      point_light_geom(S.light[0].p[0], S.light[0].p[1], S.light[0].p[2], x[i], y, view_x(S, views, i), view_y(S, views, i),
+                       view_z(S, views, i), hg[i]);
   }
   if (is_cached(kLight)) {
     // every light's geometry once per texel pair, reused by all the materials this thread walks over
-    for (int l = 0; l < L; ++l) {
+    for (int l = 0; l < p.flags.L; ++l) {
 #pragma unroll
       for (int i = 0; i < kSlots; ++i) {
         LightGeomT<V> g;
@@ -347,8 +363,22 @@ __device__ __forceinline__ CtFlags plain_flags(const CtFlags& f) {
   return F;
 }
 
-template <int WF, int kLight, bool kVec = true, int kFM = kFmGeneric>
-__global__ void __launch_bounds__(kCtThreads, fwd_min_ctas(kLight)) ct_forward_kernel(const __grid_constant__ CtKParams p) {
+// The generic kernels are one body per direction (ct_forward_body / ct_backward_body) behind two sets of entry points with
+// stable names: ct_{forward,backward}_kernel (kCam = false, the orthographic view of the reference) and
+// cam_{forward,backward}_kernel (kCam = true, pbr_ct_*_camera: the view is LaneViews<V, kSlots> instead of OrthoView).
+// The camera exists for the general flavour with element accesses, the uncached per-texel light modes and one group of
+// kSlots lane-values per thread (the group takes the thread's views as they are); its backward always computes the geometry
+// adjoints, because the camera gradient runs through h, N.V and the Fresnel term.
+PBR_HDC bool cam_ok(int light_mode, bool vec, int fm) {
+  return !vec && fm == kFmGeneric && (light_mode == kLightDirectional || light_mode == kLightPoint ||
+                                      light_mode == kLightPointHoisted) && kFwdGroup == kSlots && kBwdGroup == kSlots;
+}
+template <bool kCam>
+using ViewT = typename std::conditional<kCam, LaneViews<V, kSlots>, OrthoView>::type;
+
+template <int WF, int kLight, bool kVec, int kFM, bool kCam>
+__device__ __forceinline__ void ct_forward_body(const CtKParams& p) {
+  static_assert(!kCam || cam_ok(kLight, kVec, kFM), "camera: see cam_ok");
   constexpr int G = kFwdGroup;
   __shared__ CtStage S;
   stage_params(p, S);
@@ -359,9 +389,10 @@ __global__ void __launch_bounds__(kCtThreads, fwd_min_ctas(kLight)) ct_forward_k
 
   V x[kSlots];
   float y;
+  ViewT<kCam> views;
   LightGeomT<V> hg[kSlots];
   GeomCache<V> gc;
-  grid_coords<kLight>(S, w, p.flags.L, x, y, hg, gc);
+  grid_coords<kLight>(p, S, w, x, y, views, hg, gc);
 
   const int b0 = blockIdx.z * p.mats_per_cta;
   const int b1 = min(b0 + p.mats_per_cta, p.B);
@@ -406,7 +437,8 @@ __global__ void __launch_bounds__(kCtThreads, fwd_min_ctas(kLight)) ct_forward_k
       GeomCache<V> gcs = gc;   // lane-value i of the group is lane-value s + i of the thread
       gcs.base += s * gc.stride;
       // plain-case flavour: the light loop is one basic block, two lights interleave (L = 16: 0.717 -> 0.696 ms per 16 x 1024^2)
-      ct_forward_group<WF, kLight, V, G, decltype(emit), (kFM != kFmGeneric ? kPlainUnroll : kFwdUnroll)>(S, F, a, n, r, m, xs, y, hgs, emit, gcs);
+      ct_forward_group<WF, kLight, V, G, decltype(emit), (kFM != kFmGeneric ? kPlainUnroll : kFwdUnroll)>(S, F, a, n, r, m, xs, y, hgs, emit, gcs,
+                                                                                                          views);
     }
     if (!F.per_light) {
 #pragma unroll
@@ -414,6 +446,15 @@ __global__ void __launch_bounds__(kCtThreads, fwd_min_ctas(kLight)) ct_forward_k
         store_seg<kCtTexels>(at<kVec>(p.out, b, c, w), w.vec, w.valid, outv[c]);
     }
   }
+}
+
+template <int WF, int kLight, bool kVec = true, int kFM = kFmGeneric>
+__global__ void __launch_bounds__(kCtThreads, fwd_min_ctas(kLight)) ct_forward_kernel(const __grid_constant__ CtKParams p) {
+  ct_forward_body<WF, kLight, kVec, kFM, false>(p);
+}
+template <int WF, int kLight>
+__global__ void __launch_bounds__(kCtThreads, fwd_min_ctas(kLight)) cam_forward_kernel(const __grid_constant__ CtKParams p) {
+  ct_forward_body<WF, kLight, false, kFmGeneric, true>(p);
 }
 
 constexpr int kColdUnroll = 4;   // measured: branching over the cold path (1) is not faster than predicating it
@@ -499,11 +540,13 @@ struct CtaGeomSink {
   __device__ __forceinline__ void view(const float (&g)[3]) const { add(L, g); }
 };
 
-// kGeom: also d/d(light position | direction) and d/d(view direction) (PbrCtGrads.d_lights / d_view), which the
-// reference delivers through plain autograd (cooktorrance.py:95,125-140).  Uncached per-texel light modes only.
-template <int WF, int kLight, bool kGeom = false, bool kVec = true, int kFM = kFmGeneric>
-__global__ void __launch_bounds__(kCtThreads, kGeom ? 2 : bwd_min_ctas(kLight)) ct_backward_kernel(const __grid_constant__ CtKParams p) {
+// kGeom: also d/d(light position | direction) and d/d(view direction | camera position) (PbrCtGrads.d_lights / d_view),
+// which the reference delivers through plain autograd (cooktorrance.py:95,125-140).
+// kCam: accumulate mode with L > 1 runs the two-pass backward (no saved forward output); no Adam epilogue.
+template <int WF, int kLight, bool kGeom, bool kVec, int kFM, bool kCam>
+__device__ __forceinline__ void ct_backward_body(const CtKParams& p) {
   static_assert(kFM == kFmGeneric || (!kGeom && kVec), "plain-case flavours: map gradients, 64-bit accesses");
+  static_assert(!kCam || (kGeom && cam_ok(kLight, kVec, kFM)), "camera: see cam_ok");
   constexpr int G = kBwdGroup;
   __shared__ CtStage S;
   __shared__ float s_int[PBR_MAX_LIGHTS * 3];
@@ -514,7 +557,7 @@ __global__ void __launch_bounds__(kCtThreads, kGeom ? 2 : bwd_min_ctas(kLight)) 
   const CtFlags F = plain_flags<kFM>(p.flags);
   const bool int_grad = kFM != kFmGeneric ? false : p.d_intensity != nullptr;
   const bool is_loss = kFM != kFmGeneric ? false : p.is_loss != 0;
-  const bool adam_on = kFM != kFmGeneric ? false : p.adam_on != 0;
+  const bool adam_on = (kFM != kFmGeneric || kCam) ? false : p.adam_on != 0;
   const bool has_normal = kFM != kFmGeneric || p.normal.ptr != nullptr;
   const bool part_on = kFM != kFmGeneric ? false : p.part_on != 0;
   if (int_grad) {
@@ -540,9 +583,10 @@ __global__ void __launch_bounds__(kCtThreads, kGeom ? 2 : bwd_min_ctas(kLight)) 
 
   V x[kSlots];
   float y;
+  ViewT<kCam> views;
   LightGeomT<V> hg[kSlots];
   GeomCache<V> gc;
-  grid_coords<kLight>(S, w, p.flags.L, x, y, hg, gc);
+  grid_coords<kLight>(p, S, w, x, y, views, hg, gc);
   // Adam staging of the fused fit step: [channel slot][p | m | v][thread][texel], this thread's column
   float* const s_adam = reinterpret_cast<float*>(s_dyn + p.adam_smem_off) + tid * kCtTexels;
 
@@ -610,7 +654,7 @@ __global__ void __launch_bounds__(kCtThreads, kGeom ? 2 : bwd_min_ctas(kLight)) 
       float* ring = s_ring + tid * NT;   // [slot][channel][thread][NT]
       const int nl_src = F.per_light ? F.L : 1;
       const float* const gbase = at<kVec>(p.gsrc, b, 0, w, kLanes * s);   // once per material
-      const bool have_fout = kFM == kFmAccum ? true : p.fout.ptr != nullptr;   // accumulate mode only (nl_src == 1): slot 1 carries the saved forward output
+      const bool have_fout = kFM == kFmAccum ? true : !kCam && p.fout.ptr != nullptr;   // accumulate mode only (nl_src == 1): slot 1 carries the saved forward output
       const float* const fbase = have_fout ? at<kVec>(p.fout, b, 0, w, kLanes * s) : nullptr;
       auto issue = [&](int l) {
         const bool saved = have_fout && l == 1;
@@ -704,7 +748,8 @@ __global__ void __launch_bounds__(kCtThreads, kGeom ? 2 : bwd_min_ctas(kLight)) 
       gcs.base += s * gc.stride;
       if constexpr (kGeom) {
         ct_backward_group<WF, kLight, V, G>(S, F, a, n, r, m, xs, y, hgs, gout, int_sink, da, dn, dr, dm, fetch, gcs,
-                                            CtaGeomSink{s_geo, p.flags.L, tid, live, s_part}, CtaSavedOut{ring + 3 * (kCtThreads * NT), have_fout}, int_grad);
+                                            CtaGeomSink{s_geo, p.flags.L, tid, live, s_part}, CtaSavedOut{ring + 3 * (kCtThreads * NT), have_fout}, int_grad,
+                                            views);
       } else {
         // (plain-case flavour, light loop unrolled by two: L = 16 1.570 -> 1.549 ms, L = 8 0.916 -> 0.886 ms per 16 x 1024^2)
         ct_backward_group<WF, kLight, V, G, decltype(gout), decltype(int_sink), decltype(fetch), NoGeomSink, CtaSavedOut,
@@ -826,7 +871,8 @@ __global__ void __launch_bounds__(kCtThreads, kGeom ? 2 : bwd_min_ctas(kLight)) 
   if (is_loss || int_grad || kGeom) __syncthreads();
   if (kGeom) {
     // one thread per light (and one for the view) turns the CTA's partial sums into gradients of the RAW parameters:
-    // the Jacobians of F.normalize(dir) / F.normalize(view) are constant over the image, hence applied here, once
+    // the Jacobians of F.normalize(dir) / F.normalize(view) are constant over the image, hence applied here, once (the
+    // camera's sum is already w.r.t. its position: camera_view_bwd per texel)
     const float* view = p.view_dev ? p.view_dev : p.view;
     const float* lights = p.lights_dev ? p.lights_dev : p.lights;
     if (tid <= p.flags.L) {
@@ -834,7 +880,7 @@ __global__ void __launch_bounds__(kCtThreads, kGeom ? 2 : bwd_min_ctas(kLight)) 
       float o[3] = {g[0], g[1], g[2]};
       float* dst = nullptr;
       if (tid == p.flags.L) {
-        normalize_bwd(view, g, o);
+        if (!kCam) normalize_bwd(view, g, o);
         dst = p.d_view;
       } else {
         if (!p.flags.point) normalize_bwd(lights + 3 * tid, g, o);
@@ -857,181 +903,13 @@ __global__ void __launch_bounds__(kCtThreads, kGeom ? 2 : bwd_min_ctas(kLight)) 
   }
 }
 
-// ------------------------------------------------------------------------------------------------
-// Camera at a finite position (pbr_ct_*_camera): the view vector of a texel is F.normalize(c - P) with c = PbrCtDesc.view
-// and P = (x, -y, 0) its plane position, instead of the one CTA-uniform direction of the ct_* kernels.
-// The design of the generic kernels: V = f2, kCtThreads threads, a walk over up to kHoistMats materials, element-access
-// loads and stores (any alignment and width).  The view vectors - and, for one point light, its geometry - are computed
-// once per texel and reused by every material of the walk (they do not depend on the material).  Light modes:
-// kLightDirectional (l is image-constant, h and (1 - h.v)^5 per texel), kLightPointHoisted (L == 1) and kLightPoint.
-// The backward always computes the geometry adjoints (the camera gradient runs through h, N.V and the Fresnel term).
-// ------------------------------------------------------------------------------------------------
-template <int kLight>
-__device__ __forceinline__ void cam_setup(const CtKParams& p, const CtStage& S, const Where& w, V (&x)[kSlots], float& y,
-                                          LaneViews<V, kSlots>& cv, LightGeomT<V> (&hg)[kSlots]) {
-  GeomCache<V> gc;
-  grid_coords<kLightPoint>(S, w, p.flags.L, x, y, hg, gc);   // the plane coordinates only
-  const float* cam = p.view_dev ? p.view_dev : p.view;
-  const float c[3] = {cam[0], cam[1], cam[2]};
-#pragma unroll
-  for (int i = 0; i < kSlots; ++i) {
-    camera_view(c, x[i], y, cv.x[i], cv.y[i], cv.z[i], cv.len[i]);
-    if (kLight == kLightPointHoisted)
-      point_light_geom(S.light[0].p[0], S.light[0].p[1], S.light[0].p[2], x[i], y, cv.x[i], cv.y[i], cv.z[i], hg[i]);
-  }
+template <int WF, int kLight, bool kGeom = false, bool kVec = true, int kFM = kFmGeneric>
+__global__ void __launch_bounds__(kCtThreads, kGeom ? 2 : bwd_min_ctas(kLight)) ct_backward_kernel(const __grid_constant__ CtKParams p) {
+  ct_backward_body<WF, kLight, kGeom, kVec, kFM, false>(p);
 }
-
-template <int WF, int kLight>
-__global__ void __launch_bounds__(kCtThreads, kFwdMinCtas) cam_forward_kernel(const __grid_constant__ CtKParams p) {
-  __shared__ CtStage S;
-  stage_params(p, S);
-  const Where w = locate_ct<false>(p);
-  if (!w.active) return;
-  const CtFlags& F = p.flags;
-  const bool has_normal = p.normal.ptr != nullptr;
-  V x[kSlots];
-  float y;
-  LaneViews<V, kSlots> cv;
-  LightGeomT<V> hg[kSlots];
-  cam_setup<kLight>(p, S, w, x, y, cv, hg);
-
-  const int b0 = blockIdx.z * p.mats_per_cta;
-  const int b1 = min(b0 + p.mats_per_cta, p.B);
-  for (int b = b0; b < b1; ++b) {
-    float araw[3][kCtTexels], nraw[3][kCtTexels], rough[kCtTexels], mraw[3][kCtTexels];
-    load_material<WF, false>(p, w, b, araw, nraw, rough, mraw, has_normal);
-    if (b + 1 < b1) prefetch_material<WF, false>(p, w, b + 1, has_normal);
-    V a[3][kSlots], n[3][kSlots], r[kSlots], m[3][kSlots];
-    pairs_of3<kSlots>(araw, 0, a); pairs_of3<kSlots>(nraw, 0, n); pairs_of3<kSlots>(mraw, 0, m); pairs_of<kSlots>(rough, 0, r);
-    auto emit = [&](int l, const V(&v)[3][kSlots]) {   // light l (per-light mode) or the accumulated image (l = 0)
-#pragma unroll
-      for (int c = 0; c < 3; ++c) {
-        float tv[kCtTexels];
-        unpair_to<kSlots>(v[c], 0, tv);
-        store_seg<kCtTexels>(at<false>(p.out, b, c, w) + (F.per_light ? (int64_t)l * p.out_sl : 0), w.vec, w.valid, tv);
-      }
-    };
-    ct_forward_group<WF, kLight, V, kSlots, decltype(emit), kFwdUnroll, LaneViews<V, kSlots>>(S, F, a, n, r, m, x, y, hg, emit,
-                                                                                                GeomCache<V>(), cv);
-  }
-}
-
-// Backward / fused loss (p.is_loss), with d_intensity, d_lights and d_view (= d camera position) when their pointers are
-// set.  Accumulate mode with L > 1 runs the two-pass backward (the summed image is recomputed).  The shared-parameter
-// gradients go warp shuffle -> shared atomics per light, and one global atomic per CTA and value.
 template <int WF, int kLight>
 __global__ void __launch_bounds__(kCtThreads, 2) cam_backward_kernel(const __grid_constant__ CtKParams p) {
-  __shared__ CtStage S;
-  __shared__ float s_int[PBR_MAX_LIGHTS * 3];
-  __shared__ float s_geo[(PBR_MAX_LIGHTS + 1) * 3];
-  __shared__ float s_loss[kCtThreads / 32];
-  const int tid = threadIdx.y * blockDim.x + threadIdx.x;
-  const CtFlags& F = p.flags;
-  const bool int_grad = p.d_intensity != nullptr;
-  const bool is_loss = p.is_loss != 0;
-  const bool has_normal = p.normal.ptr != nullptr;
-  for (int i = tid; i < F.L * 3; i += kCtThreads) s_int[i] = 0.0f;
-  for (int i = tid; i < (F.L + 1) * 3; i += kCtThreads) s_geo[i] = 0.0f;
-  stage_params(p, S);  // ends with __syncthreads()
-  const Where w = locate_ct<false>(p);
-  const float live = w.active ? 1.0f : 0.0f;   // edge threads stay for the warp-wide reductions
-
-  V x[kSlots];
-  float y;
-  LaneViews<V, kSlots> cv;
-  LightGeomT<V> hg[kSlots];
-  cam_setup<kLight>(p, S, w, x, y, cv, hg);
-
-  float loss_local = 0.0f;
-  const int b0 = blockIdx.z * p.mats_per_cta;
-  const int b1 = min(b0 + p.mats_per_cta, p.B);
-  for (int b = b0; b < b1; ++b) {
-    float araw[3][kCtTexels], nraw[3][kCtTexels], rough[kCtTexels], mraw[3][kCtTexels];
-    load_material<WF, false>(p, w, b, araw, nraw, rough, mraw, has_normal);
-    if (b + 1 < b1) prefetch_material<WF, false>(p, w, b + 1, has_normal);
-    V a[3][kSlots], n[3][kSlots], r[kSlots], m[3][kSlots];
-    pairs_of3<kSlots>(araw, 0, a); pairs_of3<kSlots>(nraw, 0, n); pairs_of3<kSlots>(mraw, 0, m); pairs_of<kSlots>(rough, 0, r);
-    // dLoss/d out of light l (per-light mode) or of the accumulated image: grad_out, or 2 * loss_scale * (out - target)
-    auto gout = [&](int l, const V(&outv)[3][kSlots], V(&g)[3][kSlots]) {
-#pragma unroll
-      for (int c = 0; c < 3; ++c) {
-        float src[kCtTexels], ov[kCtTexels], gv[kCtTexels];
-        load_seg<kCtTexels>(at<false>(p.gsrc, b, c, w) + (F.per_light ? (int64_t)l * p.gsrc_sl : 0), w.vec, w.valid, src);
-        unpair_to<kSlots>(outv[c], 0, ov);
-#pragma unroll
-        for (int i = 0; i < kCtTexels; ++i) {
-          if (is_loss) {
-            const float diff = (i < w.valid) ? ov[i] - src[i] : 0.0f;
-            loss_local += diff * diff;
-            gv[i] = 2.0f * p.loss_scale * diff;
-          } else {
-            gv[i] = (i < w.valid) ? src[i] : 0.0f;
-          }
-        }
-        pairs_of<kSlots>(gv, 0, g[c]);
-      }
-    };
-    auto int_sink = [&](int l, const float(&gi)[3]) {
-#pragma unroll
-      for (int c = 0; c < 3; ++c) {
-        const float sum = warp_sum(gi[c] * live);
-        if ((tid & 31) == 0) atomicAdd(&s_int[3 * l + c], sum);
-      }
-    };
-    V da[3][kSlots], dn[3][kSlots], dr[kSlots], dm[3][kSlots];
-    ct_backward_group<WF, kLight, V, kSlots, decltype(gout), decltype(int_sink), NoFetch, CtaGeomSink, NoSavedOut, kBwdUnroll,
-                      LaneViews<V, kSlots>>(S, F, a, n, r, m, x, y, hg, gout, int_sink, da, dn, dr, dm, NoFetch(), GeomCache<V>(),
-                                            CtaGeomSink{s_geo, F.L, tid, live, nullptr}, NoSavedOut(), int_grad, cv);
-    if (w.active) {
-      float d_albedo[3][kCtTexels], d_normal[3][kCtTexels], d_rough[kCtTexels], d_met[3][kCtTexels];
-#pragma unroll
-      for (int c = 0; c < 3; ++c) { unpair_to<kSlots>(da[c], 0, d_albedo[c]); unpair_to<kSlots>(dn[c], 0, d_normal[c]); unpair_to<kSlots>(dm[c], 0, d_met[c]); }
-      unpair_to<kSlots>(dr, 0, d_rough);
-      if (p.d_albedo.ptr) {
-#pragma unroll
-        for (int c = 0; c < 3; ++c) store_seg<kCtTexels>(at<false>(p.d_albedo, b, c, w), w.vec, w.valid, d_albedo[c]);
-      }
-      if (has_normal && p.d_normal.ptr) {
-#pragma unroll
-        for (int c = 0; c < 3; ++c) store_seg<kCtTexels>(at<false>(p.d_normal, b, c, w), w.vec, w.valid, d_normal[c]);
-      }
-      if (p.d_roughness.ptr) store_seg<kCtTexels>(at<false>(p.d_roughness, b, 0, w), w.vec, w.valid, d_rough);
-      if (p.d_metspec.ptr) {
-#pragma unroll
-        for (int c = 0; c < (WF == 0 ? 1 : 3); ++c) store_seg<kCtTexels>(at<false>(p.d_metspec, b, c, w), w.vec, w.valid, d_met[c]);
-      }
-    }
-  }
-
-  if (is_loss) {
-    const float sum = warp_sum(loss_local * live);
-    if ((tid & 31) == 0) s_loss[tid >> 5] = sum;
-  }
-  __syncthreads();
-  if (tid <= F.L) {
-    // the camera sum is already d/d c (camera_view_bwd per texel); a directional light's sum is w.r.t. its UNIT
-    // direction, whose Jacobian is image-constant and applied here, once
-    const float g[3] = {s_geo[3 * tid], s_geo[3 * tid + 1], s_geo[3 * tid + 2]};
-    float o[3] = {g[0], g[1], g[2]};
-    float* dst = p.d_view;
-    if (tid < F.L) {
-      const float* lights = p.lights_dev ? p.lights_dev : p.lights;
-      if (!F.point) normalize_bwd(lights + 3 * tid, g, o);
-      dst = p.d_lights ? p.d_lights + 3 * tid : nullptr;
-    }
-    if (dst) {
-#pragma unroll
-      for (int c = 0; c < 3; ++c) atomicAdd(dst + c, o[c]);
-    }
-  }
-  if (is_loss && tid == 0) {
-    float sum = 0.0f;
-    for (int i = 0; i < kCtThreads / 32; ++i) sum += s_loss[i];
-    atomicAdd(p.loss_sum, sum);
-  }
-  if (int_grad) {
-    for (int i = tid; i < F.L * 3; i += kCtThreads) atomicAdd(&p.d_intensity[i], s_int[i]);
-  }
+  ct_backward_body<WF, kLight, true, false, kFmGeneric, true>(p);
 }
 
 }  // namespace pbr
@@ -1333,6 +1211,7 @@ static size_t geom_cache_bytes(int L, int light_mode) { return (size_t)L * geom_
 
 static int light_mode(const CtKParams& k, bool backward) {
   if (!k.flags.point) return kLightDirectional;
+  if (k.camera) return k.flags.L == 1 ? kLightPointHoisted : kLightPoint;
   if (!k.vec_fast) return kLightPoint;              // the element-access flavour only exists for the uncached light modes
   if (k.d_lights || k.d_view) {
     // geometry gradients (shared parameters of a fit with unknown lighting): the 6-field cache when a walk over several
@@ -1354,7 +1233,8 @@ static int light_mode(const CtKParams& k, bool backward) {
 static void ct_launch_shape(CtKParams& k, dim3& grid, dim3& block, bool backward) {
   launch_shape(k.B, k.H, k.W, grid, block, kCtThreads, kCtTexels);
   const int lm = light_mode(k, backward);
-  k.mats_per_cta = (lm == kLightPointHoisted || is_cached(lm)) ? (k.B < kHoistMats ? k.B : kHoistMats) : 1;
+  // (the camera's views are per texel: computed once for the whole walk in every light mode)
+  k.mats_per_cta = (k.camera || lm == kLightPointHoisted || is_cached(lm)) ? (k.B < kHoistMats ? k.B : kHoistMats) : 1;
   grid.z = (k.B + k.mats_per_cta - 1) / k.mats_per_cta;
 }
 
@@ -1390,6 +1270,12 @@ static bool plain_case(const CtKParams& k) {
 template <int WF>
 static void launch_fwd(const CtKParams& k, dim3 grid, dim3 block, cudaStream_t st) {
   const int lm = light_mode(k, false);
+  if (k.camera) {
+    if (lm == kLightDirectional) cam_forward_kernel<WF, kLightDirectional><<<grid, block, 0, st>>>(k);
+    else if (lm == kLightPointHoisted) cam_forward_kernel<WF, kLightPointHoisted><<<grid, block, 0, st>>>(k);
+    else cam_forward_kernel<WF, kLightPoint><<<grid, block, 0, st>>>(k);
+    return;
+  }
   if (!k.vec_fast) {   // any alignment / ragged width: element accesses, uncached light modes
     if (lm == kLightDirectional) ct_forward_kernel<WF, kLightDirectional, false><<<grid, block, 0, st>>>(k);
     else ct_forward_kernel<WF, kLightPoint, false><<<grid, block, 0, st>>>(k);
@@ -1426,15 +1312,22 @@ static void launch_bwd(const CtKParams& k_in, dim3 grid, dim3 block, cudaStream_
   size_t smem = cache + (k.adam_on ? kAdamSmemBytes : 0);
   // per-thread slots of the shared-parameter gradients, when they fit next to the cache (else: warp-shuffle reduction per light)
   k.part_on = 0;
-  if (k.d_intensity || k.d_lights || k.d_view) {
-    const size_t part = (size_t)k.flags.L * ((k.d_lights || k.d_view) ? 6 : 3) * kCtThreads * sizeof(float);
+  const bool geom = k.camera || k.d_lights || k.d_view;   // a kGeom kernel (the camera's always is)
+  if (k.d_intensity || geom) {
+    const size_t part = (size_t)k.flags.L * (geom ? 6 : 3) * kCtThreads * sizeof(float);
     if (part <= 48 * 1024 && smem + part <= kMaxDynSmem) {
       k.part_on = 1;
       k.part_smem_off = (int)smem;
       smem += part;
     }
   }
-  if (k.d_lights || k.d_view) {   // geometry gradients: the uncached per-texel light modes
+  if (k.camera) {
+    if (lm == kLightDirectional) launch_dyn<cam_backward_kernel<WF, kLightDirectional>>(k, grid, block, smem, st);
+    else if (lm == kLightPointHoisted) launch_dyn<cam_backward_kernel<WF, kLightPointHoisted>>(k, grid, block, smem, st);
+    else launch_dyn<cam_backward_kernel<WF, kLightPoint>>(k, grid, block, smem, st);
+    return;
+  }
+  if (geom) {   // geometry gradients: the uncached per-texel light modes
     if (k.vec_fast) {
       if (lm == kLightPointCached) launch_dyn<ct_backward_kernel<WF, kLightPointCached, true>>(k, grid, block, smem, st);
       else if (k.flags.point) launch_dyn<ct_backward_kernel<WF, kLightPoint, true>>(k, grid, block, smem, st);
@@ -1494,7 +1387,7 @@ static bool fits_i32(const PbrPlane& pl, int H, int W) {
 }
 
 static bool stream_shape(const CtKParams& k, dim3& grid, dim3& block, int& mats) {
-  if (k.force_generic || k.flags.L != 1 || !k.vec_ok || (k.W % 4) != 0) return false;
+  if (k.force_generic || k.camera || k.flags.L != 1 || !k.vec_ok || (k.W % 4) != 0) return false;
   const int groups = k.W / kST;
   if (groups < 32) return false;   // narrower than one warp segment: the generic kernels take it
   int bx = 32;                     // per-warp copy pipelines: a warp must sit inside one tile row
@@ -1587,38 +1480,6 @@ void launch_wf1(CtKParams& k, dim3 grid, dim3 block, bool stream, bool backward,
 void launch_wf2(CtKParams& k, dim3 grid, dim3 block, bool stream, bool backward, cudaStream_t st) { launch_wf<2>(k, grid, block, stream, backward, st); }
 #endif
 
-// the camera kernels of one workflow (pbr_ct_*_camera): directional lights, one point light (hoisted), several point lights
-template <int WF>
-static void launch_cam(const CtKParams& k, dim3 grid, dim3 block, bool backward, cudaStream_t st) {
-  const int lm = !k.flags.point ? kLightDirectional : (k.flags.L == 1 ? kLightPointHoisted : kLightPoint);
-  switch (lm) {
-    case kLightDirectional:
-      if (backward) cam_backward_kernel<WF, kLightDirectional><<<grid, block, 0, st>>>(k);
-      else cam_forward_kernel<WF, kLightDirectional><<<grid, block, 0, st>>>(k);
-      break;
-    case kLightPointHoisted:
-      if (backward) cam_backward_kernel<WF, kLightPointHoisted><<<grid, block, 0, st>>>(k);
-      else cam_forward_kernel<WF, kLightPointHoisted><<<grid, block, 0, st>>>(k);
-      break;
-    default:
-      if (backward) cam_backward_kernel<WF, kLightPoint><<<grid, block, 0, st>>>(k);
-      else cam_forward_kernel<WF, kLightPoint><<<grid, block, 0, st>>>(k);
-      break;
-  }
-}
-void launch_cam_wf0(const CtKParams& k, dim3 grid, dim3 block, bool backward, cudaStream_t st);
-void launch_cam_wf1(const CtKParams& k, dim3 grid, dim3 block, bool backward, cudaStream_t st);
-void launch_cam_wf2(const CtKParams& k, dim3 grid, dim3 block, bool backward, cudaStream_t st);
-#if PBR_HAS_WF(0)
-void launch_cam_wf0(const CtKParams& k, dim3 grid, dim3 block, bool backward, cudaStream_t st) { launch_cam<0>(k, grid, block, backward, st); }
-#endif
-#if PBR_HAS_WF(1)
-void launch_cam_wf1(const CtKParams& k, dim3 grid, dim3 block, bool backward, cudaStream_t st) { launch_cam<1>(k, grid, block, backward, st); }
-#endif
-#if PBR_HAS_WF(2)
-void launch_cam_wf2(const CtKParams& k, dim3 grid, dim3 block, bool backward, cudaStream_t st) { launch_cam<2>(k, grid, block, backward, st); }
-#endif
-
 #if PBR_MAIN_PART
 // shared tail of the three Cook-Torrance entry points
 // every in-plane offset (row * sh + col) of a plane fits 32 bits
@@ -1634,7 +1495,7 @@ static bool planes_fit_i32(const CtKParams& k) {
 static int ct_dispatch(CtKParams& k, int wf, bool backward, cudaStream_t st) {
   dim3 grid, block;
   int mats = 1;
-  k.vec_fast = k.vec_ok && (k.W % kCtTexels) == 0 && planes_fit_i32(k);
+  k.vec_fast = !k.camera && k.vec_ok && (k.W % kCtTexels) == 0 && planes_fit_i32(k);
   bool stream = stream_shape(k, grid, block, mats);
   if (stream) {
     if (backward) stream = fits_i32(k.d_albedo, k.H, k.W) && fits_i32(k.d_normal, k.H, k.W) && fits_i32(k.d_roughness, k.H, k.W) && fits_i32(k.d_metspec, k.H, k.W);
@@ -1648,24 +1509,6 @@ static int ct_dispatch(CtKParams& k, int wf, bool backward, cudaStream_t st) {
     default: launch_wf2(k, grid, block, stream, backward, st); break;
   }
   return launch_result();
-}
-
-// the same for the camera kernels: every material walk spans up to kHoistMats materials (the views are per texel)
-static int cam_dispatch(CtKParams& k, int wf, bool backward, cudaStream_t st) {
-  dim3 grid, block;
-  launch_shape(k.B, k.H, k.W, grid, block, kCtThreads, kCtTexels);
-  k.mats_per_cta = k.B < kHoistMats ? k.B : kHoistMats;
-  grid.z = (k.B + k.mats_per_cta - 1) / k.mats_per_cta;
-  switch (wf) {
-    case 0: launch_cam_wf0(k, grid, block, backward, st); break;
-    case 1: launch_cam_wf1(k, grid, block, backward, st); break;
-    default: launch_cam_wf2(k, grid, block, backward, st); break;
-  }
-  return launch_result();
-}
-
-static int dispatch(CtKParams& k, int wf, bool backward, bool camera, cudaStream_t st) {
-  return camera ? cam_dispatch(k, wf, backward, st) : ct_dispatch(k, wf, backward, st);
 }
 #endif   // PBR_MAIN_PART
 
@@ -1724,7 +1567,8 @@ static int ct_forward(const PbrCtDesc* desc, bool camera, pbr_stream_t stream) {
   if (int rc = fill_ct_params(desc, k)) return rc;
   if (!desc->out.ptr) return PBR_E_NULL;
   k.vec_ok = k.vec_ok && plane_vec_ok(desc->out) && (desc->out_sl % kTexels == 0);
-  return dispatch(k, kernel_workflow(desc), false, camera, (cudaStream_t)stream);
+  k.camera = camera;
+  return ct_dispatch(k, kernel_workflow(desc), false, (cudaStream_t)stream);
 }
 
 static int ct_backward(const PbrCtDesc* desc, const PbrCtGrads* grads, bool camera, pbr_stream_t stream) {
@@ -1739,7 +1583,8 @@ static int ct_backward(const PbrCtDesc* desc, const PbrCtGrads* grads, bool came
     k.fout = grads->fwd_out;
     k.vec_ok = k.vec_ok && plane_vec_ok(grads->fwd_out);
   }
-  return dispatch(k, kernel_workflow(desc), true, camera, (cudaStream_t)stream);
+  k.camera = camera;
+  return ct_dispatch(k, kernel_workflow(desc), true, (cudaStream_t)stream);
 }
 
 static int ct_loss_fwd_bwd(const PbrCtDesc* desc, const PbrCtLoss* loss, const PbrCtGrads* grads, bool camera,
@@ -1752,7 +1597,8 @@ static int ct_loss_fwd_bwd(const PbrCtDesc* desc, const PbrCtLoss* loss, const P
   k.is_loss = 1;
   k.loss_scale = loss->loss_scale; k.loss_sum = loss->loss_sum;
   k.vec_ok = k.vec_ok && plane_vec_ok(loss->target) && (loss->target_sl % kTexels == 0);
-  return dispatch(k, kernel_workflow(desc), true, camera, (cudaStream_t)stream);
+  k.camera = camera;
+  return ct_dispatch(k, kernel_workflow(desc), true, (cudaStream_t)stream);
 }
 
 int pbr_ct_forward(const PbrCtDesc* desc, pbr_stream_t stream) { return ct_forward(desc, false, stream); }

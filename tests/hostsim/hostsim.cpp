@@ -5,6 +5,7 @@
 // Never loaded by the product package.
 #include <cstdint>
 #include <cstring>
+#include <type_traits>
 #include <vector>
 
 #include "pbr_shade.cuh"
@@ -17,7 +18,8 @@ struct Dims {
   int B, H, W, L;
 };
 
-// sums in double: [L][3] w.r.t. light position / unit direction, then [3] w.r.t. the unit view direction
+// sums in double: [L][3] w.r.t. light position / unit direction, then [3] w.r.t. the unit view direction (or the camera
+// position)
 struct HostGeomSink {
   static constexpr bool kOn = true;
   double* d_geo;
@@ -47,11 +49,29 @@ GeomCache<V> fill_cache(const CtStage& S, int L, V x, float y, V* store) {
   return gc;
 }
 
+// The view of one call's lane-values: the staged direction (OrthoView), or with CAM a camera at the position `cam`, what
+// the kernels' cam_* entry points compute per texel (LaneViews from camera_view).
+template <bool CAM, class V>
+using ViewT = typename std::conditional<CAM, LaneViews<V, 1>, OrthoView>::type;
+template <class V>
+void fill_views(const float*, V, float, OrthoView&) {}
+template <class V>
+void fill_views(const float* cam, V x, float y, LaneViews<V, 1>& v) { camera_view(cam, x, y, v.x[0], v.y[0], v.z[0], v.len[0]); }
+
+// per texel, as the kernels' grid_coords: the views, then the geometry of a hoisted point light
+template <int LIGHT, bool CAM, class V>
+void texel_views(const CtStage& S, const float* cam, V x, float y, ViewT<CAM, V>& views, LightGeomT<V>& hg) {
+  fill_views(cam, x, y, views);
+  if (LIGHT == kLightPointHoisted)
+    point_light_geom(S.light[0].p[0], S.light[0].p[1], S.light[0].p[2], x, y, view_x(S, views, 0), view_y(S, views, 0),
+                     view_z(S, views, 0), hg);
+}
+
 // One call shades Lanes<V>::n horizontally adjacent texels (V = float: 1, V = f2: 2, the packing the
 // CUDA kernels use); at a ragged right edge the second lane repeats the last column and is dropped.
-template <int WF, bool HASN, int LIGHT, class V>
+template <int WF, bool HASN, int LIGHT, class V, bool CAM = false>
 void fwd_impl(const Dims& d, const CtStage& S, const CtFlags& F, const float* albedo, const float* normal,
-              const float* rough, const float* metspec, float* out) {
+              const float* rough, const float* metspec, float* out, const float* cam = nullptr) {
   constexpr int NL = Lanes<V>::n;
   const int mc = WF == 0 ? 1 : 3;  // WF 2: metallic with 3 channels
   const int64_t HW = (int64_t)d.H * d.W;
@@ -77,19 +97,20 @@ void fwd_impl(const Dims& d, const CtStage& S, const CtFlags& F, const float* al
               out[idx] = lane_get(v[c][0], k);
             }
         };
+        ViewT<CAM, V> views;
         LightGeomT<V> hg[1];
-        if (LIGHT == kLightPointHoisted)
-          point_light_geom(S.light[0].p[0], S.light[0].p[1], S.light[0].p[2], x[0], y, S.vx, S.vy, S.vz, hg[0]);
+        texel_views<LIGHT, CAM>(S, cam, x[0], y, views, hg[0]);
         V store[PBR_MAX_LIGHTS * 8];
-        ct_forward_group<WF, LIGHT, V, 1>(S, F, a, n, r, m, x, y, hg, emit, fill_cache<LIGHT, V>(S, d.L, x[0], y, store));
+        ct_forward_group<WF, LIGHT, V, 1>(S, F, a, n, r, m, x, y, hg, emit, fill_cache<LIGHT, V>(S, d.L, x[0], y, store),
+                                          views);
       }
 }
 
-template <int WF, bool HASN, int LIGHT, class V>
+template <int WF, bool HASN, int LIGHT, class V, bool CAM = false>
 void bwd_impl(const Dims& d, const CtStage& S, const CtFlags& F, const float* albedo, const float* normal,
               const float* rough, const float* metspec, const float* grad_out, const float* target,
               float loss_scale, double* loss_sum, float* d_albedo, float* d_normal, float* d_rough, float* d_met,
-              double* d_int, double* d_geo = nullptr, bool use_saved_out = false) {
+              double* d_int, double* d_geo = nullptr, bool use_saved_out = false, const float* cam = nullptr) {
   constexpr int NL = Lanes<V>::n;
   const int mc = WF == 0 ? 1 : 3;  // WF 2: metallic with 3 channels
   const int64_t HW = (int64_t)d.H * d.W;
@@ -130,9 +151,9 @@ void bwd_impl(const Dims& d, const CtStage& S, const CtFlags& F, const float* al
             for (int c = 0; c < 3; ++c) d_int[3 * l + c] += gi[c];
         };
         V da[3][1], dn[3][1], dr[1], dm[3][1];
+        ViewT<CAM, V> views;
         LightGeomT<V> hg[1];
-        if (LIGHT == kLightPointHoisted)
-          point_light_geom(S.light[0].p[0], S.light[0].p[1], S.light[0].p[2], x[0], y, S.vx, S.vy, S.vz, hg[0]);
+        texel_views<LIGHT, CAM>(S, cam, x[0], y, views, hg[0]);
         V store[PBR_MAX_LIGHTS * 8];
         // accumulate mode, L > 1, "saved forward output" flavour: what the forward launch wrote for these texels
         HostSavedOut<V> saved{false, {}};
@@ -142,16 +163,16 @@ void bwd_impl(const Dims& d, const CtStage& S, const CtFlags& F, const float* al
           saved.on = true;
         }
         bool done = false;
-        if constexpr (LIGHT == kLightDirectional || LIGHT == kLightPoint) {
-          if (d_geo) {   // gradients of the light positions / directions and of the view direction
+        if constexpr (LIGHT == kLightDirectional || LIGHT == kLightPoint || (CAM && LIGHT == kLightPointHoisted)) {
+          if (d_geo) {   // gradients of the light positions / directions and of the view direction (camera position)
             ct_backward_group<WF, LIGHT, V, 1>(S, F, a, n, r, m, x, y, hg, gout, sink, da, dn, dr, dm, NoFetch(),
-                                               GeomCache<V>(), HostGeomSink{d_geo, d.L}, saved);
+                                               GeomCache<V>(), HostGeomSink{d_geo, d.L}, saved, true, views);
             done = true;
           }
         }
         if (!done)
           ct_backward_group<WF, LIGHT, V, 1>(S, F, a, n, r, m, x, y, hg, gout, sink, da, dn, dr, dm, NoFetch(),
-                                             fill_cache<LIGHT, V>(S, d.L, x[0], y, store), NoGeomSink(), saved);
+                                             fill_cache<LIGHT, V>(S, d.L, x[0], y, store), NoGeomSink(), saved, true, views);
         for (int k = 0; k < live; ++k) {
           for (int c = 0; c < 3; ++c) d_albedo[(b * 3 + c) * HW + o[k]] = lane_get(da[c][0], k);
           if (HASN && d_normal)
@@ -175,31 +196,47 @@ void make_stage(const Dims& d, int light_type, float light_size, const float* vi
 // (the kernels pick it for L > 1 when a thread walks over several materials).
 // `force_generic` bit 0: generic light mode; bit 1: V = f2 (two texels per call, the packing of the CUDA kernels);
 // bit 2: point lights with L > 1 go through the geometry cache (kLightPointCached); bits 2+3: kLightPointCachedAll.
-#define DISPATCH_LM(fn, WF, HN, V, ...)                                  \
+// CAM: the camera at a finite position, whose kernels have no cached mode: with force_generic 0 the same formula picks their
+// directional / per-texel point / hoisted modes, and the cached cases compile nothing of their own.
+#define DISPATCH_LM(fn, WF, HN, V, CAM, ...)                             \
   switch (lm) {                                                           \
-    case 0: fn<WF, HN, 0, V>(__VA_ARGS__); break;                         \
-    case 1: fn<WF, HN, 1, V>(__VA_ARGS__); break;                         \
-    case 2: fn<WF, HN, 2, V>(__VA_ARGS__); break;                         \
-    case 3: fn<WF, HN, 3, V>(__VA_ARGS__); break;                         \
-    default: fn<WF, HN, 4, V>(__VA_ARGS__); break;                        \
+    case 0: fn<WF, HN, 0, V, CAM>(__VA_ARGS__); break;                    \
+    case 1: fn<WF, HN, 1, V, CAM>(__VA_ARGS__); break;                    \
+    case 2: fn<WF, HN, 2, V, CAM>(__VA_ARGS__); break;                    \
+    case 3: fn<WF, HN, (CAM ? 1 : 3), V, CAM>(__VA_ARGS__); break;        \
+    default: fn<WF, HN, (CAM ? 1 : 4), V, CAM>(__VA_ARGS__); break;       \
   }
-#define DISPATCH_V(fn, V, ...)                                                                            \
+#define DISPATCH_V(fn, V, CAM, ...)                                                                       \
   do {                                                                                                     \
     int lm = light_type == 1 ? ((L == 1 && !(force_generic & 1)) ? 2 : ((L > 1 && (force_generic & 4)) ? ((force_generic & 8) ? 4 : 3) : 1)) : 0; \
     switch (workflow * 2 + (normal != nullptr)) {                                                          \
-      case 0: DISPATCH_LM(fn, 0, false, V, __VA_ARGS__) break;                                             \
-      case 1: DISPATCH_LM(fn, 0, true, V, __VA_ARGS__) break;                                              \
-      case 2: DISPATCH_LM(fn, 1, false, V, __VA_ARGS__) break;                                             \
-      case 3: DISPATCH_LM(fn, 1, true, V, __VA_ARGS__) break;                                              \
-      case 4: DISPATCH_LM(fn, 2, false, V, __VA_ARGS__) break;                                             \
-      case 5: DISPATCH_LM(fn, 2, true, V, __VA_ARGS__) break;                                              \
+      case 0: DISPATCH_LM(fn, 0, false, V, CAM, __VA_ARGS__) break;                                        \
+      case 1: DISPATCH_LM(fn, 0, true, V, CAM, __VA_ARGS__) break;                                         \
+      case 2: DISPATCH_LM(fn, 1, false, V, CAM, __VA_ARGS__) break;                                        \
+      case 3: DISPATCH_LM(fn, 1, true, V, CAM, __VA_ARGS__) break;                                         \
+      case 4: DISPATCH_LM(fn, 2, false, V, CAM, __VA_ARGS__) break;                                        \
+      case 5: DISPATCH_LM(fn, 2, true, V, CAM, __VA_ARGS__) break;                                         \
     }                                                                                                      \
   } while (0)
 #define DISPATCH(fn, ...)                                                                   \
   do {                                                                                      \
-    if (force_generic & 2) DISPATCH_V(fn, f2, __VA_ARGS__);                                 \
-    else DISPATCH_V(fn, float, __VA_ARGS__);                                                \
+    if (force_generic & 2) DISPATCH_V(fn, f2, false, __VA_ARGS__);                          \
+    else DISPATCH_V(fn, float, false, __VA_ARGS__);                                         \
   } while (0)
+
+// the kernels' flush of the geometry gradients: the Jacobians of F.normalize(dir) / F.normalize(view) applied once to the
+// sums (`view` null: the sum is already w.r.t. the camera position)
+void flush_geom(const std::vector<double>& geo, int L, int light_type, const float* lights, const float* view,
+                double* d_lights, double* d_view) {
+  for (int l = 0; l <= L; ++l) {
+    const float g[3] = {(float)geo[3 * l], (float)geo[3 * l + 1], (float)geo[3 * l + 2]};
+    float o[3] = {g[0], g[1], g[2]};
+    if (l == L && view) normalize_bwd(view, g, o);
+    else if (l < L && light_type != 1) normalize_bwd(lights + 3 * l, g, o);
+    double* dst = l == L ? d_view : d_lights + 3 * l;
+    for (int c = 0; c < 3; ++c) dst[c] = o[c];
+  }
+}
 
 }  // namespace
 
@@ -252,14 +289,42 @@ int hs_ct_backward_geom(int B, int H, int W, int L, int workflow, int light_type
   force_generic = (force_generic & 2) | 1;
   DISPATCH(bwd_impl, d, S, F, albedo, normal, rough, metspec, grad_out, target, loss_scale, loss_sum, d_albedo,
            d_normal, d_rough, d_met, d_int, geo.data());
-  for (int l = 0; l <= L; ++l) {
-    const float g[3] = {(float)geo[3 * l], (float)geo[3 * l + 1], (float)geo[3 * l + 2]};
-    float o[3] = {g[0], g[1], g[2]};
-    if (l == L) normalize_bwd(view, g, o);
-    else if (light_type != 1) normalize_bwd(lights + 3 * l, g, o);
-    double* dst = l == L ? d_view : d_lights + 3 * l;
-    for (int c = 0; c < 3; ++c) dst[c] = o[c];
-  }
+  flush_geom(geo, L, light_type, lights, view, d_lights, d_view);
+  return 0;
+}
+
+// A camera at a finite position (view_type="point"): `cam` is its position, the texels are shaded as the kernels' kCam
+// instantiations shade them (V = f2, per-texel views, directional / per-texel point / hoisted lights).  d_int, d_lights
+// [L][3] and d_cam [3] are sums in double; d_int is accumulated into.
+int hs_ct_forward_camera(int B, int H, int W, int L, int workflow, int light_type, float light_size, int albedo_is_srgb,
+                         int specular_is_srgb, int return_srgb, int per_light, const float* cam, const float* lights,
+                         const float* inten, const float* albedo, const float* normal, const float* rough,
+                         const float* metspec, float* out) {
+  if (L > PBR_MAX_LIGHTS) return -4;
+  Dims d{B, H, W, L};
+  static CtStage S;
+  make_stage(d, light_type, light_size, cam, lights, inten, S);
+  CtFlags F{L, light_type == 1, albedo_is_srgb != 0, specular_is_srgb != 0, return_srgb != 0, per_light != 0};
+  const int force_generic = 0;
+  DISPATCH_V(fwd_impl, f2, true, d, S, F, albedo, normal, rough, metspec, out, cam);
+  return 0;
+}
+
+int hs_ct_backward_camera(int B, int H, int W, int L, int workflow, int light_type, float light_size, int albedo_is_srgb,
+                          int specular_is_srgb, int return_srgb, int per_light, const float* cam, const float* lights,
+                          const float* inten, const float* albedo, const float* normal, const float* rough,
+                          const float* metspec, const float* grad_out, float* d_albedo, float* d_normal, float* d_rough,
+                          float* d_met, double* d_int, double* d_lights, double* d_cam) {
+  if (L > PBR_MAX_LIGHTS) return -4;
+  Dims d{B, H, W, L};
+  static CtStage S;
+  make_stage(d, light_type, light_size, cam, lights, inten, S);
+  CtFlags F{L, light_type == 1, albedo_is_srgb != 0, specular_is_srgb != 0, return_srgb != 0, per_light != 0};
+  std::vector<double> geo(3 * L + 3, 0.0);
+  const int force_generic = 0;
+  DISPATCH_V(bwd_impl, f2, true, d, S, F, albedo, normal, rough, metspec, grad_out, nullptr, 0.0f, nullptr, d_albedo,
+             d_normal, d_rough, d_met, d_int, geo.data(), false, cam);
+  flush_geom(geo, L, light_type, lights, nullptr, d_lights, d_cam);
   return 0;
 }
 

@@ -1,36 +1,29 @@
 """
 The camera at a finite position (view_type="point") on the CPU: the device math headers compiled for the host with the
-camera view type (tests/hostsim/camsim.cpp: the cam_* kernels' per-texel-pair arithmetic, V = f2) against the camera
-oracle (tests/camera_oracle.py) - the forward at rel 1e-5, every map gradient at rel 1e-4, and the intensity, light and
+camera view type (hs_ct_*_camera of tests/hostsim/hostsim.cpp: the per-texel-pair arithmetic of the kernels' camera
+instantiations, V = f2) against the camera oracle (tests/camera_oracle.py) - the forward at rel 1e-5, every map gradient at rel 1e-4, and the intensity, light and
 camera gradients against the fp64 oracle at 1e-4 |g| + 1e-4 mean|g|.  Also the API's refusals, which need no GPU.
 """
 import ctypes
-import os
-import subprocess
 
 import numpy as np
 import pytest
 import torch
 
 import camera_oracle as CO
-from conftest import ROOT, fwd_ok, grad_ok
+from conftest import fwd_ok, grad_ok
 
-CSRC = os.path.join(ROOT, "pypbr_b200", "csrc")
-SRC = os.path.join(ROOT, "tests", "hostsim", "camsim.cpp")
 WFS = {"metallic": 0, "specular": 1, "metallic3": 2}
 SHARED = ("intensity", "lights", "camera")
 
 
 @pytest.fixture(scope="module")
-def camsim(tmp_path_factory):
-    out = str(tmp_path_factory.mktemp("camsim") / "libcamsim.so")
-    subprocess.run(["g++", "-O2", "-ffp-contract=off", "-std=c++17", "-shared", "-fPIC", "-I", CSRC, SRC, "-o", out], check=True)
-    lib = ctypes.CDLL(out)
+def camera_sim(hostsim):
     f, i, p = ctypes.c_float, ctypes.c_int, ctypes.c_void_p
     head = [i] * 6 + [f] + [i] * 4 + [p] * 3
-    lib.cs_forward.argtypes = head + [p] * 5
-    lib.cs_backward.argtypes = head + [p] * 5 + [p] * 4 + [p] * 3
-    return lib
+    hostsim.hs_ct_forward_camera.argtypes = head + [p] * 5
+    hostsim.hs_ct_backward_camera.argtypes = head + [p] * 5 + [p] * 4 + [p] * 3
+    return hostsim
 
 
 def _ptr(a):
@@ -84,7 +77,7 @@ def _id(c):
 
 
 @pytest.mark.parametrize("c", CASES, ids=[_id(c) for c in CASES])
-def test_camera_matches_oracle_on_host(camsim, c):
+def test_camera_matches_oracle_on_host(camera_sim, c):
     B, H, W, L = 2, 5, 9, c["L"]   # odd W: the last texel pair is ragged
     maps, lights, inten, g = _case(100 + CASES.index(c), c["wf"], B, H, W, L, c["light"], c.get("normal", True))
     camera = torch.tensor(c.get("camera", (0.1, -0.15, 1.2)))
@@ -109,14 +102,14 @@ def test_camera_matches_oracle_on_host(camsim, c):
     par = [_np(camera), _np(lights), _np(inten)]
     args = head + tuple(_ptr(x) for x in par) + tuple(_ptr(a.get(k)) for k in ("albedo", "normal", "roughness", mkey))
     out = np.zeros(ref.shape, np.float32)
-    assert camsim.cs_forward(*args, _ptr(out)) == 0
+    assert camera_sim.hs_ct_forward_camera(*args, _ptr(out)) == 0
     ratio, ok = fwd_ok(out, ref.detach().numpy())
     assert ok, f"forward {ratio}"
 
     grads = {k: np.zeros(v.shape, np.float32) for k, v in a.items()}
     d_int, d_lights, d_cam = np.zeros(3 * L), np.zeros(3 * L), np.zeros(3)
     gout = _np(go)
-    assert camsim.cs_backward(*args, _ptr(gout), *(_ptr(grads.get(k)) for k in ("albedo", "normal", "roughness", mkey)),
+    assert camera_sim.hs_ct_backward_camera(*args, _ptr(gout), *(_ptr(grads.get(k)) for k in ("albedo", "normal", "roughness", mkey)),
                               _ptr(d_int), _ptr(d_lights), _ptr(d_cam)) == 0
     for k in maps:
         ratio, ok = grad_ok(grads[k], leaves[k].grad.numpy())

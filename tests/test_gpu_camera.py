@@ -11,8 +11,10 @@ plus projection applied to the oracle's gradients) and checks under torch.profil
 ct_* kernel, ran.  test_every_camera_kernel_has_a_row is the ledger: the cam_* instantiations defined in libpbrcuda.so
 must be exactly the union of the rows' kernels.
 
-Kernel names: cam_forward_kernel<WF, light>, cam_backward_kernel<WF, light>; WF 0 metallic (1-channel map), 1 specular,
-2 metallic with a 3-channel map; light 0 directional, 1 several point lights (per texel), 2 one point light (hoisted).
+Kernel names: cam_forward_kernel<WF, light>, cam_backward_kernel<WF, light> (the entry points of the generic kernels' bodies
+with the camera view, kCam); WF 0 metallic (1-channel map), 1 specular, 2 metallic with a 3-channel map; light 0
+directional, 1 several point lights (per texel), 2 one point light (hoisted).  test_the_two_ledgers_partition_the_library:
+every Cook-Torrance kernel of the library is in exactly one ledger, this file's or test_gpu_kernel_coverage.py's.
 """
 import os
 import re
@@ -115,6 +117,18 @@ def test_every_camera_kernel_has_a_row():
     assert not named - compiled, f"rows name kernels the library does not contain: {sorted(named - compiled)}"
     ids = [r["id"] for r in CASES]
     assert len(ids) == len(set(ids))
+
+
+def test_the_two_ledgers_partition_the_library():
+    from test_gpu_kernel_coverage import CASES as ORTHO_CASES, norm_kernel as norm_ct
+
+    out = subprocess.run(["nm", "-C", "--defined-only", LIB], check=True, capture_output=True, text=True).stdout
+    compiled = {norm_kernel(m.group(0)) or norm_ct(m.group(0))
+                for m in re.finditer(r"pbr::(?:ct|cam)_(?:forward|backward)_(?:kernel|stream)<[^<>]*>", out)}
+    cam = {k for r in CASES for k in r["kernels"]}
+    ortho = {k for r in ORTHO_CASES for k in r["kernels"]}
+    assert not cam & ortho, sorted(cam & ortho)
+    assert cam | ortho == compiled, sorted(compiled ^ (cam | ortho))
 
 
 def test_kernel_names_normalise():

@@ -1,7 +1,7 @@
 """
 tools/bench_camera.py — what a camera at a finite position costs: one forward + backward step through autograd
-(CookTorranceBRDF(view_type="point"), the cam_* kernels) against the same step with the orthographic view (the ct_*
-kernels), in the same process, the two alternating step by step, timed with CUDA events.
+(CookTorranceBRDF(view_type="point"), the cam_* kernels: the generic kernels' bodies with the camera view) against the same
+step with the orthographic view (the ct_* kernels), in the same process, the two alternating step by step, timed with CUDA events.
 
 Shapes: the C2 shape of bench.py (64 x 1024^2, one point light) and its C3 shape (16 x 2048^2, 16 point lights,
 accumulated), metallic workflow, every map gradient requested.  The maps, grad_out and gradients of either shape take
