@@ -366,6 +366,30 @@ int pbr_ct_forward_camera(const PbrCtDesc* desc, pbr_stream_t stream);
 int pbr_ct_backward_camera(const PbrCtDesc* desc, const PbrCtGrads* grads, pbr_stream_t stream);
 int pbr_ct_loss_fwd_bwd_camera(const PbrCtDesc* desc, const PbrCtLoss* loss, const PbrCtGrads* grads, pbr_stream_t stream);
 
+/*
+ * Per-material parameters of a batch: material b is shaded with its own view (or camera position), lights and intensities
+ * at desc->view + b*view_sb, desc->lights + b*lights_sb and desc->intensity + b*intensity_sb (strides in floats).  A stride
+ * of 0 shares that parameter across the batch, as the calls above do; each of the three is shared or per material on its
+ * own.  The gradient buffers grads->d_view / d_lights / d_intensity (and the fit step's d_intensity) take the same
+ * strides: a per-material parameter receives its own material's sums, a shared one the sum over the batch.  Results are
+ * those of B calls with B = 1, one per material.  camera = 1 reads desc->view as the camera position (pbr_ct_*_camera).
+ * Argument errors, before any launch: pb == NULL -> PBR_E_NULL; camera not 0 / 1, or a non-zero stride with
+ * params_on_device = 0 -> PBR_E_ENUM; a non-zero stride below 3 (view) or 3L (lights, intensity) -> PBR_E_SHAPE;
+ * camera = 1 on the fit step -> PBR_E_ENUM.  Otherwise the checks and codes of the calls without _pb.
+ */
+typedef struct PbrCtParamBatch {
+  int32_t camera;           /* 0: desc->view is the view direction; 1: the camera position */
+  int32_t pad;
+  int64_t view_sb, lights_sb, intensity_sb;
+} PbrCtParamBatch;
+
+int pbr_ct_forward_pb(const PbrCtDesc* desc, const PbrCtParamBatch* pb, pbr_stream_t stream);
+int pbr_ct_backward_pb(const PbrCtDesc* desc, const PbrCtParamBatch* pb, const PbrCtGrads* grads, pbr_stream_t stream);
+int pbr_ct_loss_fwd_bwd_pb(const PbrCtDesc* desc, const PbrCtParamBatch* pb, const PbrCtLoss* loss, const PbrCtGrads* grads,
+                           pbr_stream_t stream);
+int pbr_ct_fit_step_pb(const PbrCtDesc* desc, const PbrCtParamBatch* pb, const PbrCtLoss* loss, const PbrCtAdam* adam,
+                       float* d_intensity, pbr_stream_t stream);
+
 int pbr_convert_m2s(const PbrConvDesc* desc, pbr_stream_t stream);
 int pbr_convert_s2m(const PbrConvDesc* desc, pbr_stream_t stream);
 int pbr_convert_m2s_backward(const PbrConvDesc* desc, const PbrConvGrads* grads, pbr_stream_t stream);
@@ -384,7 +408,7 @@ int pbr_normal_op(const PbrNormalOpDesc* desc, pbr_stream_t stream);
 /* sizeof() of the descriptor structs as THIS library was compiled (binding self-check):
    which = 0 PbrPlane, 1 PbrCtDesc, 2 PbrCtGrads, 3 PbrCtLoss, 4 PbrConvDesc, 5 PbrBlendMap, 6 PbrBlendDesc,
    7 PbrColorDesc, 8 PbrNormalDesc, 9 PbrIngestDesc, 10 PbrIndexMap, 11 PbrIndexDesc, 12 PbrAdamMap, 13 PbrAdamDesc, 14 PbrCtAdam, 15 PbrNormalOpDesc,
-   16 PbrConvGrads, 17 PbrBlendGradMap, 18 PbrBlendGrads, 19 PbrNormalGrads;
+   16 PbrConvGrads, 17 PbrBlendGradMap, 18 PbrBlendGrads, 19 PbrNormalGrads, 20 PbrCtParamBatch;
    anything else returns 0. */
 uint64_t pbr_sizeof(int which);
 

@@ -63,6 +63,10 @@ class PbrCtLoss(Structure):
     _fields_ = [("target", PbrPlane), ("target_sl", c_int64), ("loss_scale", c_float), ("loss_sum", c_void_p)]
 
 
+class PbrCtParamBatch(Structure):
+    _fields_ = [("camera", c_int32), ("pad", c_int32), ("view_sb", c_int64), ("lights_sb", c_int64), ("intensity_sb", c_int64)]
+
+
 class PbrConvDesc(Structure):
     _fields_ = [
         ("B", c_int32), ("H", c_int32), ("W", c_int32), ("albedo_is_srgb", c_int32),
@@ -177,7 +181,7 @@ NORMAL_OP_ROTATE_BWD, NORMAL_OP_DIVERGENCE_BWD = 4, 5
 # order = the `which` argument of pbr_sizeof()
 STRUCTS = (PbrPlane, PbrCtDesc, PbrCtGrads, PbrCtLoss, PbrConvDesc, PbrBlendMap, PbrBlendDesc, PbrColorDesc, PbrNormalDesc,
            PbrIngestDesc, PbrIndexMap, PbrIndexDesc, PbrAdamMap, PbrAdamDesc, PbrCtAdam, PbrNormalOpDesc,
-           PbrConvGrads, PbrBlendGradMap, PbrBlendGrads, PbrNormalGrads)
+           PbrConvGrads, PbrBlendGradMap, PbrBlendGrads, PbrNormalGrads, PbrCtParamBatch)
 
 _lib = None
 
@@ -188,6 +192,7 @@ EXPORTS = (
     "pbr_normal_ingest", "pbr_ingest_image", "pbr_index_transform", "pbr_adam_step", "pbr_normal_op", "pbr_launch_count", "pbr_sizeof",
     "pbr_convert_m2s_backward", "pbr_convert_s2m_backward", "pbr_blend_backward", "pbr_normal_ingest_backward",
     "pbr_ct_forward_camera", "pbr_ct_backward_camera", "pbr_ct_loss_fwd_bwd_camera",
+    "pbr_ct_forward_pb", "pbr_ct_backward_pb", "pbr_ct_loss_fwd_bwd_pb", "pbr_ct_fit_step_pb",
 )
 
 
@@ -220,6 +225,12 @@ def load():
     lib.pbr_ct_forward_camera.argtypes = [POINTER(PbrCtDesc), c_void_p]
     lib.pbr_ct_backward_camera.argtypes = [POINTER(PbrCtDesc), POINTER(PbrCtGrads), c_void_p]
     lib.pbr_ct_loss_fwd_bwd_camera.argtypes = [POINTER(PbrCtDesc), POINTER(PbrCtLoss), POINTER(PbrCtGrads), c_void_p]
+    lib.pbr_ct_forward_pb.argtypes = [POINTER(PbrCtDesc), POINTER(PbrCtParamBatch), c_void_p]
+    lib.pbr_ct_backward_pb.argtypes = [POINTER(PbrCtDesc), POINTER(PbrCtParamBatch), POINTER(PbrCtGrads), c_void_p]
+    lib.pbr_ct_loss_fwd_bwd_pb.argtypes = [POINTER(PbrCtDesc), POINTER(PbrCtParamBatch), POINTER(PbrCtLoss), POINTER(PbrCtGrads),
+                                           c_void_p]
+    lib.pbr_ct_fit_step_pb.argtypes = [POINTER(PbrCtDesc), POINTER(PbrCtParamBatch), POINTER(PbrCtLoss), POINTER(PbrCtAdam),
+                                       c_void_p, c_void_p]
     lib.pbr_convert_m2s.argtypes = [POINTER(PbrConvDesc), c_void_p]
     lib.pbr_convert_s2m.argtypes = [POINTER(PbrConvDesc), c_void_p]
     lib.pbr_blend.argtypes = [POINTER(PbrBlendDesc), c_void_p]

@@ -227,7 +227,7 @@ __global__ void __launch_bounds__(kStreamThreads, kStreamFwdMinCtas) ct_forward_
     for (int s = 0; s < kStages * kPipes; ++s) mbar_init(&sh.full[s], 1);
     mbar_init_fence();
   }
-  stage_params(p, S);  // ends with __syncthreads()
+  stage_params<false>(p, S);  // ends with __syncthreads()  (never shades per-material parameters)
 
   const int b0 = blockIdx.z * p.mats_per_cta;
   const int ntiles = min(b0 + p.mats_per_cta, p.B) - b0;
@@ -317,7 +317,7 @@ __global__ void __launch_bounds__(kStreamThreads, kStreamBwdMinCtas) ct_backward
     for (int s = 0; s < kStages * kPipes; ++s) mbar_init(&sh.full[s], 1);
     mbar_init_fence();
   }
-  stage_params(p, S);  // ends with __syncthreads()
+  stage_params<false>(p, S);  // ends with __syncthreads()  (never shades per-material parameters)
 
   const int b0 = blockIdx.z * p.mats_per_cta;
   const int ntiles = min(b0 + p.mats_per_cta, p.B) - b0;

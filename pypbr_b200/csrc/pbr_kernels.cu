@@ -167,14 +167,25 @@ struct CtKParams {
   float view[3];
   float lights[PBR_MAX_LIGHTS * 3];
   float inten[PBR_MAX_LIGHTS * 3];
+  // per-material parameters (pbr_ct_*_pb): floats from one material's view / lights / intensities to the next material's,
+  // also between their gradients (d_view, d_lights, d_intensity); 0 = one set shared by the batch
+  int64_t view_sb, lights_sb, inten_sb;
 };
 
+// Offset of this CTA's parameters (and their gradients) for a per-material stride `sb`: the host gives a CTA one material
+// (mats_per_cta = 1, material blockIdx.z) whenever a stride is non-zero, so the one staged set is that material's.
+// kPm: the kernel can be launched with per-material parameters.  The host picks only the uncached light modes of the
+// generic kernels for them, so the streamed kernels and the geometry-cache modes compile with offset 0, as before.
+template <bool kPm>
+__device__ __forceinline__ int64_t mat_off(int64_t sb) { return kPm ? (int64_t)blockIdx.z * sb : 0; }
+
+template <bool kPm>
 __device__ __forceinline__ void stage_params(const CtKParams& p, CtStage& S) {
   const int tid = threadIdx.y * blockDim.x + threadIdx.x;
   const int nth = blockDim.x * blockDim.y;
-  const float* view = p.view_dev ? p.view_dev : p.view;
-  const float* lights = p.lights_dev ? p.lights_dev : p.lights;
-  const float* inten = p.inten_dev ? p.inten_dev : p.inten;
+  const float* view = (p.view_dev ? p.view_dev : p.view) + mat_off<kPm>(p.view_sb);
+  const float* lights = (p.lights_dev ? p.lights_dev : p.lights) + mat_off<kPm>(p.lights_sb);
+  const float* inten = (p.inten_dev ? p.inten_dev : p.inten) + mat_off<kPm>(p.inten_sb);
   if (tid < p.flags.L || tid == 0) {
     float vx, vy, vz;
     stage_view(view, vx, vy, vz);
@@ -292,7 +303,7 @@ extern __shared__ __align__(16) unsigned char s_dyn[];
 // view vector F.normalize(c - P) with P = (x, -y, 0) its plane position, and |c - P| for the adjoint.
 __device__ __forceinline__ void fill_views(const CtKParams&, const V (&)[kSlots], float, OrthoView&) {}
 __device__ __forceinline__ void fill_views(const CtKParams& p, const V (&x)[kSlots], float y, LaneViews<V, kSlots>& v) {
-  const float* cam = p.view_dev ? p.view_dev : p.view;
+  const float* cam = (p.view_dev ? p.view_dev : p.view) + mat_off<true>(p.view_sb);
   const float c[3] = {cam[0], cam[1], cam[2]};
 #pragma unroll
   for (int i = 0; i < kSlots; ++i) camera_view(c, x[i], y, v.x[i], v.y[i], v.z[i], v.len[i]);
@@ -381,7 +392,7 @@ __device__ __forceinline__ void ct_forward_body(const CtKParams& p) {
   static_assert(!kCam || cam_ok(kLight, kVec, kFM), "camera: see cam_ok");
   constexpr int G = kFwdGroup;
   __shared__ CtStage S;
-  stage_params(p, S);
+  stage_params<!is_cached(kLight)>(p, S);
   const Where w = locate_ct<kVec>(p);
   if (!w.active) return;
   const CtFlags F = plain_flags<kFM>(p.flags);
@@ -576,7 +587,8 @@ __device__ __forceinline__ void ct_backward_body(const CtKParams& p) {
   if (s_part) {
     for (int i = 0; i < p.flags.L * K; ++i) s_part[i * kCtThreads] = 0.0f;
   }
-  stage_params(p, S);  // ends with __syncthreads()
+  constexpr bool kPm = !is_cached(kLight);
+  stage_params<kPm>(p, S);  // ends with __syncthreads()
   const Where w = locate_ct<kVec>(p);
   const float live = w.active ? 1.0f : 0.0f;
   if (!w.active && !int_grad && !is_loss && !kGeom) return;  // nothing to reduce: edge threads may leave
@@ -873,18 +885,18 @@ __device__ __forceinline__ void ct_backward_body(const CtKParams& p) {
     // one thread per light (and one for the view) turns the CTA's partial sums into gradients of the RAW parameters:
     // the Jacobians of F.normalize(dir) / F.normalize(view) are constant over the image, hence applied here, once (the
     // camera's sum is already w.r.t. its position: camera_view_bwd per texel)
-    const float* view = p.view_dev ? p.view_dev : p.view;
-    const float* lights = p.lights_dev ? p.lights_dev : p.lights;
+    const float* view = (p.view_dev ? p.view_dev : p.view) + mat_off<kPm>(p.view_sb);
+    const float* lights = (p.lights_dev ? p.lights_dev : p.lights) + mat_off<kPm>(p.lights_sb);
     if (tid <= p.flags.L) {
       const float g[3] = {s_geo[3 * tid], s_geo[3 * tid + 1], s_geo[3 * tid + 2]};
       float o[3] = {g[0], g[1], g[2]};
       float* dst = nullptr;
       if (tid == p.flags.L) {
         if (!kCam) normalize_bwd(view, g, o);
-        dst = p.d_view;
+        dst = p.d_view ? p.d_view + mat_off<kPm>(p.view_sb) : nullptr;
       } else {
         if (!p.flags.point) normalize_bwd(lights + 3 * tid, g, o);
-        dst = p.d_lights ? p.d_lights + 3 * tid : nullptr;
+        dst = p.d_lights ? p.d_lights + mat_off<kPm>(p.lights_sb) + 3 * tid : nullptr;
       }
       if (dst) {
 #pragma unroll
@@ -899,7 +911,8 @@ __device__ __forceinline__ void ct_backward_body(const CtKParams& p) {
     atomicAdd(p.loss_sum, sum);
   }
   if (int_grad) {
-    for (int i = tid; i < p.flags.L * 3; i += kCtThreads) atomicAdd(&p.d_intensity[i], s_int[i]);
+    float* const d_int = p.d_intensity + mat_off<kPm>(p.inten_sb);
+    for (int i = tid; i < p.flags.L * 3; i += kCtThreads) atomicAdd(&d_int[i], s_int[i]);
   }
 }
 
@@ -1209,19 +1222,24 @@ constexpr int kGcAllMaxLights = 4;   // up to here all 8 geometry fields are cac
 constexpr int kGcBigMaxLights = 8;   // backward, 4 < L <= 8: all 8 fields cached, full register budget (2 CTAs per SM by registers anyway)
 static size_t geom_cache_bytes(int L, int light_mode) { return (size_t)L * geom_fields(light_mode) * kSlots * kCtThreads * sizeof(V); }
 
+// per-material parameters: each CTA stages its own material's, so it shades that one material and nothing is shared
+// across a walk (no streamed kernel, no geometry cache, mats_per_cta = 1)
+static bool per_material(const CtKParams& k) { return k.view_sb != 0 || k.lights_sb != 0 || k.inten_sb != 0; }
+
 static int light_mode(const CtKParams& k, bool backward) {
+  const bool walk = k.B >= 2 && !per_material(k);   // a CTA shades several materials with one set of parameters
   if (!k.flags.point) return kLightDirectional;
   if (k.camera) return k.flags.L == 1 ? kLightPointHoisted : kLightPoint;
   if (!k.vec_fast) return kLightPoint;              // the element-access flavour only exists for the uncached light modes
   if (k.d_lights || k.d_view) {
     // geometry gradients (shared parameters of a fit with unknown lighting): the 6-field cache when a walk over several
     // materials pays for it, else the per-texel geometry
-    if (backward && k.flags.L > 1 && k.B >= 2 && geom_cache_bytes(k.flags.L, kLightPointCached) <= kGcMaxBytes)
+    if (backward && k.flags.L > 1 && walk && geom_cache_bytes(k.flags.L, kLightPointCached) <= kGcMaxBytes)
       return kLightPointCached;
     return kLightPoint;
   }
   if (k.flags.L == 1) return kLightPointHoisted;
-  if (k.B >= 2) {
+  if (walk) {
     if (k.flags.L <= kGcAllMaxLights) return kLightPointCachedAll;
     // (not under the Adam epilogue: with its 30 KB of staging the two CTAs would leave the SM almost no L1, 12.21 -> 12.35 ms on C5)
     if (backward && !k.adam_on && k.flags.L <= kGcBigMaxLights) return kLightPointCachedAllBig;
@@ -1234,7 +1252,8 @@ static void ct_launch_shape(CtKParams& k, dim3& grid, dim3& block, bool backward
   launch_shape(k.B, k.H, k.W, grid, block, kCtThreads, kCtTexels);
   const int lm = light_mode(k, backward);
   // (the camera's views are per texel: computed once for the whole walk in every light mode)
-  k.mats_per_cta = (k.camera || lm == kLightPointHoisted || is_cached(lm)) ? (k.B < kHoistMats ? k.B : kHoistMats) : 1;
+  const bool walk = !per_material(k) && (k.camera || lm == kLightPointHoisted || is_cached(lm));
+  k.mats_per_cta = walk ? (k.B < kHoistMats ? k.B : kHoistMats) : 1;
   grid.z = (k.B + k.mats_per_cta - 1) / k.mats_per_cta;
 }
 
@@ -1387,7 +1406,7 @@ static bool fits_i32(const PbrPlane& pl, int H, int W) {
 }
 
 static bool stream_shape(const CtKParams& k, dim3& grid, dim3& block, int& mats) {
-  if (k.force_generic || k.camera || k.flags.L != 1 || !k.vec_ok || (k.W % 4) != 0) return false;
+  if (k.force_generic || k.camera || per_material(k) || k.flags.L != 1 || !k.vec_ok || (k.W % 4) != 0) return false;
   const int groups = k.W / kST;
   if (groups < 32) return false;   // narrower than one warp segment: the generic kernels take it
   int bx = 32;                     // per-warp copy pipelines: a warp must sit inside one tile row
@@ -1555,69 +1574,75 @@ uint64_t pbr_sizeof(int which) {
     case 17: return sizeof(PbrBlendGradMap);
     case 18: return sizeof(PbrBlendGrads);
     case 19: return sizeof(PbrNormalGrads);
+    case 20: return sizeof(PbrCtParamBatch);
     default: return 0;
   }
 }
 
 uint64_t pbr_launch_count(void) { return g_launches.load(std::memory_order_relaxed); }
 
-// camera: desc->view is the camera position (cam_* kernels) instead of the view direction (ct_* kernels)
-static int ct_forward(const PbrCtDesc* desc, bool camera, pbr_stream_t stream) {
+// Per-material parameters and the camera flag (PbrCtParamBatch), checked before any launch.  The plain entry points pass
+// strides of 0 (one set of parameters for the whole batch).
+static int fill_param_batch(const PbrCtDesc* d, const PbrCtParamBatch* pb, CtKParams& k) {
+  if (!pb) return PBR_E_NULL;
+  if (pb->camera != 0 && pb->camera != 1) return PBR_E_ENUM;
+  const int64_t sb[3] = {pb->view_sb, pb->lights_sb, pb->intensity_sb};
+  const int64_t least[3] = {3, 3 * (int64_t)d->L, 3 * (int64_t)d->L};
+  for (int i = 0; i < 3; ++i) {
+    if (sb[i] == 0) continue;
+    if (!d->params_on_device) return PBR_E_ENUM;   // host parameters travel in the launch: one set only
+    if (sb[i] < least[i]) return PBR_E_SHAPE;
+  }
+  k.camera = pb->camera;
+  k.view_sb = pb->view_sb; k.lights_sb = pb->lights_sb; k.inten_sb = pb->intensity_sb;
+  return PBR_OK;
+}
+
+static int ct_forward(const PbrCtDesc* desc, const PbrCtParamBatch* pb, pbr_stream_t stream) {
   CtKParams k{};
   if (int rc = fill_ct_params(desc, k)) return rc;
+  if (int rc = fill_param_batch(desc, pb, k)) return rc;
   if (!desc->out.ptr) return PBR_E_NULL;
   k.vec_ok = k.vec_ok && plane_vec_ok(desc->out) && (desc->out_sl % kTexels == 0);
-  k.camera = camera;
   return ct_dispatch(k, kernel_workflow(desc), false, (cudaStream_t)stream);
 }
 
-static int ct_backward(const PbrCtDesc* desc, const PbrCtGrads* grads, bool camera, pbr_stream_t stream) {
+static int ct_backward(const PbrCtDesc* desc, const PbrCtParamBatch* pb, const PbrCtGrads* grads, pbr_stream_t stream) {
   CtKParams k{};
   if (int rc = fill_ct_params(desc, k)) return rc;
+  if (int rc = fill_param_batch(desc, pb, k)) return rc;
   if (int rc = fill_grads(grads, k)) return rc;
   if (!grads->grad_out.ptr) return PBR_E_NULL;
   k.gsrc = grads->grad_out; k.gsrc_sl = grads->grad_out_sl;
   k.is_loss = 0;
   k.vec_ok = k.vec_ok && plane_vec_ok(grads->grad_out) && (grads->grad_out_sl % kTexels == 0);
-  if (!camera && !desc->per_light && desc->L > 1) {   // only the accumulate-mode backward of several lights has a use for it
+  if (!k.camera && !desc->per_light && desc->L > 1) {   // only the accumulate-mode backward of several lights has a use for it
     k.fout = grads->fwd_out;
     k.vec_ok = k.vec_ok && plane_vec_ok(grads->fwd_out);
   }
-  k.camera = camera;
   return ct_dispatch(k, kernel_workflow(desc), true, (cudaStream_t)stream);
 }
 
-static int ct_loss_fwd_bwd(const PbrCtDesc* desc, const PbrCtLoss* loss, const PbrCtGrads* grads, bool camera,
+static int ct_loss_fwd_bwd(const PbrCtDesc* desc, const PbrCtParamBatch* pb, const PbrCtLoss* loss, const PbrCtGrads* grads,
                            pbr_stream_t stream) {
   CtKParams k{};
   if (int rc = fill_ct_params(desc, k)) return rc;
+  if (int rc = fill_param_batch(desc, pb, k)) return rc;
   if (int rc = fill_grads(grads, k)) return rc;
   if (!loss || !loss->target.ptr || !loss->loss_sum) return PBR_E_NULL;
   k.gsrc = loss->target; k.gsrc_sl = loss->target_sl;
   k.is_loss = 1;
   k.loss_scale = loss->loss_scale; k.loss_sum = loss->loss_sum;
   k.vec_ok = k.vec_ok && plane_vec_ok(loss->target) && (loss->target_sl % kTexels == 0);
-  k.camera = camera;
   return ct_dispatch(k, kernel_workflow(desc), true, (cudaStream_t)stream);
 }
 
-int pbr_ct_forward(const PbrCtDesc* desc, pbr_stream_t stream) { return ct_forward(desc, false, stream); }
-int pbr_ct_backward(const PbrCtDesc* desc, const PbrCtGrads* grads, pbr_stream_t stream) { return ct_backward(desc, grads, false, stream); }
-int pbr_ct_loss_fwd_bwd(const PbrCtDesc* desc, const PbrCtLoss* loss, const PbrCtGrads* grads, pbr_stream_t stream) {
-  return ct_loss_fwd_bwd(desc, loss, grads, false, stream);
-}
-int pbr_ct_forward_camera(const PbrCtDesc* desc, pbr_stream_t stream) { return ct_forward(desc, true, stream); }
-int pbr_ct_backward_camera(const PbrCtDesc* desc, const PbrCtGrads* grads, pbr_stream_t stream) {
-  return ct_backward(desc, grads, true, stream);
-}
-int pbr_ct_loss_fwd_bwd_camera(const PbrCtDesc* desc, const PbrCtLoss* loss, const PbrCtGrads* grads, pbr_stream_t stream) {
-  return ct_loss_fwd_bwd(desc, loss, grads, true, stream);
-}
-
-int pbr_ct_fit_step(const PbrCtDesc* desc, const PbrCtLoss* loss, const PbrCtAdam* adam, float* d_intensity,
-                    pbr_stream_t stream) {
+static int ct_fit_step(const PbrCtDesc* desc, const PbrCtParamBatch* pb, const PbrCtLoss* loss, const PbrCtAdam* adam,
+                       float* d_intensity, pbr_stream_t stream) {
   CtKParams k{};
   if (int rc = fill_ct_params(desc, k)) return rc;
+  if (int rc = fill_param_batch(desc, pb, k)) return rc;
+  if (k.camera) return PBR_E_ENUM;   // the Adam epilogue is not compiled into the camera kernels
   if (!loss || !loss->target.ptr || !loss->loss_sum || !adam) return PBR_E_NULL;
   // the maps are updated in place: a batch-broadcast map (sb == 0) would be written by every material
   if (desc->B > 1 && (desc->albedo.sb == 0 || desc->roughness.sb == 0 || desc->metspec.sb == 0 || (desc->normal.ptr && desc->normal.sb == 0)))
@@ -1640,6 +1665,40 @@ int pbr_ct_fit_step(const PbrCtDesc* desc, const PbrCtLoss* loss, const PbrCtAda
   k.adam = AdamCoef{adam->step_size, adam->one_minus_beta1, adam->beta2, adam->one_minus_beta2, adam->bias2_sqrt, adam->eps};
   k.force_generic = 1;   // the Adam epilogue lives in the generic kernels (any L)
   return ct_dispatch(k, kernel_workflow(desc), true, (cudaStream_t)stream);
+}
+
+// the entry points with one set of parameters for the batch: the orthographic view (ct_* kernels) or a camera (cam_* kernels)
+static const PbrCtParamBatch kOrtho = {0, 0, 0, 0, 0};
+static const PbrCtParamBatch kCamera = {1, 0, 0, 0, 0};
+
+int pbr_ct_forward(const PbrCtDesc* desc, pbr_stream_t stream) { return ct_forward(desc, &kOrtho, stream); }
+int pbr_ct_backward(const PbrCtDesc* desc, const PbrCtGrads* grads, pbr_stream_t stream) { return ct_backward(desc, &kOrtho, grads, stream); }
+int pbr_ct_loss_fwd_bwd(const PbrCtDesc* desc, const PbrCtLoss* loss, const PbrCtGrads* grads, pbr_stream_t stream) {
+  return ct_loss_fwd_bwd(desc, &kOrtho, loss, grads, stream);
+}
+int pbr_ct_forward_camera(const PbrCtDesc* desc, pbr_stream_t stream) { return ct_forward(desc, &kCamera, stream); }
+int pbr_ct_backward_camera(const PbrCtDesc* desc, const PbrCtGrads* grads, pbr_stream_t stream) {
+  return ct_backward(desc, &kCamera, grads, stream);
+}
+int pbr_ct_loss_fwd_bwd_camera(const PbrCtDesc* desc, const PbrCtLoss* loss, const PbrCtGrads* grads, pbr_stream_t stream) {
+  return ct_loss_fwd_bwd(desc, &kCamera, loss, grads, stream);
+}
+int pbr_ct_fit_step(const PbrCtDesc* desc, const PbrCtLoss* loss, const PbrCtAdam* adam, float* d_intensity,
+                    pbr_stream_t stream) {
+  return ct_fit_step(desc, &kOrtho, loss, adam, d_intensity, stream);
+}
+
+int pbr_ct_forward_pb(const PbrCtDesc* desc, const PbrCtParamBatch* pb, pbr_stream_t stream) { return ct_forward(desc, pb, stream); }
+int pbr_ct_backward_pb(const PbrCtDesc* desc, const PbrCtParamBatch* pb, const PbrCtGrads* grads, pbr_stream_t stream) {
+  return ct_backward(desc, pb, grads, stream);
+}
+int pbr_ct_loss_fwd_bwd_pb(const PbrCtDesc* desc, const PbrCtParamBatch* pb, const PbrCtLoss* loss, const PbrCtGrads* grads,
+                           pbr_stream_t stream) {
+  return ct_loss_fwd_bwd(desc, pb, loss, grads, stream);
+}
+int pbr_ct_fit_step_pb(const PbrCtDesc* desc, const PbrCtParamBatch* pb, const PbrCtLoss* loss, const PbrCtAdam* adam,
+                       float* d_intensity, pbr_stream_t stream) {
+  return ct_fit_step(desc, pb, loss, adam, d_intensity, stream);
 }
 
 static int run_convert(const PbrConvDesc* d, bool m2s, pbr_stream_t stream) {

@@ -10,7 +10,8 @@ d loss / d(albedo, normal, roughness, metallic | specular) - the rendered image 
 Multi-GPU: materials are independent, so the batch is sharded across ranks with no data-path
 collective; the only exchange is ONE all-reduce per step over a (1 + 3L)-float buffer holding the
 loss sum and the gradients of the shared parameters - light intensities and, on request, light positions /
-directions and the view direction (`allreduce_loss_and_shared`).
+directions and the view direction (`allreduce_loss_and_shared`).  Per-material parameters (one view, set of lights or
+set of intensities per material) belong to the rank that holds the material and never enter that collective.
 """
 
 from __future__ import annotations
@@ -23,7 +24,7 @@ import torch.nn as nn
 
 from . import _cabi
 from .materials import MaterialBase
-from .models.cooktorrance import _fill_desc, _out_plane, _prepare, check_view_type
+from .models.cooktorrance import _fill_desc, _out_plane, _prepare, check_view_type, ct_call
 
 
 def shard_range(total: int, rank: int, world: int) -> Tuple[int, int]:
@@ -66,8 +67,11 @@ def fused_loss_step(
          want_geometry_grad) are then the gradient w.r.t. that position.
     Returns (buf, grads): buf is a device tensor [loss_sum, d_intensity(L*3)..., (d_lights(L*3)..., d_view(3))]
     (loss_sum is the UNscaled sum of squared errors; multiply by loss_scale for the mean), grads a dict of tensors.
+    Per-material parameters (view_dir (B, 3), lights (B, L, 3), intensity (B, L, 3) / (B, 1, 3), see CookTorranceBRDF):
+    their sections of buf stay zero, and their gradients, one set per material in the parameter's shape, are
+    grads["view" | "lights" | "intensity"], buffers kept in `out` and reused between steps (under the same keys; a (B, 1, 3)
+    intensity's gradient, summed over the lights, under "intensity_sum").
     """
-    lib = _cabi.load()
     cfg, (albedo, normal, roughness, metspec), _leaf, device = _prepare(
         material, device if device is not None else material.device, view_dir, lights, intensity, light_type, light_size,
         return_srgb, multi_light, view_type
@@ -103,19 +107,40 @@ def fused_loss_step(
         red = torch.empty(n_red, dtype=torch.float32, device=device)
         out["buf"] = red
     red.zero_()
-    g.d_intensity = red[1:].data_ptr() if want_intensity_grad else None
-    if want_geometry_grad:
-        g.d_lights = red[1 + 3 * cfg.L:].data_ptr()
-        g.d_view = red[1 + 6 * cfg.L:].data_ptr()
+    grads = {"albedo": d_albedo, "normal": d_normal, "roughness": d_rough,
+             ("metallic" if cfg.workflow == _cabi.WORKFLOW_METALLIC else "specular"): d_met}
+    # shared parameters: their section of buf; per-material ones: a (B, ...) buffer of their own
+    sections = (("intensity", want_intensity_grad, 1), ("lights", want_geometry_grad, 1 + 3 * cfg.L),
+                ("view", want_geometry_grad, 1 + 6 * cfg.L))
+    strides = (cfg.pb.intensity_sb, cfg.pb.lights_sb, cfg.pb.view_sb) if cfg.pb is not None else (0, 0, 0)
+    ptrs, per_material = [], {}
+    for (key, want, at), shape, sb in zip(sections, cfg.param_shapes, strides):
+        if not want:
+            ptrs.append(None)
+        elif sb:
+            t = out.get(key)
+            if t is None or t.shape != shape or t.device != red.device:
+                t = torch.empty(shape, dtype=torch.float32, device=device)
+                out[key] = t
+            t.zero_()
+            ptrs.append(t.data_ptr())
+            per_material[key] = (t, tuple(torch.as_tensor(intensity).shape) if key == "intensity" else shape)
+        else:
+            ptrs.append(red[at:].data_ptr())
+    g.d_intensity, g.d_lights, g.d_view = ptrs
     ls = _cabi.PbrCtLoss()
     ls.target, ls.target_sl = _out_plane(target, cfg.per_light, cfg.batched)
     ls.loss_scale = float(loss_scale)
     ls.loss_sum = red.data_ptr()
-    fn = "pbr_ct_loss_fwd_bwd_camera" if cfg.camera else "pbr_ct_loss_fwd_bwd"
     with torch.cuda.device(device):
-        _cabi.check(getattr(lib, fn)(_cabi.byref(d), _cabi.byref(ls), _cabi.byref(g), _cabi.stream_ptr(device)), fn)
-    grads = {"albedo": d_albedo, "normal": d_normal, "roughness": d_rough,
-             ("metallic" if cfg.workflow == _cabi.WORKFLOW_METALLIC else "specular"): d_met}
+        ct_call("loss_fwd_bwd", cfg, d, _cabi.byref(ls), _cabi.byref(g), device=device)
+    for key, (t, given) in per_material.items():
+        if t.shape != given:   # (B, L, 3) onto a (B, 1, 3) intensity, into a buffer of its own kept in `out`
+            r = out.get(key + "_sum")
+            if r is None or r.shape != given or r.device != t.device:
+                r = out[key + "_sum"] = torch.empty(given, dtype=torch.float32, device=device)
+            t = torch.sum(t, dim=1, keepdim=True, out=r)
+        grads[key] = t
     return red, grads
 
 
@@ -309,10 +334,11 @@ def fused_fit_step(
     if the material has one) - the very tensors stored in the material, contiguous, not batch-broadcast - with the
     default projection for all of them or none at all.  Anything else: use `fit_step(..., fused=False)`.
     The one-launch kernel shades with the view direction only: view_type="point" (a camera position) raises ValueError.
+    Per-material parameters are accepted as CookTorranceBRDF takes them; a per-material intensity's gradient goes to
+    scratch["d_intensity"] (B, L, 3) instead of the buffer.
     Returns the device buffer [sum of squared errors, d_intensity(L*3)...] (not all-reduced).
     """
     _no_camera(view_type)
-    lib = _cabi.load()
     cfg, (albedo, normal, roughness, metspec), _leaf, device = _prepare(
         material, material.device, view_dir, lights, intensity, light_type, light_size, return_srgb, multi_light
     )
@@ -363,12 +389,18 @@ def fused_fit_step(
     a.bias2_sqrt = (1.0 - b2 ** t) ** 0.5
     a.eps = optimizer.eps
     a.project = 1 if kinds == {True} else 0
-    d_int = ctypes.c_void_p(red[1:].data_ptr()) if want_intensity_grad else None
+    d_int = None
+    if want_intensity_grad:
+        if cfg.pb is not None and cfg.pb.intensity_sb:
+            d_int_buf = scratch.get("d_intensity")
+            if d_int_buf is None or d_int_buf.shape != cfg.param_shapes[0] or d_int_buf.device != red.device:
+                d_int_buf = scratch["d_intensity"] = torch.empty(cfg.param_shapes[0], dtype=torch.float32, device=device)
+            d_int_buf.zero_()
+            d_int = ctypes.c_void_p(d_int_buf.data_ptr())
+        else:
+            d_int = ctypes.c_void_p(red[1:].data_ptr())
     with torch.cuda.device(device):
-        _cabi.check(
-            lib.pbr_ct_fit_step(_cabi.byref(d), _cabi.byref(ls), _cabi.byref(a), d_int, _cabi.stream_ptr(device)),
-            "pbr_ct_fit_step",
-        )
+        ct_call("fit_step", cfg, d, _cabi.byref(ls), _cabi.byref(a), d_int, device=device)
     _cabi.touch(*optimizer.params.values())
     optimizer.step_count = t
     return red
@@ -387,6 +419,8 @@ def fit_step(material: MaterialBase, optimizer: FusedAdam, target: torch.Tensor,
     after its all-reduce of two steps ago has completed.
     `global_numel`: element count of the target over ALL ranks (the MSE denominator); default: this rank's.
     `view_type`: as CookTorranceBRDF's ("point": view_dir is the camera position); "point" needs fused=False.
+    Per-material parameters (view_dir (B, 3), lights (B, L, 3), intensity (B, L, 3) / (B, 1, 3)) belong to the materials:
+    a sharded fit passes each rank the same `shard_range` slice of them as of the maps and the target.
     Returns the all-reduced buffer [sum of squared errors, ...] (device tensor; multiply [0] by 1/global_numel), or
     the PendingLoss that will deliver it.
     """
@@ -454,7 +488,7 @@ class RenderingLoss(nn.Module):
         kw = dict(light_type=self.light_type, light_size=self.light_size, multi_light="per_light",
                   want_map_grads=want_maps, want_intensity_grad=want_int, want_geometry_grad=want_geo,
                   device=self.brdf.override_device, view_type=self.view_type)
-        L = shared[1].shape[0] if shared[1].dim() == 2 else 1
+        L = shared[1].shape[-2] if shared[1].dim() >= 2 else 1
 
         class _Fn(torch.autograd.Function):
             @staticmethod
@@ -465,10 +499,11 @@ class RenderingLoss(nn.Module):
                 ctx.grads = [grads[k].sum_to_size(t.shape) if (want_maps and grads.get(k) is not None) else None
                              for k, t in zip(names, leaves)]
                 red = red.detach()
-                g_int = red[1:1 + 3 * L].view(L, 3) if want_int else None
-                g_light = red[1 + 3 * L:1 + 6 * L].view(L, 3) if want_geo else None
-                g_view = red[1 + 6 * L:1 + 6 * L + 3] if want_geo else None
-                def onto(g, t):   # (L,3) rows onto a (3,) or (L,3) leaf; (3,) onto any 3-element view tensor
+                # a per-material parameter's gradient is grads[key] ((B, ...), its own shape); a shared one's is in buf
+                g_int = grads.get("intensity", red[1:1 + 3 * L].view(L, 3)) if want_int else None
+                g_light = grads.get("lights", red[1 + 3 * L:1 + 6 * L].view(L, 3)) if want_geo else None
+                g_view = grads.get("view", red[1 + 6 * L:1 + 6 * L + 3]) if want_geo else None
+                def onto(g, t):   # (L,3) rows onto a (3,), (L,3) or (1,L,3) leaf; (3,) onto any 3-element view tensor
                     if g is None:
                         return None
                     g = g.reshape(t.shape) if g.numel() == t.numel() else g.sum_to_size(t.shape)

@@ -14,7 +14,10 @@ Extensions over the reference (which is single-material, single-light, cooktorra
       multi_light="per_light"  -> one image per light, shape (..., L, 3, H, W)
     both reduce to the reference for L = 1;
   * view_type="point": `view_dir` is the position of a camera at a finite distance, and every texel is shaded with its own
-    view vector F.normalize(camera - P) (texel (i, j) at P = (x_j, -y_i, 0) on the plane of side `light_size or 1.0`).
+    view vector F.normalize(camera - P) (texel (i, j) at P = (x_j, -y_i, 0) on the plane of side `light_size or 1.0`);
+  * per-material parameters for batched maps: `view_dir` (B, 3), `light_dir_or_position` (B, L, 3), `light_intensity`
+    (B, L, 3) or (B, 1, 3), each on its own; a leading dimension of 1 is shared by the batch.  Material b is shaded exactly
+    as a call with material[b], view_dir[b], lights[b], intensity[b] would shade it (pbr_ct_*_pb).
 """
 
 from __future__ import annotations
@@ -44,16 +47,67 @@ def _as_f32_rows(t: Tensor, name: str) -> Tensor:
         t = torch.as_tensor(t, dtype=torch.float32)
     if t.dim() == 1:
         t = t.view(1, -1)
-    if t.dim() != 2 or t.shape[1] != 3:
-        raise ValueError(f"{name} must have shape (3,) or (L, 3), got {tuple(t.shape)}")
+    if t.dim() not in (2, 3) or t.shape[-1] != 3:
+        raise ValueError(f"{name} must have shape (3,), (L, 3) or (B, L, 3), got {tuple(t.shape)}")
     return t
+
+
+def _per_material(t: Tensor, B: int, batched: bool, name: str) -> bool:
+    """Whether a parameter with a leading batch dimension holds one set per material (B) or one for the batch (1)."""
+    if t.shape[0] == 1:
+        return False
+    if not batched:
+        raise ValueError(f"{name} of shape {tuple(t.shape)} holds per-material parameters, which need batched (B, 3, H, W) maps")
+    if t.shape[0] != B:
+        raise ValueError(f"{name} has {t.shape[0]} parameter sets for a batch of {B} materials; expected {B} or 1")
+    return True
+
+
+def _parse_params(view_dir, light, intensity, B: int, batched: bool):
+    """The view, lights and intensities of a call on B materials -> (view, lights (L, 3) | (B, L, 3), intensities of the
+    lights' shape, whether the lights count as several, which of (intensity, lights, view) are per material).  Each is
+    shared by the batch or, with a leading dimension of B, one set per material; a leading dimension of 1 is shared."""
+    view = torch.as_tensor(view_dir, dtype=torch.float32) if not isinstance(view_dir, Tensor) else view_dir
+    lights = _as_f32_rows(light, "light_dir_or_position")
+    multi = lights.dim() == 3 or (isinstance(light, Tensor) and light.dim() == 2)
+    pm_lights = lights.dim() == 3 and _per_material(lights, B, batched, "light_dir_or_position")
+    if lights.dim() == 3 and not pm_lights:
+        lights = lights[0]
+    inten = _as_f32_rows(intensity, "light_intensity")   # (a 2-D intensity is (L, 3), whatever B is)
+    pm_inten = inten.dim() == 3 and _per_material(inten, B, batched, "light_intensity")
+    if inten.dim() == 3 and not pm_inten:
+        inten = inten[0]
+    L = lights.shape[-2]
+    if inten.shape[-2] != L:
+        if inten.shape[-2] != 1:
+            raise ValueError(f"light_intensity has {inten.shape[-2]} rows for {L} lights")
+        inten = inten.expand(*inten.shape[:-2], L, 3)
+    if L > _cabi.PBR_MAX_LIGHTS:
+        raise ValueError(f"at most {_cabi.PBR_MAX_LIGHTS} lights per call, got {L}")
+    pm_view = view.numel() != 3 and view.dim() == 2 and view.shape[1] == 3 and _per_material(view, B, batched, "view_dir")
+    if view.numel() != 3 and not pm_view:
+        raise ValueError(f"view_dir must have shape (3,) or (B, 3), got {tuple(view.shape)}")
+    return view, lights, inten, multi, (pm_inten, pm_lights, pm_view)
 
 
 class _ShadeCfg:
     """Everything about one shading call that is not a texture map."""
 
     __slots__ = ("workflow", "metallic_channels", "light_type", "albedo_is_srgb", "specular_is_srgb", "return_srgb",
-                 "per_light", "light_size", "L", "view", "lights", "intensity", "on_device", "batched", "multi", "camera")
+                 "per_light", "light_size", "L", "view", "lights", "intensity", "on_device", "batched", "multi", "camera",
+                 "pb", "param_shapes")
+
+
+def ct_call(kind: str, cfg: _ShadeCfg, desc, *args, device) -> None:
+    """pbr_ct_<kind>: with per-material parameters its _pb form, with a camera its _camera form."""
+    lib = _cabi.load()
+    if cfg.pb is not None:
+        fn = f"pbr_ct_{kind}_pb"
+        rc = getattr(lib, fn)(_cabi.byref(desc), _cabi.byref(cfg.pb), *args, _cabi.stream_ptr(device))
+    else:
+        fn = f"pbr_ct_{kind}_camera" if cfg.camera else f"pbr_ct_{kind}"
+        rc = getattr(lib, fn)(_cabi.byref(desc), *args, _cabi.stream_ptr(device))
+    _cabi.check(rc, fn)
 
 
 def _fill_desc(cfg: _ShadeCfg, albedo, normal, roughness, metspec, keep: list) -> "_cabi.PbrCtDesc":
@@ -115,14 +169,12 @@ def check_view_type(view_type: str) -> str:
 class _CookTorranceFn(torch.autograd.Function):
     @staticmethod
     def forward(ctx, cfg: _ShadeCfg, albedo, normal, roughness, metspec, intensity_leaf, lights_leaf=None, view_leaf=None):
-        lib = _cabi.load()
         keep: list = []
         d = _fill_desc(cfg, albedo, normal, roughness, metspec, keep)
         out = torch.empty(_out_shape(cfg, albedo), dtype=torch.float32, device=albedo.device)
         d.out, d.out_sl = _out_plane(out, cfg.per_light, cfg.batched)
-        fn = "pbr_ct_forward_camera" if cfg.camera else "pbr_ct_forward"
         with _cabi.device_guard(albedo.device):
-            _cabi.check(getattr(lib, fn)(_cabi.byref(d), _cabi.stream_ptr(albedo.device)), fn)
+            ct_call("forward", cfg, d, device=albedo.device)
         ctx.cfg = cfg
         ctx.has_normal = normal is not None
         # the shared parameters may live on another device than the maps (the reference moves them with .to(device))
@@ -140,7 +192,6 @@ class _CookTorranceFn(torch.autograd.Function):
         albedo, normal, roughness, metspec, fwd_out = ctx.saved_tensors
         if not ctx.has_normal:
             normal = None
-        lib = _cabi.load()
         keep: list = []
         d = _fill_desc(cfg, albedo, normal, roughness, metspec, keep)
         grad_out = grad_out.contiguous()
@@ -154,20 +205,20 @@ class _CookTorranceFn(torch.autograd.Function):
         d_normal = torch.empty(normal.shape, dtype=torch.float32, device=dev) if (need[2] and normal is not None) else None
         d_rough = torch.empty(roughness.shape, dtype=torch.float32, device=dev) if need[3] else None
         d_met = torch.empty(metspec.shape, dtype=torch.float32, device=dev) if need[4] else None
-        d_int = torch.zeros(cfg.L, 3, dtype=torch.float32, device=dev) if need[5] else None
+        # the shared parameters' gradients are sums over the batch; a per-material parameter's, one set per material
+        # (the gradient buffers take the parameters' strides)
+        d_int, d_lights, d_view = (torch.zeros(shape, dtype=torch.float32, device=dev) if want else None
+                                   for shape, want in zip(cfg.param_shapes, need[5:8]))
         g.d_albedo = _cabi.plane(d_albedo)
         g.d_normal = _cabi.plane(d_normal)
         g.d_roughness = _cabi.plane(d_rough)
         g.d_metspec = _cabi.plane(d_met)
         g.d_intensity = d_int.data_ptr() if d_int is not None else None
         # gradients of the light positions / directions and of the view direction (plain autograd in the reference)
-        d_lights = torch.zeros(cfg.L, 3, dtype=torch.float32, device=dev) if need[6] else None
-        d_view = torch.zeros(3, dtype=torch.float32, device=dev) if need[7] else None
         g.d_lights = d_lights.data_ptr() if d_lights is not None else None
         g.d_view = d_view.data_ptr() if d_view is not None else None
-        fn = "pbr_ct_backward_camera" if cfg.camera else "pbr_ct_backward"
         with _cabi.device_guard(dev):
-            _cabi.check(getattr(lib, fn)(_cabi.byref(d), _cabi.byref(g), _cabi.stream_ptr(dev)), fn)
+            ct_call("backward", cfg, d, _cabi.byref(g), device=dev)
         shared = []
         for t, meta in zip((d_int, d_lights, d_view), ctx.leaf_meta):
             shared.append(t.reshape(meta[1]).to(meta[0]) if (t is not None and meta is not None) else None)
@@ -251,20 +302,13 @@ def _prepare(material: MaterialBase, device, view_dir, light, intensity, light_t
     cfg.light_size = float(light_size or 1.0) if (light_type == "point" or cfg.camera) else 0.0
     cfg.return_srgb = bool(return_srgb)
 
-    view = torch.as_tensor(view_dir, dtype=torch.float32) if not isinstance(view_dir, Tensor) else view_dir
-    lights = _as_f32_rows(light, "light_dir_or_position")
-    cfg.multi = isinstance(light, Tensor) and light.dim() == 2
-    inten = _as_f32_rows(intensity, "light_intensity")
-    cfg.L = lights.shape[0]
-    if inten.shape[0] != cfg.L:
-        if inten.shape[0] != 1:
-            raise ValueError(f"light_intensity has {inten.shape[0]} rows for {cfg.L} lights")
-        inten = inten.expand(cfg.L, 3)
-    if cfg.L > _cabi.PBR_MAX_LIGHTS:
-        raise ValueError(f"at most {_cabi.PBR_MAX_LIGHTS} lights per call, got {cfg.L}")
+    B = albedo.shape[0] if cfg.batched else 1
+    view, lights, inten, cfg.multi, (pm_inten, pm_lights, pm_view) = _parse_params(view_dir, light, intensity, B, cfg.batched)
+    cfg.L = lights.shape[-2]
     cfg.per_light = cfg.multi and multi_light == "per_light"
-    if view.numel() != 3:
-        raise ValueError(f"view_dir must have shape (3,), got {tuple(view.shape)}")
+    # shapes of the kernels' gradient buffers (intensity, lights, view): one set per material, or the sum over the batch
+    cfg.param_shapes = ((B, cfg.L, 3) if pm_inten else (cfg.L, 3), (B, cfg.L, 3) if pm_lights else (cfg.L, 3),
+                        (B, 3) if pm_view else (3,))
 
     # views of the caller's tensors: their (L, 3) / (3,) gradients reach the caller through autograd's view tracking
     shared_leaves = (inten if inten.requires_grad else None,
@@ -273,16 +317,19 @@ def _prepare(material: MaterialBase, device, view_dir, light, intensity, light_t
     # compare with the device the maps actually live on: torch.device("cuda") (no index) never equals "cuda:0", and the
     # device-resident fast path (no .tolist() sync, graph-capturable) would be dead for material.to("cuda")
     device = albedo.device
-    all_dev = all(t.is_cuda and t.device == device for t in (view, lights, inten))
+    cfg.pb = None
+    if pm_view or pm_lights or pm_inten:
+        # per-material parameters are read from device memory (the launch carries one set only): all three go there
+        cfg.pb = _cabi.PbrCtParamBatch(int(cfg.camera), 0, 3 if pm_view else 0, 3 * cfg.L if pm_lights else 0,
+                                       3 * cfg.L if pm_inten else 0)
+    all_dev = cfg.pb is not None or all(t.is_cuda and t.device == device for t in (view, lights, inten))
     cfg.on_device = all_dev
     if all_dev:
         def f32c(t):
-            t = t.detach()
-            if t.dtype != torch.float32:
-                t = t.to(torch.float32)
+            t = t.detach().to(device=device, dtype=torch.float32)
             return t if t.is_contiguous() else t.contiguous()
 
-        cfg.view = f32c(view).reshape(3)
+        cfg.view = f32c(view).reshape(cfg.param_shapes[2])
         cfg.lights = f32c(lights)
         cfg.intensity = f32c(inten)
     else:  # small host arrays are copied into the kernel launch parameters: no H2D copy, no sync for CPU inputs
@@ -299,6 +346,12 @@ class CookTorranceBRDF(BRDFModel):
     view_type: "directional" (the reference: `view_dir` is one view direction for the whole image) or "point"
     (`view_dir` is the position of a camera at a finite distance, in the frame of a point light's position; each
     texel is shaded with its own view vector).
+
+    Per-material parameters (batched maps only): view_dir (B, 3), light_dir_or_position (B, L, 3), light_intensity
+    (B, L, 3) or (B, 1, 3), each on its own; material b is shaded as a call on material[b] with view_dir[b], lights[b],
+    intensity[b] would shade it.  Such a call reads all three parameters from the maps' device, so any of them given on
+    the CPU is copied there (a synchronous copy from pageable memory) on every call: keep them on the maps' device in a
+    loop.
 
     Example:
         brdf = CookTorranceBRDF(light_type="point")
